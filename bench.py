@@ -33,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the bench runs from a built tree that may be read-only: it leaves no caches in it
 
 NTAPS, DECIM, NFFT, K_AVG = 64, 10, 1024, 64
 FRAMES = 65536                      # 2^26 decimated samples / 1024
@@ -421,6 +422,19 @@ def run_extras(ctx, world, rank, peak_hbm, quick=False):
     return out
 
 
+def dump_rows(out_dir, rows, world, rank):
+    """DIR/psd_rows.npy: the f32 PSD rows of the last timed step, every rank's rows in rank order (4 MB per rank)"""
+    import torch
+    import torch.distributed as dist
+    if world > 1:
+        full = torch.empty((world * rows.shape[0], rows.shape[1]), dtype=rows.dtype, device=rows.device)
+        dist.all_gather_into_tensor(full, rows)
+        rows = full
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "psd_rows.npy"), rows.cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------------
@@ -611,6 +625,8 @@ def run_ours(args):
 
     total_ms, kern_ms = timed_loop(True)
     torch.cuda.synchronize()
+    if args.dump_outputs:
+        dump_rows(args.dump_outputs, outs[(args.steps - 1) & 1], world, rank)
     if world > 1:
         dist.barrier()
     if gather is not None:
@@ -916,7 +932,14 @@ def main():
                          "rank 0's GPU (a gather over NVLink), every rank (all-gather), or a receiver that rotates from step to step")
     ap.add_argument("--gather", default="ce", choices=["ce", "nccl"],
                     help="N > 1: output gather by lrc_gather (copy engines over NVLink, default) or NCCL all-gather")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", dest="dump_outputs",
+                    help="write the PSD rows of the last timed step to DIR/psd_rows.npy (f32; the input is seeded, so two "
+                         "builds run with the same arguments can be compared row for row)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the rows of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

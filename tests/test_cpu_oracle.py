@@ -161,8 +161,19 @@ def test_fft_self_test_thresholds_of_reference(n):
     assert D.snr_db(np.fft.ifft(x.astype(np.complex128)) * n, oracle.fft(x, True)) >= 100.0
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
-def test_restated_fft_and_fastfir_bit_exact_vs_vendored_build():
+def test_restated_fft_and_fastfir_bit_exact_vs_vendored_build(golden):
+    """Bit for bit against the vendored kissfft: its stored outputs (tests/golden) always -- radix 4/2 and the generic odd-prime
+    butterfly (7; 11 and 13 inside 1001), kiss_fastfir with and without flush -- and the live build too where oracle/_ref exists."""
+    import tests.golden.make_golden as mg
+    for n in (2, 64, 1024, 8192, 7, 97, 1001, 7919):
+        x = mg.fft_input(n)
+        for inv, key in ((False, f"fwd_{n}"), (True, f"inv_{n}")):
+            assert np.array_equal(oracle.fft(x, inv).view(np.uint32), golden[key].view(np.uint32)), (n, inv)
+    h, x = mg.fastfir_case()
+    for flush, key in ((False, "fastfir_noflush"), (True, "fastfir_flush")):
+        assert np.array_equal(oracle.fastfir(h, x, 0, flush).view(np.uint32), golden[key].view(np.uint32)), flush
+    if not oracle.have_ref():
+        return
     rng = np.random.default_rng(1)
     for n in (2, 64, 1024, 8192, 7, 11):
         x = (rng.standard_normal(n) + 1j * rng.standard_normal(n)).astype(np.complex64)
