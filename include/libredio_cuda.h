@@ -295,6 +295,36 @@ int lrc_ook_fetch_packets(lrc_ook *ook, lrc_ook_packet *h_packets, size_t cap, s
  * (value<<31 | length) u32 [n_streams][max_runs] */
 int lrc_ook_debug_ptrs(lrc_ook *ook, const float **d_block_sums, const uint32_t **d_run_counts,
                        const uint32_t **d_runs, const uint32_t **d_n_bits);
+/* Streaming form of the same chain, for a live receiver that delivers the capture a few blocks at a time.
+ * Every stream carries the state the reference's blocks hold between two messages (trigger threshold and counter,
+ * the burst still being collected, the open run of rle, the matchers' pending pulse and partial packet), so the
+ * packets emitted after any push are exactly those the reference emits on the concatenation of all pushes so far,
+ * whatever the push sizes.  The blocks of a burst still open at the end of a push are kept in a per-stream carry of
+ * max_carry_blocks blocks (0 = the trigger's OOM guard + 1 = 50 001 blocks, 51 MB per stream: exact for every
+ * input); a smaller carry is a memory choice, and a burst that outgrows it is reported (LRC_ERR_CAPACITY naming the
+ * stream, no packet from it), never decoded wrongly.  LRC_OOK_TEST_GUARD_BLOCKS is read at create, as for lrc_ook.
+ * The slicer always runs in its split form here (LRC_OOK_KC is not read). */
+typedef struct lrc_ook_stream lrc_ook_stream;
+int lrc_ook_stream_create(lrc_ctx *ctx, size_t n_streams, size_t max_push_blocks, unsigned sample_rate,
+                          size_t max_carry_blocks, size_t max_runs_per_push, size_t max_packets_per_fetch,
+                          lrc_ook_stream **st);
+int lrc_ook_stream_destroy(lrc_ook_stream *st);
+/* back to the reference's initial state (every stream; packet sequence numbers restart at 0) */
+int lrc_ook_stream_reset(lrc_ook_stream *st);
+/* n_blocks (1..max_push_blocks, may differ from push to push) new blocks per stream, stream s at
+ * d_iq + s*stream_stride_bytes; 16-byte aligned like lrc_ook_decode.  Asynchronous. */
+int lrc_ook_stream_push(lrc_ook_stream *st, const uint8_t *d_iq, size_t n_blocks, size_t stream_stride_bytes,
+                        void *stream);
+/* synchronises; the packets completed since the previous fetch, ordered by (stream, proto, seq), seq counting from
+ * create/reset.  LRC_ERR_CAPACITY if cap is too small (then *n_packets = required and nothing is consumed), and
+ * naming the stream if one overflowed max_carry_blocks, max_runs_per_push, max_packets_per_fetch or its bursts per
+ * push: then no packet is returned and every push and fetch fails until lrc_ook_stream_reset. */
+int lrc_ook_stream_fetch_packets(lrc_ook_stream *st, lrc_ook_packet *h_packets, size_t cap, size_t *n_packets);
+/* stage-by-stage parity for the last push, as lrc_ook_debug_ptrs: its block sums [n_streams][n_blocks of that push],
+ * the number of runs it completed, those runs (value<<31 | length, the first one including its length before the
+ * push), and the bits it emitted; bit positions count from the start of the push */
+int lrc_ook_stream_debug_ptrs(lrc_ook_stream *st, const float **d_block_sums, const uint32_t **d_run_counts,
+                              const uint32_t **d_runs, const uint32_t **d_n_bits);
 /* kpn::eat (kpn.rs:116-124): split MSB-first bit fields; pure host helper for the wrappers */
 int lrc_eat(const uint8_t *bits, size_t nbits, const size_t *widths, size_t n_widths, size_t *out);
 /* |i2f(b0) + j*i2f(b1)| for all 65536 byte pairs computed ON THE DEVICE with the envelope routine the

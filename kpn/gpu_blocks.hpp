@@ -12,13 +12,14 @@
 //   (north-star) discriminator                    kpn_gpu::fm_demod
 //   (north-star) FIR->FFT->|X|^2 chain            kpn_gpu::chain_psd
 //   (north-star) config-3 FM receiver, N channels  kpn_gpu::fm_receiver_multi (lrc_fmrx: one kernel per batch)
-//   trigger..shaper_optional  ratpak.rs:60-111    kpn_gpu::ook_decode
+//   trigger..shaper_optional  ratpak.rs:60-111    kpn_gpu::ook_decode, kpn_gpu::ook_decode_stream (live, message by message)
 //
 // Errors: a non-zero status of the C ABI is thrown as std::runtime_error -- the analogue of the
 // reference's `panic!(src_strerror(..))` (samplerate.rs:77-83); spawn() lets the thread die, which drops
 // the block's ports and tears the graph down like any other panic.  There is no CPU fallback.
 #pragma once
 #include <cuda_runtime_api.h>
+#include <algorithm>
 #include <complex>
 #include <cstdint>
 #include <cstring>
@@ -387,6 +388,46 @@ inline void ook_decode(Gpu &g, Receiver<std::vector<uint8_t>> u, Sender<OokPacke
             }
         }
     } catch (...) { lrc_ook_destroy(ook); in.release(g); throw; }
+}
+
+// The streaming form, for a live receiver: every message holds the NEXT k blocks of each of the n_streams streams,
+// stream-major (n_streams * k * 1024 bytes), k free to change from message to message.  The state of the reference's
+// trigger .. shaper_optional blocks lives on the device between messages, so the packets sent after a message are exactly
+// those the reference's per-block threads would have sent on all the bytes so far: a packet that crosses a message
+// boundary is not lost.  A message longer than max_push_blocks per stream is pushed in pieces (the result does not depend
+// on how the stream is cut).  max_carry_blocks = 0: the exact carry (the trigger's OOM guard + 1 blocks per stream).
+inline void ook_decode_stream(Gpu &g, Receiver<std::vector<uint8_t>> u, Sender<OokPacket> v, size_t n_streams, unsigned s_rate,
+                              size_t max_push_blocks = 1024, size_t max_carry_blocks = 0, size_t max_runs_per_push = 1 << 16,
+                              size_t max_packets_per_fetch = 256)
+{
+    g.bind();
+    lrc_ook_stream *ook = nullptr;
+    check(lrc_ook_stream_create(g.ctx, n_streams, max_push_blocks, s_rate, max_carry_blocks, max_runs_per_push,
+                                max_packets_per_fetch, &ook), "lrc_ook_stream_create");
+    Stream st; Slot in;
+    std::vector<lrc_ook_packet> pk(n_streams * 2 * max_packets_per_fetch);
+    try {
+        for (;;) {
+            std::vector<uint8_t> msg = u.recv();
+            if (msg.empty() || msg.size() % (n_streams * 1024) != 0)
+                throw std::length_error("ook_decode_stream: message size is not n_streams * k * 1024 bytes");
+            const size_t k = msg.size() / (n_streams * 1024);
+            in.reserve(g, msg.size());
+            std::memcpy(in.h, msg.data(), msg.size());
+            cuda_check(cudaMemcpyAsync(in.d, in.h, msg.size(), cudaMemcpyHostToDevice, st.s), "H2D");
+            for (size_t b = 0; b < k; b += max_push_blocks) {
+                const size_t n = std::min(max_push_blocks, k - b);
+                check(lrc_ook_stream_push(ook, (const uint8_t *)in.d + b * 1024, n, k * 1024, st.s), "lrc_ook_stream_push");
+                size_t np = 0;
+                check(lrc_ook_stream_fetch_packets(ook, pk.data(), pk.size(), &np), "lrc_ook_stream_fetch_packets");
+                for (size_t q = 0; q < np; ++q) {
+                    OokPacket p{pk[q].stream, pk[q].proto, {}};
+                    for (uint32_t i = 0; i < pk[q].nbits; ++i) p.bits.push_back(pk[q].bits[i]);
+                    v.send(std::move(p));
+                }
+            }
+        }
+    } catch (...) { lrc_ook_stream_destroy(ook); in.release(g); throw; }
 }
 
 // the packets of ook_decode back onto the reference's two ports: what shaper_optional(36) and shaper_optional(24) send

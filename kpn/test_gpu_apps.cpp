@@ -7,6 +7,11 @@
 //                                 protocol B (24 bits): applicator(|x| {x.push(0); x})          (ratpak.rs:60-123)
 //         every field tuple must equal the expected file's (written by tests/test_gpu_kpn.py from the bits the synthetic
 //         capture was built to carry AND from the CPU oracle's decode of the same capture).
+//   ook_stream <capture.iq> <k> <expected.txt>
+//         the same graph as a live receiver runs it: iq_file_source_u8 -> batch(k) (the last message holds what is left)
+//           -> kpn_gpu::ook_decode_stream (state carried on the device from message to message) -> split_protocols -> ...
+//         k is meant not to divide a burst's length: packets cross message boundaries.  The expected file is the `ook`
+//         mode's for the whole capture.
 //   psd   <file.wav> <rate> <chunk> <k_avg> <expected.f32>
 //         wav_source_complex_chunks (wavio.rs:30-46 as Vec chunks) -> kpn_gpu::chain_psd (FIR64/10 -> Hann FFT1024 -> |X|^2)
 //         rows within 1e-4 x RMS of the expected rows (oracle FIR + f64 PSD, per chunk).
@@ -36,9 +41,27 @@ static void batch(Receiver<std::vector<uint8_t>> u, Sender<std::vector<uint8_t>>
     }
 }
 
-static int app_ook(int argc, char **argv)
+// like batch, but the end of the input sends what was collected: a live stream has no whole number of messages
+static void batch_flush(Receiver<std::vector<uint8_t>> u, Sender<std::vector<uint8_t>> v, size_t n_blocks)
 {
-    if (argc < 5) { std::printf("usage: ook capture.iq n_blocks expected.txt\n"); return 2; }
+    for (;;) {
+        std::vector<uint8_t> cap;
+        try {
+            for (size_t k = 0; k < n_blocks; ++k) {
+                std::vector<uint8_t> x = u.recv();
+                cap.insert(cap.end(), x.begin(), x.end());
+            }
+        } catch (const PortClosed &) {
+            if (!cap.empty()) v.send(std::move(cap));
+            throw;
+        }
+        v.send(std::move(cap));
+    }
+}
+
+static int app_ook(int argc, char **argv, bool streaming)
+{
+    if (argc < 5) { std::printf("usage: ook|ook_stream capture.iq n_blocks|k expected.txt\n"); return 2; }
     const std::string cap = argv[2], expf = argv[4];
     const size_t n_blocks = (size_t)std::atol(argv[3]);
     kpn_gpu::Gpu gpu(0);
@@ -53,9 +76,11 @@ static int app_ook(int argc, char **argv)
     auto [sf2, rf2] = channel<std::vector<size_t>>();
     auto [sfb, rfb] = channel<std::vector<size_t>>();
     std::thread t0 = spawn([s = std::move(s0), cap]() mutable { iq_file_source_u8(std::move(s), cap, 512); });
-    std::thread t1 = spawn([r = std::move(r0), s = std::move(s1), n_blocks]() mutable { batch(std::move(r), std::move(s), n_blocks); });
-    std::thread t2 = spawn([&gpu, r = std::move(r1), s = std::move(s2), n_blocks]() mutable {
-        kpn_gpu::ook_decode(gpu, std::move(r), std::move(s), 1, n_blocks, 256000); });
+    std::thread t1 = spawn([r = std::move(r0), s = std::move(s1), n_blocks, streaming]() mutable {
+        if (streaming) batch_flush(std::move(r), std::move(s), n_blocks); else batch(std::move(r), std::move(s), n_blocks); });
+    std::thread t2 = spawn([&gpu, r = std::move(r1), s = std::move(s2), n_blocks, streaming]() mutable {
+        if (streaming) kpn_gpu::ook_decode_stream(gpu, std::move(r), std::move(s), 1, 256000);
+        else kpn_gpu::ook_decode(gpu, std::move(r), std::move(s), 1, n_blocks, 256000); });
     std::thread t3 = spawn([r = std::move(r2), a = std::move(sa), b = std::move(sb)]() mutable {
         kpn_gpu::split_protocols(std::move(r), std::move(a), std::move(b)); });
     // ratpak.rs:98-101: the 36-bit packets fork to BOTH field layouts; :112-119
@@ -92,7 +117,7 @@ static int app_ook(int argc, char **argv)
         CHECK(!rxs[p]->try_recv().has_value());
     }
     CHECK(n_got >= 1);
-    std::printf("kpn app ook OK (%zu packets)\n", n_got);
+    std::printf("kpn app %s OK (%zu packets)\n", streaming ? "ook_stream" : "ook", n_got);
     return 0;
 }
 
@@ -139,8 +164,9 @@ static int app_psd(int argc, char **argv)
 
 int main(int argc, char **argv)
 {
-    if (argc >= 2 && !std::strcmp(argv[1], "ook")) return app_ook(argc, argv);
+    if (argc >= 2 && !std::strcmp(argv[1], "ook")) return app_ook(argc, argv, false);
+    if (argc >= 2 && !std::strcmp(argv[1], "ook_stream")) return app_ook(argc, argv, true);
     if (argc >= 2 && !std::strcmp(argv[1], "psd")) return app_psd(argc, argv);
-    std::printf("usage: test_gpu_apps ook|psd ...\n");
+    std::printf("usage: test_gpu_apps ook|ook_stream|psd ...\n");
     return 2;
 }

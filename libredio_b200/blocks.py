@@ -514,6 +514,65 @@ class Ook:
             self.h = C.c_void_p()
 
 
+class OokStream:
+    """The OOK chain of ratpak.rs:60-111 on n_streams endless streams, pushed a few 512-sample blocks at a time: the
+    packets after any push are those the reference emits on everything pushed so far, whatever the push sizes.
+    max_carry_blocks = 0 keeps the exact carry (the trigger's OOM guard + 1 blocks per stream)."""
+
+    def __init__(self, ctx: Context, n_streams: int, max_push_blocks: int, sample_rate: int = 256000,
+                 max_carry_blocks: int = 0, max_runs: int = 4096, max_packets: int = 64):
+        self.ctx, self.n_streams, self.max_push_blocks = ctx, n_streams, max_push_blocks
+        self.max_runs, self.max_packets = max_runs, max_packets
+        self.last_push = 0
+        self.h = C.c_void_p()
+        check(ctx.lib.lrc_ook_stream_create(ctx.h, n_streams, max_push_blocks, sample_rate, max_carry_blocks, max_runs,
+                                            max_packets, C.byref(self.h)), "lrc_ook_stream_create")
+
+    def push(self, iq: torch.Tensor):
+        """iq: uint8 [n_streams, k*1024] on the device, the next k blocks of every stream.  Asynchronous."""
+        assert iq.dtype == torch.uint8 and iq.is_cuda and iq.dim() == 2 and iq.stride(1) == 1
+        assert iq.shape[0] == self.n_streams and iq.shape[1] % 1024 == 0
+        n = iq.shape[1] // 1024
+        check(self.ctx.lib.lrc_ook_stream_push(self.h, _p(iq), n, iq.stride(0), _stream()), "lrc_ook_stream_push")
+        self.last_push = n
+
+    def packets(self):
+        """-> the packets completed since the last call, as (stream, proto, seq, bits uint8[nbits]) ordered by
+        (stream, proto, seq); seq counts from create / reset."""
+        n = C.c_size_t()
+        cap = self.n_streams * 2 * self.max_packets
+        buf = (capi.OokPacket * max(cap, 1))()
+        check(self.ctx.lib.lrc_ook_stream_fetch_packets(self.h, buf, cap, C.byref(n)), "lrc_ook_stream_fetch_packets")
+        out = []
+        for k in range(n.value):
+            p = buf[k]
+            out.append((p.stream, p.proto, p.seq, np.frombuffer(bytes(p.bits)[: p.nbits], dtype=np.uint8).copy()))
+        return out
+
+    def reset(self):
+        check(self.ctx.lib.lrc_ook_stream_reset(self.h), "lrc_ook_stream_reset")
+        self.last_push = 0
+
+    def debug(self) -> dict:
+        """The last push's intermediate products on the host: block_sums [S, k] f32, n_runs [S] (runs it completed),
+        runs [S, max_runs] as (value << 31 | length), n_bits [S] (bits it emitted)."""
+        ps = [C.c_void_p() for _ in range(4)]
+        check(self.ctx.lib.lrc_ook_stream_debug_ptrs(self.h, *[C.byref(p) for p in ps]), "lrc_ook_stream_debug_ptrs")
+        S, B, R = self.n_streams, self.last_push, self.max_runs
+        out = {}
+        for name, ptr, shape, dt in (("block_sums", ps[0], (S, B), np.float32), ("n_runs", ps[1], (S,), np.uint32),
+                                     ("runs", ps[2], (S, R), np.uint32), ("n_bits", ps[3], (S,), np.uint32)):
+            host = np.empty(shape, dtype=dt)
+            check(self.ctx.lib.lrc_copy_to_host(self.ctx.h, _p(host), ptr, host.nbytes), "lrc_copy_to_host")
+            out[name] = host
+        return out
+
+    def close(self):
+        if self.h:
+            self.ctx.lib.lrc_ook_stream_destroy(self.h)
+            self.h = C.c_void_p()
+
+
 def ook_envelope_table(ctx: Context) -> torch.Tensor:
     """|i2f(b0) + j i2f(b1)| for all 65536 byte pairs, computed by the device routine the OOK kernels use."""
     t = torch.empty(65536, dtype=torch.float32, device=ctx.tdev)

@@ -110,6 +110,12 @@ SIGNATURES = {
     "lrc_ook_decode": (_i, [_vp, _u8p, _sz, _vp]),
     "lrc_ook_fetch_packets": (_i, [_vp, _vp, _sz, _szp]),
     "lrc_ook_debug_ptrs": (_i, [_vp, _pp, _pp, _pp, _pp]),
+    "lrc_ook_stream_create": (_i, [_vp, _sz, _sz, C.c_uint, _sz, _sz, _sz, _pp]),
+    "lrc_ook_stream_destroy": (_i, [_vp]),
+    "lrc_ook_stream_reset": (_i, [_vp]),
+    "lrc_ook_stream_push": (_i, [_vp, _u8p, _sz, _sz, _vp]),
+    "lrc_ook_stream_fetch_packets": (_i, [_vp, _vp, _sz, _szp]),
+    "lrc_ook_stream_debug_ptrs": (_i, [_vp, _pp, _pp, _pp, _pp]),
     "lrc_eat": (_i, [_vp, _sz, _vp, _sz, _vp]),
     "lrc_ook_envelope_table": (_i, [_vp, _fp, _vp]),
     "lrc_gather_create": (_i, [_vp, _i, _i, _sz, _i, _pp]),

@@ -27,6 +27,12 @@
 //                              bit stream and the transition list, every block writes its transitions in place
 //   K-D  ook_match_kernel    : per stream: run lengths -> seconds (dle, IEEE f32 division) -> matcher A and B ->
 //                              shaper_optional -> packed packets
+//
+// Two plans run these kernels.  lrc_ook decodes finite captures, every stream from the reference's initial state.
+// lrc_ook_stream decodes endless streams pushed a few blocks at a time: K-B, K-B2, the split K-C and K-D take a per-stream
+// OokSeam (null for lrc_ook) with what the reference's blocks hold between two messages, and ook_carry_kernel keeps the
+// blocks of the burst still open at the end of a push, which the slicer reads in place, in front of the push's blocks, when
+// that burst is sent.  The packets after any push are those of the reference on everything pushed so far.
 #include "common.cuh"
 #include "unpack.cuh"
 #include <cuda.h>
@@ -158,6 +164,49 @@ struct lrc_ook {
     uint16_t *d_rank;                 // [65536] rank of the pair's envelope among the distinct envelope values
     float    *d_uniq;                 // [n_uniq] the distinct envelope values, ascending
     uint32_t  n_uniq;
+    size_t    cpitch;                 // carry slots per stream in front of the blocks of d_mask / d_bsum / d_binfo (0: batch plan)
+};
+
+// ---- streaming (lrc_ook_stream) -------------------------------------------------------------------------------------------
+// Everything one stream holds between two pushes: the state of the reference's blocks as they stand between two messages.  The
+// kernels take a pointer to an array of these that is null on the batch path (initial state, nothing carried).
+struct OokSeam {
+    // K-B walker (bitfount.rs:41-44, :46-70): threshold, counter (clamped at -1: every counter below 0 walks the same way), and the
+    // two look-ahead predicates of the walk; keeper (:43, :52-54, :73-81): buffer length in samples, buffer starts with the 0.0
+    float    threshold;
+    int32_t  trig;
+    uint32_t buf_len;
+    uint8_t  fired, low2, lead0, pad0;
+    // the open burst: collected blocks held in the carry region, and their running maximum (discretize :90 is order-free)
+    uint32_t n_carry;
+    float    run_max;
+    // K-C2: value of the last bit emitted, whether any bit was
+    uint32_t prev, any;
+    // K-D: the open run of rle (kpn.rs:17-29), the matchers' state (ratpak.rs:88-97, kpn.rs:266-275) per protocol
+    unsigned long long run_len;
+    uint32_t run_val;
+    uint32_t m_pending[2], m_n[2], m_count[2];
+    float    m_d[2];
+    unsigned long long m_acc[2];
+    uint32_t err;                     // OOK_ERR_* bits, sticky until reset
+};
+constexpr uint32_t OOK_ERR_CARRY = 1u, OOK_ERR_RUNS = 2u, OOK_ERR_BURSTS = 4u;
+constexpr int32_t OOK_TAG_OPEN = -2;  // stream plans: a block collected into the burst still open at the end of the push
+
+static OokSeam ook_seam_initial()
+{
+    OokSeam z;
+    memset(&z, 0, sizeof(z));
+    z.buf_len = 1; z.low2 = 1; z.lead0 = 1;   // sample_buffer = vec!(0.0) (:43); 0 - 1 < 0 on the first block
+    return z;
+}
+
+// the carry region [stream][cpitch] in front of a push's blocks [stream][n_blocks] form one virtual row per stream, read in place
+struct OokCarry {
+    size_t          cpitch;           // slots per stream (a multiple of 32: a group of 32 is all carry or all push)
+    const uint8_t  *bytes;            // [stream][cpitch][1024]
+    const float    *bmax;             // [stream][cpitch] block maxima
+    const uint32_t *live;             // [stream] carried blocks that belong to a burst sent in this push (0 otherwise)
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -421,10 +470,13 @@ constexpr int KB_THREADS = 2 * KB_STREAMS + KB_HELPERS;
 constexpr int KB_TILE = 32;                   // blocks per staged tile
 constexpr int KB_LD = KB_TILE + 1;            // conflict-free both ways: helpers move rows, the walker reads columns
 
+// STREAM (stream plans): the walker and the keeper start from the stream's OokSeam and store it back after the last block, and the
+// burst still open at the end is tagged OOK_TAG_OPEN (for ook_carry_kernel) instead of un-tagged.
+template <bool STREAM>
 __global__ void __launch_bounds__(KB_THREADS)
 ook_trigger_kernel(const float *__restrict__ d_sum, size_t n_streams, size_t n_blocks, size_t max_bursts, uint32_t guard_samples,
                    int32_t *__restrict__ d_tag, uint32_t *__restrict__ d_bend, uint8_t *__restrict__ d_bflags,
-                   uint32_t *__restrict__ d_nbursts)
+                   uint32_t *__restrict__ d_nbursts, OokSeam *__restrict__ seam)
 {
     __shared__ float s_sum[4][KB_STREAMS * KB_LD];        // tile t in buffer t & 3: copies run two tiles ahead of the divisions
     __shared__ float s_q[2][KB_STREAMS * KB_LD];
@@ -512,6 +564,13 @@ ook_trigger_kernel(const float *__restrict__ d_sum, size_t n_streams, size_t n_b
     bool lead0 = true;                        // the buffer currently starts with that 0.0
     uint32_t burst = 0;                       // index of the burst being collected
     bool dropped = false;                     // the OOM guard abandoned a burst of this stream
+    // the walker's state after the last block of the push (the walk goes on over the padding of a ragged last tile)
+    int sv_trigger = 0; float sv_threshold = 0.0f; bool sv_fired = false, sv_low2 = true;
+    if (STREAM && live) {
+        const OokSeam &z = seam[st];
+        trigger = z.trig; threshold = z.threshold; fired = z.fired != 0; low2 = z.low2 != 0;
+        buf_len = z.buf_len; lead0 = z.lead0 != 0;
+    }
     if (helper) {
         stage(0);
         stage(1);
@@ -574,6 +633,9 @@ ook_trigger_kernel(const float *__restrict__ d_sum, size_t n_streams, size_t n_b
                         // what the book-keeping needs of the counter: collect (:73) and send (:78)
                         c8 |= (trigger > 1 ? 1u : 0u) << k;
                         s8 |= (trigger == 0 ? 1u : 0u) << k;
+                        if (STREAM && u0 + k == nb - 1 && tile == n_tiles - 1) {     // off the chain: selects only
+                            sv_trigger = trigger; sv_threshold = threshold; sv_fired = fired; sv_low2 = low2;
+                        }
                     }
                     cm |= c8 << u0;
                     sm |= s8 << u0;
@@ -647,6 +709,14 @@ ook_trigger_kernel(const float *__restrict__ d_sum, size_t n_streams, size_t n_b
     if (keeper && live) {                                             // [32] guard fired -- s_q is free after the last tile
         if (burst < max_bursts) flags[burst] = 0;
         d_nbursts[st] = burst;                // may exceed max_bursts -> reported by fetch
+        if (STREAM) {
+            seam[st].buf_len = buf_len; seam[st].lead0 = lead0 ? 1 : 0;
+            if (burst >= max_bursts) seam[st].err |= OOK_ERR_BURSTS;  // the open burst's blocks could not be tagged
+        }
+    }
+    if (STREAM && walker && live) {
+        seam[st].trig = sv_trigger < -1 ? -1 : sv_trigger; seam[st].threshold = sv_threshold;
+        seam[st].fired = sv_fired ? 1 : 0; seam[st].low2 = sv_low2 ? 1 : 0;
     }
     __syncthreads();                          // all tags are in global memory, s_q is no longer read
     if (keeper) {
@@ -656,7 +726,7 @@ ook_trigger_kernel(const float *__restrict__ d_sum, size_t n_streams, size_t n_b
     }
     __syncthreads();
     // The unsent burst's blocks end within the last two blocks of the capture (it is still being collected, or the counter just
-    // reached 1) and lie at most one block apart.  The warps share the streams out (warp w: streams w, w + 14, w + 28): the last 64
+    // reached 1) and lie at most one block apart.  A stream plan tags them OOK_TAG_OPEN: ook_carry_kernel appends them to the carry.  The warps share the streams out (warp w: streams w, w + 14, w + 28): the last 64
     // tags of a warp's streams are loaded first (independent loads, one latency), matched and cleared; a run longer than that
     // (rare) is followed backwards chunk by chunk.
     {
@@ -681,8 +751,9 @@ ook_trigger_kernel(const float *__restrict__ d_sum, size_t n_streams, size_t n_b
             const int32_t bidx = (int32_t)s_open[32 + r];
             const long long k0 = (long long)n_blocks - 1 - lane, k1 = k0 - 32;
             const bool m0 = t0[j] == bidx, m1 = t1[j] == bidx;
-            if (m0) tag[k0] = -1;
-            if (m1) tag[k1] = -1;
+            const int32_t untag = STREAM ? OOK_TAG_OPEN : -1;
+            if (m0) tag[k0] = untag;
+            if (m1) tag[k1] = untag;
             // the burst reaches past the 64 tags: keep going while a chunk of 32 still holds one of its blocks (a burst may skip
             // single blocks -- the block at counter 1 is not collected, a re-fire on the next one continues the burst -- so a
             // chunk without any of its blocks is the end)
@@ -690,7 +761,7 @@ ook_trigger_kernel(const float *__restrict__ d_sum, size_t n_streams, size_t n_b
             bool more = __any_sync(0xffffffffu, m1);
             while (more && __any_sync(0xffffffffu, k >= 0)) {
                 const bool m = k >= 0 && tag[k] == bidx;
-                if (m) tag[k] = -1;
+                if (m) tag[k] = untag;
                 more = __any_sync(0xffffffffu, m);
                 k -= 32;
             }
@@ -972,12 +1043,16 @@ __device__ __forceinline__ uint32_t kc_inner_transitions(uint32_t m, int lane)
 // max) -- order-free, so the per-block maxima of the blocks that carry its tag can be reduced in any order), max/2 (:91), and that
 // threshold in the rank domain  #{distinct envelope values <= max/2}  (see ook_rle_kernel).  The burst's blocks lie between the
 // block that ended the previous burst and the one that ended this one (d_bend).
+// Stream plans (STREAM): burst 0 is the one that was open when the push started; its carried blocks' running maximum is folded
+// in, and the carried blocks take part in this push's slicing (live = their number) only if it is sent here.
 constexpr int KC0_WARPS = 8;
+template <bool STREAM>
 __global__ void __launch_bounds__(KC0_WARPS * 32)
 ook_burst_kernel(size_t n_streams, size_t n_blocks, size_t max_bursts, const float *__restrict__ d_max,
                  const int32_t *__restrict__ d_tag, const uint32_t *__restrict__ d_bend, const uint8_t *__restrict__ d_bflags,
                  const uint32_t *__restrict__ d_nbursts, const float *__restrict__ uniq, uint32_t n_uniq,
-                 float *__restrict__ d_half, uint32_t *__restrict__ d_hrank, uint32_t *__restrict__ d_next, uint32_t next_init)
+                 float *__restrict__ d_half, uint32_t *__restrict__ d_hrank, uint32_t *__restrict__ d_next, uint32_t next_init,
+                 const OokSeam *__restrict__ seam, uint32_t *__restrict__ d_live)
 {
     const int lane = threadIdx.x & 31;
     const size_t w = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -986,8 +1061,10 @@ ook_burst_kernel(size_t n_streams, size_t n_blocks, size_t max_bursts, const flo
     const size_t st = w / max_bursts, j = w % max_bursts;
     const uint32_t nbu = d_nbursts[st], fl = d_bflags[w];                // independent loads: one latency (slots past the stream's
     const uint32_t hi = d_bend[w], lo = j ? d_bend[w - 1] + 1u : 0u;     // last burst hold stale values, never used)
-    if (j >= nbu || !(fl & 1u)) return;                                  // never sent: no block carries its index
-    float mx = 0.0f;
+    const bool sent = j < nbu && (fl & 1u);
+    if (STREAM && j == 0 && lane == 0) d_live[st] = sent ? seam[st].n_carry : 0u;
+    if (!sent) return;                                                   // never sent: no block carries its index
+    float mx = STREAM && j == 0 ? seam[st].run_max : 0.0f;
     const size_t end = (size_t)hi + 1 < n_blocks ? (size_t)hi + 1 : n_blocks;
     for (size_t b0 = lo; b0 < end; b0 += 128) {                          // 128 blocks per step, all loads independent: one latency
         int32_t tg[4]; float v[4];
@@ -1009,11 +1086,12 @@ ook_burst_kernel(size_t n_streams, size_t n_blocks, size_t max_bursts, const flo
     if (lane == 0) { d_half[w] = hv; d_hrank[w] = h; }
 }
 
+template <bool STREAM>
 __global__ void __launch_bounds__(KC1_WARPS * 32, 1)
 ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_streams, size_t n_blocks, size_t max_bursts,
                  const uint16_t *__restrict__ g_rank, const int32_t *__restrict__ d_tag, const uint32_t *__restrict__ d_hrank,
                  const float *__restrict__ d_half, const float *__restrict__ d_max,
-                 uint32_t *__restrict__ d_next, uint16_t *__restrict__ d_mask, uint32_t *__restrict__ d_bsum)
+                 uint32_t *__restrict__ d_next, uint16_t *__restrict__ d_mask, uint32_t *__restrict__ d_bsum, OokCarry carry)
 {
     extern __shared__ __align__(16) uint16_t kc_rank[];
     for (int i = threadIdx.x; i < OOK_RANK_BYTES / 16; i += blockDim.x)
@@ -1023,7 +1101,9 @@ ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_
     // leaves out the divergence guards (BRA.DIV / WARPSYNC.COLLECTIVE) it put around every vote and shuffle of the loop
     const int lane = threadIdx.x & 31, warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
     const uint32_t rank_s = smem_u32(kc_rank);
-    const size_t groups_per_stream = (n_blocks + 31) / 32;
+    // a stream's row: carry.cpitch carried slots, then the push's blocks (a batch plan has no carry)
+    const size_t cp = STREAM ? carry.cpitch : 0, row = cp + n_blocks;
+    const size_t groups_per_stream = (row + 31) / 32;
     const size_t n_groups = groups_per_stream * n_streams;
     const size_t warps_total = (size_t)gridDim.x * KC1_WARPS;
     constexpr int PF = 2;
@@ -1039,7 +1119,8 @@ ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_
     auto tag_of = [&](uint32_t g) -> int32_t {
         if (g >= ng) return -1;
         const size_t b = (size_t)(g % gps) * 32 + lane;
-        return b < n_blocks ? d_tag[(size_t)(g / gps) * n_blocks + b] : -1;
+        if (STREAM && b < cp) return b < carry.live[g / gps] ? 0 : -1;                            // carried blocks belong to burst 0
+        return b - cp < n_blocks ? d_tag[(size_t)(g / gps) * n_blocks + b - cp] : -1;
     };
     auto thr_of = [&](uint32_t g, int32_t tg) -> uint32_t {
         return tg >= 0 ? d_hrank[(size_t)(g / gps) * max_bursts + tg] - 1u : 0u;           // rank >= h  <=>  (h - 1) - rank < 0
@@ -1047,8 +1128,9 @@ ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_
     // quiet block (see ook_rle_kernel): its maximum does not exceed the burst's max/2, it slices to 512 zeros without being read
     auto quiet_of = [&](uint32_t g, int32_t tg) -> bool {
         if (tg < 0) return false;
-        const size_t st = g / gps;
-        return d_max[st * n_blocks + (size_t)(g % gps) * 32 + lane] <= d_half[st * max_bursts + tg];
+        const size_t st = g / gps, b = (size_t)(g % gps) * 32 + lane;
+        const float bm = STREAM && b < cp ? carry.bmax[st * cp + b] : d_max[st * n_blocks + b - cp];
+        return bm <= d_half[st * max_bursts + tg];
     };
     const uint32_t wt = (uint32_t)warps_total;
     uint32_t g0 = blockIdx.x * KC1_WARPS + warp, g1 = g0 + wt, g2 = g1 + wt;
@@ -1062,10 +1144,11 @@ ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_
         const bool q_n1 = quiet_of(g1, tg_n1);
         const int32_t tg_n2 = tag_of(g2);
         const size_t st = g0 / gps, b0 = (size_t)(g0 % gps) * 32;
-        if (tg_l >= 0 && q_l) d_bsum[st * n_blocks + b0 + lane] = 0u;      // quiet: no transition inside, first and last bit 0
+        if (tg_l >= 0 && q_l) d_bsum[st * row + b0 + lane] = 0u;           // quiet: no transition inside, first and last bit 0
         unsigned rem = __ballot_sync(0xffffffffu, tg_l >= 0 && !q_l);
         if (rem != 0u) {
-            const uint8_t *base = iq + st * stream_stride + b0 * (size_t)(OOK_BLOCK * 2);
+            const uint8_t *base = STREAM && b0 < cp ? carry.bytes + (st * cp + b0) * (size_t)(OOK_BLOCK * 2)
+                                          : iq + st * stream_stride + (b0 - cp) * (size_t)(OOK_BLOCK * 2);
             int kA[PF], kB[PF];
             uint4 dA[PF][2], dB[PF][2];
             auto take = [&](int (&ks)[PF], uint4 (&d)[PF][2]) {
@@ -1080,8 +1163,8 @@ ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_
                 }
             };
             // the group's rows of the two outputs: a block adds its index
-            uint16_t *mask_g = d_mask + (st * n_blocks + b0) * 32 + lane;
-            uint32_t *bsum_g = d_bsum + st * n_blocks + b0;
+            uint16_t *mask_g = d_mask + (st * row + b0) * 32 + lane;
+            uint32_t *bsum_g = d_bsum + st * row + b0;
             auto slice = [&](const int (&ks)[PF], const uint4 (&d)[PF][2]) {
 #pragma unroll
                 for (int i = 0; i < PF; ++i) {
@@ -1123,19 +1206,21 @@ ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_
 constexpr uint32_t KC_INFO_PRE = 1u, KC_INFO_FIRST = 2u;
 constexpr int KC2_WARPS = 4;
 
+template <bool STREAM>
 __global__ void __launch_bounds__(KC2_WARPS * 32)
 ook_scan_kernel(size_t n_streams, size_t n_blocks, size_t max_bursts, size_t max_runs, const int32_t *__restrict__ d_tag,
                 const uint32_t *__restrict__ d_bsum, const uint8_t *__restrict__ d_bflags, const uint32_t *__restrict__ d_nbursts,
                 uint4 *__restrict__ d_binfo, uint32_t *__restrict__ d_trans, uint32_t *__restrict__ d_ntrans,
-                uint32_t *__restrict__ d_nbits)
+                uint32_t *__restrict__ d_nbits, OokCarry carry, OokSeam *__restrict__ seam)
 {
     const int lane = threadIdx.x & 31;
     const size_t st = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (st >= n_streams) return;
+    const size_t cp = STREAM ? carry.cpitch : 0, row = cp + n_blocks;
     const int32_t *tag = d_tag + st * n_blocks;
-    const uint32_t *bsum = d_bsum + st * n_blocks;
+    const uint32_t *bsum = d_bsum + st * row;
     const uint8_t *flags = d_bflags + st * max_bursts;
-    uint4 *binfo = d_binfo + st * n_blocks;
+    uint4 *binfo = d_binfo + st * row;
     // bursts that were sent without a collected block (the OOM guard reset the buffer to [0.0] with the counter at 1, :52-54 and
     // :78-81): one 0 bit each, found among the burst indices the walk steps over (flags == 3: sent, leading 0.0)
     auto lone_zero_bursts = [&](int32_t from, int32_t to) {
@@ -1144,19 +1229,26 @@ ook_scan_kernel(size_t n_streams, size_t n_blocks, size_t max_bursts, size_t max
         return n;
     };
     uint32_t pos = 0, ntr = 0, prev = 0;          // the walk's carry: bits so far, transitions so far, value of the last bit
+    // a stream plan's bit positions count from the start of the push; `any`: bits were emitted before it (the value of the last one
+    // is `prev`), so the push's very first bit may be a transition
+    const bool any = STREAM && seam[st].any;
+    if (any) prev = seam[st].prev;
     int32_t cur_burst = -1;
     constexpr int CH = 4;                         // groups whose tags and summaries are fetched together (one latency per 128 blocks)
-    for (size_t c0 = 0; c0 < n_blocks; c0 += 32 * CH) {
+    // the row: the carried blocks of a burst sent in this push (all of burst 0), then the push's blocks
+    const size_t live = STREAM ? carry.live[st] : 0;
+    // one step: 32 x CH blocks of the row from c0 (row positions below hi); carried blocks all belong to burst 0
+    auto step = [&](size_t c0, size_t hi, bool carried) {
         int32_t tgs[CH]; uint32_t sms[CH];
 #pragma unroll
         for (int c = 0; c < CH; ++c) {
             const size_t b = c0 + 32 * c + lane;
-            tgs[c] = b < n_blocks ? tag[b] : -1;
+            tgs[c] = b < hi ? (carried ? 0 : tag[b - cp]) : -1;
         }
 #pragma unroll
         for (int c = 0; c < CH; ++c) {
             const size_t b = c0 + 32 * c + lane;
-            sms[c] = b < n_blocks ? bsum[b] : 0u;          // not behind the tag's latency; only read where the block is collected
+            sms[c] = b < hi ? bsum[b] : 0u;                // not behind the tag's latency; only read where the block is collected
         }
 #pragma unroll
         for (int c = 0; c < CH; ++c) {
@@ -1186,8 +1278,8 @@ ook_scan_kernel(size_t n_streams, size_t n_blocks, size_t max_bursts, size_t max
             const uint32_t pos_ins = pos + incl - bits;                    // where the inserted zeros start
             const uint32_t pos_base = pos_ins + n_ins;                     // the block's first bit
             const uint32_t before = n_ins ? 0u : plast;                    // value of the bit before it
-            const bool pre = col && n_ins && pos_ins > 0u && plast != 0u;  // 1 -> 0 at the first inserted zero
-            const bool firstT = col && pos_base > 0u && first != before;
+            const bool pre = col && n_ins && (pos_ins > 0u || any) && plast != 0u;   // 1 -> 0 at the first inserted zero
+            const bool firstT = col && (pos_base > 0u || any) && first != before;
             const uint32_t mine = col ? cnt + (pre ? 1u : 0u) + (firstT ? 1u : 0u) : 0u;
             uint32_t tincl = mine;
 #pragma unroll
@@ -1204,16 +1296,23 @@ ook_scan_kernel(size_t n_streams, size_t n_blocks, size_t max_bursts, size_t max
             cur_burst = __shfl_sync(0xffffffffu, tg, lastc);
             prev = __shfl_sync(0xffffffffu, last, lastc);
         }
-    }
+    };
+    if constexpr (STREAM)
+        for (size_t c0 = 0; c0 < live; c0 += 32 * CH) step(c0, live, true);
+    for (size_t c0 = cp; c0 < row; c0 += 32 * CH) step(c0, row, false);
     {   // lone [0.0] bursts after the last collected block
         const uint32_t nbu = d_nbursts[st];
         const uint32_t n = lone_zero_bursts(cur_burst + 1, (int32_t)(nbu < max_bursts ? nbu : max_bursts));
         if (n) {
-            if (pos > 0u && prev != 0u) { if (lane == 0 && ntr < max_runs) d_trans[st * max_runs + ntr] = pos; ntr++; }
+            if ((pos > 0u || any) && prev != 0u) { if (lane == 0 && ntr < max_runs) d_trans[st * max_runs + ntr] = pos; ntr++; }
             pos += n;
+            prev = 0u;
         }
     }
-    if (lane == 0) { d_ntrans[st] = ntr; d_nbits[st] = pos; }
+    if (lane == 0) {
+        d_ntrans[st] = ntr; d_nbits[st] = pos;
+        if (STREAM && pos > 0u) { seam[st].prev = prev; seam[st].any = 1u; }
+    }
 }
 
 constexpr int KC3_WARPS = 8;
@@ -1221,20 +1320,22 @@ constexpr int KC3_WARPS = 8;
 // C3: lane l of a warp owns block l of a (stream, group): its transitions go to consecutive entries of the list starting at the
 // index C2 gave it, so no lane needs another's count -- the blocks of a group are written side by side, each lane fetching the 64
 // bytes of its own mask in one go
+template <bool STREAM>
 __global__ void __launch_bounds__(KC3_WARPS * 32)
 ook_scatter_kernel(size_t n_streams, size_t n_blocks, size_t max_runs, const int32_t *__restrict__ d_tag,
                    const uint32_t *__restrict__ d_bsum, const uint4 *__restrict__ d_binfo, const uint16_t *__restrict__ d_mask,
-                   uint32_t *__restrict__ d_trans)
+                   uint32_t *__restrict__ d_trans, OokCarry carry)
 {
     const int lane = threadIdx.x & 31;
-    const size_t groups_per_stream = (n_blocks + 31) / 32;
+    const size_t cp = STREAM ? carry.cpitch : 0, row = cp + n_blocks;
+    const size_t groups_per_stream = (row + 31) / 32;
     const size_t n_groups = groups_per_stream * n_streams;
     const size_t grp = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (grp >= n_groups) return;
-    const size_t st = grp / groups_per_stream, b0 = (grp % groups_per_stream) * 32;
-    if (b0 + lane >= n_blocks) return;
-    const size_t blk = st * n_blocks + b0 + lane;
-    if (d_tag[blk] < 0) return;
+    const size_t st = grp / groups_per_stream, b = (grp % groups_per_stream) * 32 + lane;
+    if (b >= row) return;
+    if (STREAM && b < cp ? b >= carry.live[st] : d_tag[st * n_blocks + b - cp] < 0) return;
+    const size_t blk = st * row + b;
     const uint32_t sm = d_bsum[blk];
     const uint4 info = d_binfo[blk];
     uint32_t *trans = d_trans + st * max_runs;
@@ -1280,7 +1381,7 @@ struct Matcher {
     float a1lo, a1hi, a2lo, a2hi, s1lo, s1hi, s2lo, s2hi;
     bool  proto_b;
     bool  pending; float d;
-    unsigned long long acc; uint32_t n, want, count;
+    unsigned long long acc; uint32_t n, want, count, base;      // out[k] holds packet base + k
     unsigned long long *out; size_t cap;
     __device__ __forceinline__ void init(int proto, unsigned long long *o, size_t c)
     {
@@ -1289,7 +1390,15 @@ struct Matcher {
         a2lo = proto_b ? 500e-6f : 1.0f;   a2hi = proto_b ? 650e-6f : 0.0f;                  // (A has no second range: empty)
         s1lo = proto_b ? 500e-6f : 1.5e-3f; s1hi = proto_b ? 650e-6f : 2.5e-3f;              // second run
         s2lo = proto_b ? 125e-6f : 3.5e-3f; s2hi = proto_b ? 250e-6f : 4.5e-3f;
-        pending = false; d = 0.0f; acc = 0ull; n = 0u; want = proto_b ? 24u : 36u; count = 0u; out = o; cap = c;
+        pending = false; d = 0.0f; acc = 0ull; n = 0u; want = proto_b ? 24u : 36u; count = 0u; base = 0u; out = o; cap = c;
+    }
+    __device__ __forceinline__ void load(const OokSeam &z, int p, uint32_t b)
+    {
+        pending = z.m_pending[p] != 0; d = z.m_d[p]; acc = z.m_acc[p]; n = z.m_n[p]; count = z.m_count[p]; base = b;
+    }
+    __device__ __forceinline__ void store(OokSeam &z, int p) const
+    {
+        z.m_pending[p] = pending ? 1u : 0u; z.m_d[p] = d; z.m_acc[p] = acc; z.m_n[p] = n; z.m_count[p] = count;
     }
     __device__ __forceinline__ void feed(uint32_t v, float dur)
     {
@@ -1307,7 +1416,7 @@ struct Matcher {
         n += push ? 1u : 0u;
         // None if x.len() == l => send; None => clear
         if (none) {
-            if (n == want) { if (count < cap) out[count] = acc; count++; }
+            if (n == want) { if (count - base < cap) out[count - base] = acc; count++; }
             n = 0u; acc = 0ull;
         }
     }
@@ -1316,39 +1425,127 @@ struct Matcher {
 // One warp per stream.  Run lengths -> seconds (dle) is data-parallel: the lanes turn a chunk of 256
 // transitions into durations in shared memory with coalesced reads; the matchers are sequential, so lane 0
 // (proto A) and lane 1 (proto B) then walk the chunk from shared memory instead of chasing global loads.
+// Stream plans (STREAM): the first run of the push continues the open run carried from the pushes before, the matchers
+// resume where they stopped, packets are numbered on from there and stored from d_pbase (the first one not fetched yet).
 constexpr int KD_WARPS = 4, KD_CHUNK = 256;
 
+template <bool STREAM>
 __global__ void __launch_bounds__(KD_WARPS * 32)
 ook_match_kernel(const uint32_t *__restrict__ d_trans, const uint32_t *__restrict__ d_ntrans, size_t n_streams,
                  size_t max_runs, size_t max_packets, float s_rate_f, unsigned long long *__restrict__ d_packets,
-                 uint32_t *__restrict__ d_npackets, uint32_t *__restrict__ d_runs_dbg)
+                 uint32_t *__restrict__ d_npackets, uint32_t *__restrict__ d_runs_dbg,
+                 OokSeam *__restrict__ seam, const uint32_t *__restrict__ d_nbits, const uint32_t *__restrict__ d_pbase)
 {
     __shared__ float s_dur[KD_WARPS][KD_CHUNK];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const size_t st = (size_t)blockIdx.x * KD_WARPS + warp;
     if (st >= n_streams) return;
     const uint32_t *tr = d_trans + st * max_runs;
-    uint32_t nr = d_ntrans[st];
+    const uint32_t nr_all = d_ntrans[st];
+    uint32_t nr = nr_all;
     if (nr > max_runs) nr = (uint32_t)max_runs;           // overflow is reported by fetch
-    // run k: value = k & 1 (the stream starts with the 0 bit of vec!(0.0)), length = tr[k] - tr[k-1]
+    // run k: value = (v0 + k) & 1, length = tr[k] - tr[k-1]; the stream starts with the 0 bit of vec!(0.0), so v0 = 0 from the
+    // initial state; the first run of a push adds the length the open run had reached before it
+    const unsigned long long len0 = STREAM ? seam[st].run_len : 0ull;
+    const uint32_t v0 = STREAM ? seam[st].run_val : 0u;
     uint32_t *dbg = d_runs_dbg + st * max_runs;
     Matcher mt;
     mt.init(lane & 1, d_packets + (st * 2 + (lane & 1)) * max_packets, max_packets);
+    if (STREAM && lane < 2) mt.load(seam[st], lane, d_pbase[st * 2 + lane]);
     float *dur = s_dur[warp];
     for (uint32_t k0 = 0; k0 < nr; k0 += KD_CHUNK) {
         const uint32_t nk = nr - k0 < (uint32_t)KD_CHUNK ? nr - k0 : (uint32_t)KD_CHUNK;
         for (uint32_t i = lane; i < nk; i += 32) {
             const uint32_t k = k0 + i;
             const uint32_t len = tr[k] - (k ? tr[k - 1] : 0u);
-            dbg[k] = ((k & 1u) << 31) | len;
-            dur[i] = __fdiv_rn((float)len, s_rate_f);                                   // dle kpn.rs:35
+            const uint32_t v = (v0 + k) & 1u;
+            if (k == 0 && len0) {
+                const unsigned long long l = len0 + len;
+                dbg[k] = (v << 31) | (uint32_t)(l < 0x7fffffffull ? l : 0x7fffffffull);
+                dur[i] = __fdiv_rn(__ull2float_rn(l), s_rate_f);                         // dle kpn.rs:35 (ct as f32)
+            } else {
+                dbg[k] = (v << 31) | len;
+                dur[i] = __fdiv_rn((float)len, s_rate_f);                               // dle kpn.rs:35
+            }
         }
         __syncwarp();
         if (lane < 2)
-            for (uint32_t i = 0; i < nk; ++i) mt.feed((k0 + i) & 1u, dur[i]);
+            for (uint32_t i = 0; i < nk; ++i) mt.feed((v0 + k0 + i) & 1u, dur[i]);
         __syncwarp();
     }
     if (lane < 2) d_npackets[st * 2 + lane] = mt.count;
+    if (STREAM) {
+        if (lane < 2) mt.store(seam[st], lane);
+        if (lane == 0) {
+            const uint32_t nbits = d_nbits[st];
+            OokSeam &z = seam[st];
+            if (nr == 0) z.run_len = len0 + nbits;
+            else { z.run_len = nbits - tr[nr - 1]; z.run_val = (v0 + nr) & 1u; }
+            if (nr_all > max_runs) z.err |= OOK_ERR_RUNS;
+        }
+    }
+}
+
+// Stream plans, after the slicer: the blocks of the burst still open at the end of the push (tagged OOK_TAG_OPEN by the trigger
+// kernel) are appended to the stream's carry region with their maxima.  discretize (bitfount.rs:87-96) needs the burst's maximum
+// before its first bit, so they are sliced in the push that sends the burst, read in place from here.  If no burst was sent or
+// dropped in this push (d_nbursts = 0) the open burst is the one carried in and they go after its blocks; otherwise the carry
+// starts over.  One warp per stream copies four blocks at a time (32 bytes per lane per block).
+constexpr int KCY_WARPS = 4;
+__global__ void __launch_bounds__(KCY_WARPS * 32)
+ook_carry_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_streams, size_t n_blocks, size_t cpitch,
+                 size_t max_carry, const int32_t *__restrict__ d_tag, const float *__restrict__ d_max,
+                 const uint32_t *__restrict__ d_nbursts, uint8_t *__restrict__ d_carry, float *__restrict__ d_cmax,
+                 OokSeam *__restrict__ seam)
+{
+    const int lane = threadIdx.x & 31;
+    const size_t st = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (st >= n_streams) return;
+    const bool cont = d_nbursts[st] == 0u;
+    size_t n = cont ? seam[st].n_carry : 0u;
+    float mx = cont ? seam[st].run_max : 0.0f;
+    const int32_t *tag = d_tag + st * n_blocks;
+    const float *bmax = d_max + st * n_blocks;
+    const uint8_t *src = iq + st * stream_stride + lane * 32;
+    uint8_t *dst = d_carry + st * cpitch * (size_t)(OOK_BLOCK * 2) + lane * 32;
+    float *cmax = d_cmax + st * cpitch;
+    for (size_t b0 = 0; b0 < n_blocks; b0 += 32) {
+        const size_t b = b0 + lane;
+        const bool open = b < n_blocks && tag[b] == OOK_TAG_OPEN;
+        unsigned rem = __ballot_sync(0xffffffffu, open);
+        if (!rem) continue;                                                      // warp-uniform
+        const float bm = open ? bmax[b] : 0.0f;
+        mx = fmaxf(mx, bm);
+        if (open && n + __popc(rem & ((1u << lane) - 1u)) < max_carry) cmax[n + __popc(rem & ((1u << lane) - 1u))] = bm;
+        while (rem) {
+            int k[4]; uint4 v[4][2];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                k[i] = rem ? __ffs(rem) - 1 : -1;
+                if (rem) rem &= rem - 1u;
+                if (k[i] >= 0 && n + i < max_carry) {
+                    const uint4 *p = reinterpret_cast<const uint4 *>(src + (b0 + k[i]) * (size_t)(OOK_BLOCK * 2));
+                    v[i][0] = ldg_stream_u4(p); v[i][1] = ldg_stream_u4(p + 1);
+                }
+            }
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                if (k[i] < 0) break;
+                if (n < max_carry) {
+                    uint4 *q = reinterpret_cast<uint4 *>(dst + n * (size_t)(OOK_BLOCK * 2));
+                    q[0] = v[i][0]; q[1] = v[i][1];
+                }
+                ++n;
+            }
+        }
+    }
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+    if (lane == 0) {
+        if (n > max_carry) { seam[st].err |= OOK_ERR_CARRY; n = max_carry; }
+        seam[st].n_carry = (uint32_t)n;
+        seam[st].run_max = mx;
+    }
 }
 
 __global__ void ook_envelope_table_kernel(float *__restrict__ table)
@@ -1360,17 +1557,19 @@ __global__ void ook_envelope_table_kernel(float *__restrict__ table)
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-extern "C" int lrc_ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, unsigned sample_rate,
-                              size_t max_runs, size_t max_packets, lrc_ook **out)
+// cpitch: carry slots per stream in front of the blocks of the slicer's per-block arrays (stream plans; 0 for a batch plan)
+static int ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, size_t cpitch, unsigned sample_rate,
+                      size_t max_runs, size_t max_packets, lrc_ook **out)
 {
     LRC_BIND(ctx);
     LRC_REQUIRE(out && n_streams >= 1 && n_blocks >= 1 && sample_rate >= 1, LRC_ERR_INVALID, "lrc_ook_create: bad arguments");
     LRC_REQUIRE(n_blocks * (size_t)OOK_BLOCK < 0xffffffffull, LRC_ERR_UNSUPPORTED, "lrc_ook_create: capture too long (2^32 samples)");
-    LRC_REQUIRE(n_streams * ((n_blocks + 31) / 32) < 0x7fffffffull, LRC_ERR_UNSUPPORTED, "lrc_ook_create: too many 32-block groups (2^31)");
+    LRC_REQUIRE(n_streams * ((cpitch + n_blocks + 31) / 32) < 0x7fffffffull, LRC_ERR_UNSUPPORTED,
+                "lrc_ook_create: too many 32-block groups (2^31)");
     lrc_ook *o = new (std::nothrow) lrc_ook();
     LRC_REQUIRE(o != nullptr, LRC_ERR_NOMEM, "out of host memory");
     memset(o, 0, sizeof(*o));
-    o->ctx = ctx; o->n_streams = n_streams; o->n_blocks = n_blocks; o->sample_rate = sample_rate;
+    o->ctx = ctx; o->n_streams = n_streams; o->n_blocks = n_blocks; o->sample_rate = sample_rate; o->cpitch = cpitch;
     o->max_runs = max_runs ? max_runs : 4096;
     o->max_packets = max_packets ? max_packets : 64;
     // bitfount.rs:52 `1000*trigger_duration*block_size`.  LRC_OOK_TEST_GUARD_BLOCKS shrinks it (in blocks) so that a test can reach
@@ -1381,8 +1580,9 @@ extern "C" int lrc_ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, u
     // a sent burst is at least 49 collected blocks, except the pieces the guard cuts one into (an abandoned burst of more than
     // guard_blocks blocks followed by its remainder, possibly empty): at least guard_blocks / 2 blocks per index on average
     const size_t min_burst = std::min<size_t>(49, std::max<size_t>(1, guard_blocks / 2));
-    o->max_bursts = n_blocks / min_burst + 2;
-    const size_t sb = n_streams * n_blocks;
+    // (+ 1 for a stream plan: the burst carried in may be dropped by the guard, and a lone [0.0] sent, within two blocks)
+    o->max_bursts = n_blocks / min_burst + 2 + (cpitch ? 1 : 0);
+    const size_t sb = n_streams * n_blocks, sr = n_streams * (cpitch + n_blocks);
     cudaError_t e = cudaSuccess;
 #define OOK_ALLOC(ptr, count) if (e == cudaSuccess) e = cudaMalloc(&o->ptr, (count) * sizeof(*o->ptr))
     OOK_ALLOC(d_sum, sb); OOK_ALLOC(d_max, sb); OOK_ALLOC(d_tag, sb);
@@ -1392,7 +1592,7 @@ extern "C" int lrc_ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, u
     OOK_ALLOC(d_trans, n_streams * o->max_runs); OOK_ALLOC(d_ntrans, n_streams); OOK_ALLOC(d_nbits, n_streams);
     OOK_ALLOC(d_packets, n_streams * 2 * o->max_packets); OOK_ALLOC(d_npackets, n_streams * 2);
     OOK_ALLOC(d_runs_dbg, n_streams * o->max_runs);
-    OOK_ALLOC(d_mask, sb * 32); OOK_ALLOC(d_bsum, sb); OOK_ALLOC(d_binfo, sb); OOK_ALLOC(d_hrank, n_streams * o->max_bursts); OOK_ALLOC(d_next, 1);
+    OOK_ALLOC(d_mask, sr * 32); OOK_ALLOC(d_bsum, sr); OOK_ALLOC(d_binfo, sr); OOK_ALLOC(d_hrank, n_streams * o->max_bursts); OOK_ALLOC(d_next, 1);
     OOK_ALLOC(d_lut, (size_t)OOK_LUT_N);
     OOK_ALLOC(d_flut, (size_t)OOK_FLUT_N);
     OOK_ALLOC(d_rank, (size_t)OOK_RANK_N); OOK_ALLOC(d_uniq, (size_t)65536);
@@ -1421,7 +1621,8 @@ extern "C" int lrc_ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, u
             }
         }
         if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_rle_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, OOK_RANK_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_slice_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, OOK_RANK_BYTES);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_slice_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, OOK_RANK_BYTES);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_slice_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, OOK_RANK_BYTES);
     }
     if (e == cudaSuccess) {
         // rank table for the slicer: the envelope of every byte pair, computed ON THE DEVICE by the routine the
@@ -1453,6 +1654,12 @@ extern "C" int lrc_ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, u
     return LRC_OK;
 }
 
+extern "C" int lrc_ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, unsigned sample_rate,
+                              size_t max_runs, size_t max_packets, lrc_ook **out)
+{
+    return ook_create(ctx, n_streams, n_blocks, 0, sample_rate, max_runs, max_packets, out);
+}
+
 extern "C" int lrc_ook_destroy(lrc_ook *o)
 {
     if (!o) return LRC_OK;
@@ -1465,16 +1672,23 @@ extern "C" int lrc_ook_destroy(lrc_ook *o)
     return LRC_OK;
 }
 
-extern "C" int lrc_ook_decode(lrc_ook *o, const uint8_t *d_iq, size_t stream_stride_bytes, void *stream)
+// what a stream plan adds to a launch of the chain (null: a batch plan, every stream from the initial state)
+struct OokStreamLaunch {
+    OokSeam  *seam;
+    OokCarry  carry;
+    uint8_t  *d_carry;
+    float    *d_cmax;
+    uint32_t *d_live, *d_pbase;
+    size_t    max_carry;
+};
+
+// the whole chain on n_blocks blocks per stream (n_blocks <= o->n_blocks: a stream plan's push may be shorter than its maximum).
+// STREAM = (sl != null); the batch plan's kernels are compiled without any of the stream plan's state.
+template <bool STREAM>
+static int ook_launch(lrc_ook *o, const uint8_t *d_iq, size_t n_blocks, size_t stream_stride_bytes, cudaStream_t s,
+                      const OokStreamLaunch *sl)
 {
-    LRC_REQUIRE(o != nullptr, LRC_ERR_INVALID, "null plan");
-    LRC_BIND(o->ctx);
-    LRC_REQUIRE(d_iq != nullptr, LRC_ERR_INVALID, "lrc_ook_decode: null input");
-    LRC_REQUIRE(stream_stride_bytes >= o->n_blocks * (size_t)OOK_BLOCK * 2, LRC_ERR_INVALID, "lrc_ook_decode: stride too short");
-    LRC_REQUIRE(((uintptr_t)d_iq & 15) == 0 && (stream_stride_bytes & 15) == 0, LRC_ERR_INVALID,
-                "lrc_ook_decode: input and stream stride must be 16-byte aligned");
-    cudaStream_t s = lrc_stream(o->ctx, stream);
-    const size_t groups = ((o->n_blocks + 31) / 32) * o->n_streams;
+    const size_t groups = ((n_blocks + 31) / 32) * o->n_streams;
     const size_t cap = (size_t)o->ctx->n_sm;           // one persistent CTA per SM (the table fills its shared memory)
     // LRC_OOK_KA: 3 (default) = folded table + TMA slabs, 16 warps x 2 stages, table skew as one LEA.HI (ALU pipe): 0.825 ms for the
     // whole chain; 1 = the same with the skew as IMAD.HI (FMA pipe, needs a zeroed pair register per use: 0.913 ms); 2 = like 1 with
@@ -1484,14 +1698,14 @@ extern "C" int lrc_ook_decode(lrc_ook *o, const uint8_t *d_iq, size_t stream_str
         size_t blocks = ceil_div(groups, (size_t)KA_WARPS);
         if (blocks > cap) blocks = cap;
         ook_block_kernel<<<(unsigned)blocks, KA_WARPS * 32, KA_SMEM_BYTES, s>>>(d_iq, stream_stride_bytes, o->n_streams,
-                                                                               o->n_blocks, o->d_lut, o->d_sum, o->d_max);
+                                                                               n_blocks, o->d_lut, o->d_sum, o->d_max);
     } else {
         // the capture as a byte tensor [stream][block][1024]: one box = 64 bytes of 32 consecutive blocks of one stream
         typedef CUresult (*encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                       const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                       CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
         CUtensorMap tm;
-        const cuuint64_t dims[3] = {(cuuint64_t)OOK_BLOCK * 2, (cuuint64_t)o->n_blocks, (cuuint64_t)o->n_streams};
+        const cuuint64_t dims[3] = {(cuuint64_t)OOK_BLOCK * 2, (cuuint64_t)n_blocks, (cuuint64_t)o->n_streams};
         const cuuint64_t strides[2] = {(cuuint64_t)OOK_BLOCK * 2, (cuuint64_t)stream_stride_bytes};
         const cuuint32_t box[3] = {KA2_SLAB_BYTES, 32, 1};
         const cuuint32_t estr[3] = {1, 1, 1};
@@ -1501,67 +1715,90 @@ extern "C" int lrc_ook_decode(lrc_ook *o, const uint8_t *d_iq, size_t stream_str
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (cr != CUDA_SUCCESS) {
             lrc_set_error("lrc_ook_decode: cuTensorMapEncodeTiled -> CUresult %d (n_blocks %zu, n_streams %zu, stride %zu)",
-                          (int)cr, o->n_blocks, o->n_streams, stream_stride_bytes);
+                          (int)cr, n_blocks, o->n_streams, stream_stride_bytes);
             return LRC_ERR_CUDA;
         }
         if (ka == 2) {
             size_t blocks = ceil_div(groups, (size_t)8);
             if (blocks > cap) blocks = cap;
             ook_block_tma_kernel<8, 4, true><<<(unsigned)blocks, 8 * 32, Ka2Cfg<8, 4>::SMEM_BYTES, s>>>(
-                tm, o->n_streams, o->n_blocks, o->d_flut, o->d_sum, o->d_max);
+                tm, o->n_streams, n_blocks, o->d_flut, o->d_sum, o->d_max);
         } else {
             size_t blocks = ceil_div(groups, (size_t)16);
             if (blocks > cap) blocks = cap;
             if (ka == 3)
                 ook_block_tma_kernel<16, 2, false><<<(unsigned)blocks, 16 * 32, Ka2Cfg<16, 2>::SMEM_BYTES, s>>>(
-                    tm, o->n_streams, o->n_blocks, o->d_flut, o->d_sum, o->d_max);
+                    tm, o->n_streams, n_blocks, o->d_flut, o->d_sum, o->d_max);
             else
                 ook_block_tma_kernel<16, 2, true><<<(unsigned)blocks, 16 * 32, Ka2Cfg<16, 2>::SMEM_BYTES, s>>>(
-                    tm, o->n_streams, o->n_blocks, o->d_flut, o->d_sum, o->d_max);
+                    tm, o->n_streams, n_blocks, o->d_flut, o->d_sum, o->d_max);
         }
     }
     LRC_CUDA(cudaGetLastError());
-    ook_trigger_kernel<<<(unsigned)ceil_div(o->n_streams, (size_t)KB_STREAMS), KB_THREADS, 0, s>>>(
-        o->d_sum, o->n_streams, o->n_blocks, o->max_bursts, o->guard_samples, o->d_tag, o->d_bend, o->d_bflags, o->d_nbursts);
+    ook_trigger_kernel<STREAM><<<(unsigned)ceil_div(o->n_streams, (size_t)KB_STREAMS), KB_THREADS, 0, s>>>(
+        o->d_sum, o->n_streams, n_blocks, o->max_bursts, o->guard_samples, o->d_tag, o->d_bend, o->d_bflags, o->d_nbursts,
+        sl ? sl->seam : nullptr);
     LRC_CUDA(cudaGetLastError());
-    const size_t kc1_blocks = std::min(ceil_div(groups, (size_t)KC1_WARPS), cap);
-    ook_burst_kernel<<<(unsigned)ceil_div(o->n_streams * o->max_bursts, (size_t)KC0_WARPS), KC0_WARPS * 32, 0, s>>>(
-        o->n_streams, o->n_blocks, o->max_bursts, o->d_max, o->d_tag, o->d_bend, o->d_bflags, o->d_nbursts, o->d_uniq, o->n_uniq,
-        o->d_half, o->d_hrank, o->d_next, (uint32_t)(3 * kc1_blocks * KC1_WARPS));
+    const OokCarry carry = sl ? sl->carry : OokCarry{0, nullptr, nullptr, nullptr};
+    OokSeam *seam = sl ? sl->seam : nullptr;
+    const size_t slice_groups = ((carry.cpitch + n_blocks + 31) / 32) * o->n_streams;
+    const size_t kc1_blocks = std::min(ceil_div(slice_groups, (size_t)KC1_WARPS), cap);
+    ook_burst_kernel<STREAM><<<(unsigned)ceil_div(o->n_streams * o->max_bursts, (size_t)KC0_WARPS), KC0_WARPS * 32, 0, s>>>(
+        o->n_streams, n_blocks, o->max_bursts, o->d_max, o->d_tag, o->d_bend, o->d_bflags, o->d_nbursts, o->d_uniq, o->n_uniq,
+        o->d_half, o->d_hrank, o->d_next, (uint32_t)(3 * kc1_blocks * KC1_WARPS), seam, sl ? sl->d_live : nullptr);
     LRC_CUDA(cudaGetLastError());
     // Which K-C.  Until quiet blocks were skipped the one-warp-per-stream kernel won where an SM had 20 or more streams to itself (its
     // walk's latency covered by 28 warps); with them skipped the split form wins at every size measured -- whole chain, ms,
     // one-warp-per-stream / split: 4096 streams 0.596 / 0.571, 3072 0.493 / 0.452, 2048 0.391 / 0.335, 1024 0.292 / 0.220, 512 -- one
     // GPU's share of 4096 over eight -- 0.253 / 0.163 (profiles/r2_bb_ook_forms.txt) -- and is the default.  LRC_OOK_KC = 0 / 1 forces
-    // one or the other for A/B runs and for the tests that put both through the same cases; identical transition lists.
+    // one or the other for A/B runs and for the tests that put both through the same cases; identical transition lists.  A stream
+    // plan always runs the split form (the one-warp walk has no carry).
     const char *kc_s = getenv("LRC_OOK_KC");                              // read at every call: a test runs both forms in one process
     const int kc_env = kc_s && *kc_s ? atoi(kc_s) : -1;
-    const int kc = kc_env >= 0 ? kc_env : 1;
+    const int kc = STREAM ? 1 : kc_env >= 0 ? kc_env : 1;
     if (kc == 0) {
         size_t kc_warps = ceil_div(o->n_streams, (size_t)o->ctx->n_sm);
         if (kc_warps > KC_THREADS / 32) kc_warps = KC_THREADS / 32;
         ook_rle_kernel<<<(unsigned)ceil_div(o->n_streams, kc_warps), (unsigned)(kc_warps * 32), OOK_RANK_BYTES, s>>>(
-            d_iq, stream_stride_bytes, o->n_streams, o->n_blocks, o->max_bursts, o->max_runs, o->d_rank, o->d_tag, o->d_hrank,
+            d_iq, stream_stride_bytes, o->n_streams, n_blocks, o->max_bursts, o->max_runs, o->d_rank, o->d_tag, o->d_hrank,
             o->d_half, o->d_max, o->d_bflags, o->d_nbursts, o->d_trans, o->d_ntrans, o->d_nbits);
         LRC_CUDA(cudaGetLastError());
     } else {
-        ook_slice_kernel<<<(unsigned)kc1_blocks, KC1_WARPS * 32, OOK_RANK_BYTES, s>>>(
-            d_iq, stream_stride_bytes, o->n_streams, o->n_blocks, o->max_bursts, o->d_rank, o->d_tag, o->d_hrank, o->d_half,
-            o->d_max, o->d_next, o->d_mask, o->d_bsum);
+        ook_slice_kernel<STREAM><<<(unsigned)kc1_blocks, KC1_WARPS * 32, OOK_RANK_BYTES, s>>>(
+            d_iq, stream_stride_bytes, o->n_streams, n_blocks, o->max_bursts, o->d_rank, o->d_tag, o->d_hrank, o->d_half,
+            o->d_max, o->d_next, o->d_mask, o->d_bsum, carry);
         LRC_CUDA(cudaGetLastError());
-        ook_scan_kernel<<<(unsigned)ceil_div(o->n_streams, (size_t)KC2_WARPS), KC2_WARPS * 32, 0, s>>>(
-            o->n_streams, o->n_blocks, o->max_bursts, o->max_runs, o->d_tag, o->d_bsum, o->d_bflags, o->d_nbursts, o->d_binfo,
-            o->d_trans, o->d_ntrans, o->d_nbits);
+        ook_scan_kernel<STREAM><<<(unsigned)ceil_div(o->n_streams, (size_t)KC2_WARPS), KC2_WARPS * 32, 0, s>>>(
+            o->n_streams, n_blocks, o->max_bursts, o->max_runs, o->d_tag, o->d_bsum, o->d_bflags, o->d_nbursts, o->d_binfo,
+            o->d_trans, o->d_ntrans, o->d_nbits, carry, seam);
         LRC_CUDA(cudaGetLastError());
-        ook_scatter_kernel<<<(unsigned)ceil_div(groups, (size_t)KC3_WARPS), KC3_WARPS * 32, 0, s>>>(
-            o->n_streams, o->n_blocks, o->max_runs, o->d_tag, o->d_bsum, o->d_binfo, o->d_mask, o->d_trans);
+        ook_scatter_kernel<STREAM><<<(unsigned)ceil_div(slice_groups, (size_t)KC3_WARPS), KC3_WARPS * 32, 0, s>>>(
+            o->n_streams, n_blocks, o->max_runs, o->d_tag, o->d_bsum, o->d_binfo, o->d_mask, o->d_trans, carry);
         LRC_CUDA(cudaGetLastError());
     }
-    ook_match_kernel<<<(unsigned)ceil_div(o->n_streams, (size_t)KD_WARPS), KD_WARPS * 32, 0, s>>>(
+    if constexpr (STREAM) {
+        // after the slicer has read the carried blocks of a burst sent in this push: the carry may start over
+        ook_carry_kernel<<<(unsigned)ceil_div(o->n_streams, (size_t)KCY_WARPS), KCY_WARPS * 32, 0, s>>>(
+            d_iq, stream_stride_bytes, o->n_streams, n_blocks, carry.cpitch, sl->max_carry, o->d_tag, o->d_max, o->d_nbursts,
+            sl->d_carry, sl->d_cmax, sl->seam);
+        LRC_CUDA(cudaGetLastError());
+    }
+    ook_match_kernel<STREAM><<<(unsigned)ceil_div(o->n_streams, (size_t)KD_WARPS), KD_WARPS * 32, 0, s>>>(
         o->d_trans, o->d_ntrans, o->n_streams, o->max_runs, o->max_packets, (float)o->sample_rate, o->d_packets,
-        o->d_npackets, o->d_runs_dbg);
+        o->d_npackets, o->d_runs_dbg, seam, o->d_nbits, sl ? sl->d_pbase : nullptr);
     LRC_CUDA(cudaGetLastError());
     return LRC_OK;
+}
+
+extern "C" int lrc_ook_decode(lrc_ook *o, const uint8_t *d_iq, size_t stream_stride_bytes, void *stream)
+{
+    LRC_REQUIRE(o != nullptr, LRC_ERR_INVALID, "null plan");
+    LRC_BIND(o->ctx);
+    LRC_REQUIRE(d_iq != nullptr, LRC_ERR_INVALID, "lrc_ook_decode: null input");
+    LRC_REQUIRE(stream_stride_bytes >= o->n_blocks * (size_t)OOK_BLOCK * 2, LRC_ERR_INVALID, "lrc_ook_decode: stride too short");
+    LRC_REQUIRE(((uintptr_t)d_iq & 15) == 0 && (stream_stride_bytes & 15) == 0, LRC_ERR_INVALID,
+                "lrc_ook_decode: input and stream stride must be 16-byte aligned");
+    return ook_launch<false>(o, d_iq, o->n_blocks, stream_stride_bytes, lrc_stream(o->ctx, stream), nullptr);
 }
 
 extern "C" int lrc_ook_fetch_packets(lrc_ook *o, lrc_ook_packet *h_packets, size_t cap, size_t *n_packets)
@@ -1616,6 +1853,163 @@ extern "C" int lrc_ook_debug_ptrs(lrc_ook *o, const float **d_block_sums, const 
     if (d_runs) *d_runs = o->d_runs_dbg;
     if (d_n_bits) *d_n_bits = o->d_nbits;
     return LRC_OK;
+}
+
+// ---- streaming plan --------------------------------------------------------------------------------------------------------------
+struct lrc_ook_stream {
+    lrc_ook  *o;                      // the chain's buffers, sized for max_push_blocks; its d_mask / d_bsum / d_binfo rows start
+                                      // with cpitch carry slots
+    size_t    max_carry, max_packets;
+    OokSeam  *d_seam;                 // [n_streams]
+    uint8_t  *d_carry;                // [n_streams][cpitch][1024] the open burst's collected blocks
+    float    *d_cmax;                 // [n_streams][cpitch] their maxima
+    uint32_t *d_live;                 // [n_streams] carried blocks sliced in the current push
+    uint32_t *d_pbase;                // [n_streams][2] sequence number of the first packet not fetched yet
+    size_t    last_push;              // blocks per stream of the last push (the debug block sums' row length)
+    bool      failed;                 // a fetch reported an overflow: every call fails until reset
+};
+
+extern "C" int lrc_ook_stream_reset(lrc_ook_stream *st)
+{
+    LRC_REQUIRE(st != nullptr, LRC_ERR_INVALID, "null plan");
+    LRC_BIND(st->o->ctx);
+    const size_t ns = st->o->n_streams;
+    std::vector<OokSeam> z(ns, ook_seam_initial());
+    LRC_CUDA(cudaDeviceSynchronize());
+    LRC_CUDA(cudaMemcpy(st->d_seam, z.data(), ns * sizeof(OokSeam), cudaMemcpyHostToDevice));
+    LRC_CUDA(cudaMemset(st->d_pbase, 0, ns * 2 * sizeof(uint32_t)));
+    st->failed = false;
+    st->last_push = 0;
+    return LRC_OK;
+}
+
+extern "C" int lrc_ook_stream_destroy(lrc_ook_stream *st)
+{
+    if (!st) return LRC_OK;
+    if (st->o) {
+        cudaSetDevice(st->o->ctx->device);
+        cudaFree(st->d_seam); cudaFree(st->d_carry); cudaFree(st->d_cmax); cudaFree(st->d_live); cudaFree(st->d_pbase);
+        lrc_ook_destroy(st->o);
+    }
+    delete st;
+    return LRC_OK;
+}
+
+extern "C" int lrc_ook_stream_create(lrc_ctx *ctx, size_t n_streams, size_t max_push_blocks, unsigned sample_rate,
+                                     size_t max_carry_blocks, size_t max_runs_per_push, size_t max_packets_per_fetch,
+                                     lrc_ook_stream **out)
+{
+    LRC_BIND(ctx);
+    LRC_REQUIRE(out && n_streams >= 1 && max_push_blocks >= 1 && sample_rate >= 1, LRC_ERR_INVALID,
+                "lrc_ook_stream_create: bad arguments");
+    // an open burst never holds more than guard + 1 blocks (bitfount.rs:52-54): the buffer is reset before a block is pushed once it
+    // exceeds the guard, so it ends at most one block past it, plus one more when it did not start with the 0.0.  That carry is
+    // exact for every input; a smaller one is the caller's memory choice, and a burst that outgrows it is reported.
+    size_t guard_blocks = 1000u * (size_t)OOK_TRIGGER_DURATION;
+    if (const char *g = getenv("LRC_OOK_TEST_GUARD_BLOCKS")) { const long v = atol(g); if (v >= 1) guard_blocks = (size_t)v; }
+    const size_t max_carry = max_carry_blocks ? max_carry_blocks : guard_blocks + 1;
+    const size_t cpitch = (max_carry + 31) / 32 * 32;
+    lrc_ook_stream *st = new (std::nothrow) lrc_ook_stream();
+    LRC_REQUIRE(st != nullptr, LRC_ERR_NOMEM, "out of host memory");
+    memset(st, 0, sizeof(*st));
+    const int rc = ook_create(ctx, n_streams, max_push_blocks, cpitch, sample_rate, max_runs_per_push, max_packets_per_fetch, &st->o);
+    if (rc != LRC_OK) { delete st; return rc; }
+    st->max_carry = max_carry;
+    st->max_packets = st->o->max_packets;
+    cudaError_t e = cudaMalloc(&st->d_seam, n_streams * sizeof(OokSeam));
+    if (e == cudaSuccess) e = cudaMalloc(&st->d_carry, n_streams * cpitch * (size_t)(OOK_BLOCK * 2));
+    if (e == cudaSuccess) e = cudaMalloc(&st->d_cmax, n_streams * cpitch * sizeof(float));
+    if (e == cudaSuccess) e = cudaMalloc(&st->d_live, n_streams * sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMalloc(&st->d_pbase, n_streams * 2 * sizeof(uint32_t));
+    if (e != cudaSuccess) {
+        lrc_set_error("lrc_ook_stream_create: %s (carry of %zu blocks x %zu streams)", cudaGetErrorString(e), max_carry, n_streams);
+        lrc_ook_stream_destroy(st);
+        return e == cudaErrorMemoryAllocation ? LRC_ERR_NOMEM : LRC_ERR_CUDA;
+    }
+    const int r2 = lrc_ook_stream_reset(st);
+    if (r2 != LRC_OK) { lrc_ook_stream_destroy(st); return r2; }
+    *out = st;
+    return LRC_OK;
+}
+
+extern "C" int lrc_ook_stream_push(lrc_ook_stream *st, const uint8_t *d_iq, size_t n_blocks, size_t stream_stride_bytes, void *stream)
+{
+    LRC_REQUIRE(st != nullptr, LRC_ERR_INVALID, "null plan");
+    lrc_ook *o = st->o;
+    LRC_BIND(o->ctx);
+    LRC_REQUIRE(!st->failed, LRC_ERR_CAPACITY, "lrc_ook_stream_push: the plan overflowed (see the fetch that reported it); reset it");
+    LRC_REQUIRE(d_iq != nullptr, LRC_ERR_INVALID, "lrc_ook_stream_push: null input");
+    LRC_REQUIRE(n_blocks >= 1 && n_blocks <= o->n_blocks, LRC_ERR_INVALID, "lrc_ook_stream_push: n_blocks outside 1..max_push_blocks");
+    LRC_REQUIRE(stream_stride_bytes >= n_blocks * (size_t)OOK_BLOCK * 2, LRC_ERR_INVALID, "lrc_ook_stream_push: stride too short");
+    LRC_REQUIRE(((uintptr_t)d_iq & 15) == 0 && (stream_stride_bytes & 15) == 0, LRC_ERR_INVALID,
+                "lrc_ook_stream_push: input and stream stride must be 16-byte aligned");
+    OokStreamLaunch sl;
+    sl.seam = st->d_seam;
+    sl.carry = OokCarry{o->cpitch, st->d_carry, st->d_cmax, st->d_live};
+    sl.d_carry = st->d_carry; sl.d_cmax = st->d_cmax; sl.d_live = st->d_live; sl.d_pbase = st->d_pbase;
+    sl.max_carry = st->max_carry;
+    const int rc = ook_launch<true>(o, d_iq, n_blocks, stream_stride_bytes, lrc_stream(o->ctx, stream), &sl);
+    if (rc == LRC_OK) st->last_push = n_blocks;
+    return rc;
+}
+
+extern "C" int lrc_ook_stream_fetch_packets(lrc_ook_stream *st, lrc_ook_packet *h_packets, size_t cap, size_t *n_packets)
+{
+    LRC_REQUIRE(st && n_packets, LRC_ERR_INVALID, "lrc_ook_stream_fetch_packets: null argument");
+    lrc_ook *o = st->o;
+    LRC_BIND(o->ctx);
+    *n_packets = 0;
+    LRC_REQUIRE(!st->failed, LRC_ERR_CAPACITY, "lrc_ook_stream_fetch_packets: the plan overflowed earlier; reset it");
+    LRC_CUDA(cudaDeviceSynchronize());
+    const size_t ns = o->n_streams, mp = st->max_packets;
+    std::vector<OokSeam> z(ns);
+    std::vector<uint32_t> base(ns * 2);
+    LRC_CUDA(cudaMemcpy(z.data(), st->d_seam, ns * sizeof(OokSeam), cudaMemcpyDeviceToHost));
+    LRC_CUDA(cudaMemcpy(base.data(), st->d_pbase, ns * 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    size_t total = 0;
+    for (size_t s = 0; s < ns; ++s) {
+        const uint32_t na = z[s].m_count[0] - base[2 * s], nb = z[s].m_count[1] - base[2 * s + 1];
+        if (z[s].err || na > mp || nb > mp) {
+            st->failed = true;
+            lrc_set_error("lrc_ook_stream_fetch_packets: stream %zu overflowed:%s%s%s%s (carry %zu blocks, runs per push %zu, bursts per "
+                          "push %zu, packets per fetch %zu); the plan fails until reset", s,
+                          (z[s].err & OOK_ERR_CARRY) ? " its open burst outgrew max_carry_blocks" : "",
+                          (z[s].err & OOK_ERR_RUNS) ? " runs" : "", (z[s].err & OOK_ERR_BURSTS) ? " bursts" : "",
+                          (na > mp || nb > mp) ? " packets" : "", st->max_carry, o->max_runs, o->max_bursts, mp);
+            return LRC_ERR_CAPACITY;
+        }
+        total += na + nb;
+    }
+    *n_packets = total;
+    if (total == 0) return LRC_OK;
+    if (cap < total || !h_packets) {
+        lrc_set_error("lrc_ook_stream_fetch_packets: %zu packets, capacity %zu", total, cap);
+        return LRC_ERR_CAPACITY;
+    }
+    std::vector<unsigned long long> pk(ns * 2 * mp);
+    LRC_CUDA(cudaMemcpy(pk.data(), o->d_packets, pk.size() * 8, cudaMemcpyDeviceToHost));
+    size_t w = 0;
+    for (size_t s = 0; s < ns; ++s)
+        for (int proto = 0; proto < 2; ++proto) {
+            const uint32_t nbits = proto == 0 ? 36u : 24u;
+            for (uint32_t k = 0; k < z[s].m_count[proto] - base[2 * s + proto]; ++k) {
+                lrc_ook_packet &p = h_packets[w++];
+                p.stream = (uint32_t)s; p.proto = (uint32_t)proto; p.seq = base[2 * s + proto] + k; p.nbits = nbits;
+                memset(p.bits, 0, sizeof(p.bits));
+                const unsigned long long v = pk[(s * 2 + proto) * mp + k];
+                for (uint32_t i = 0; i < nbits; ++i) p.bits[i] = (uint8_t)((v >> (nbits - 1 - i)) & 1ull);
+            }
+        }
+    for (size_t s = 0; s < ns; ++s) { base[2 * s] = z[s].m_count[0]; base[2 * s + 1] = z[s].m_count[1]; }
+    LRC_CUDA(cudaMemcpy(st->d_pbase, base.data(), ns * 2 * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    return LRC_OK;
+}
+
+extern "C" int lrc_ook_stream_debug_ptrs(lrc_ook_stream *st, const float **d_block_sums, const uint32_t **d_run_counts,
+                                         const uint32_t **d_runs, const uint32_t **d_n_bits)
+{
+    LRC_REQUIRE(st != nullptr, LRC_ERR_INVALID, "null plan");
+    return lrc_ook_debug_ptrs(st->o, d_block_sums, d_run_counts, d_runs, d_n_bits);
 }
 
 extern "C" int lrc_eat(const uint8_t *bits, size_t nbits, const size_t *widths, size_t n_widths, size_t *out)

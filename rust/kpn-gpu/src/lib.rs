@@ -19,7 +19,7 @@
 //! | (north-star) discriminator                      | [`fm_demod`]                           |
 //! | (north-star) FIR -> FFT -> \|X\|^2 chain           | [`chain_psd`]                          |
 //! | (north-star) config-3 receiver, N channels      | [`fm_receiver_multi`] (one kernel per batch) |
-//! | `trigger` .. `shaper_optional` ratpak.rs:60-111  | [`ook_decode`], [`split_protocols`]    |
+//! | `trigger` .. `shaper_optional` ratpak.rs:60-111  | [`ook_decode`], [`ook_decode_stream`], [`split_protocols`] |
 //! | `kpn::eat` kpn.rs:116-124                        | [`eat`]                                |
 use libredio_cuda_sys as sys;
 use num_complex::Complex;
@@ -118,6 +118,7 @@ plan_guard!(ResamplerPlan, sys::lrc_resampler, sys::lrc_resampler_destroy);
 plan_guard!(ChainPlan, sys::lrc_chain, sys::lrc_chain_destroy);
 plan_guard!(FmRxPlan, sys::lrc_fmrx, sys::lrc_fmrx_destroy);
 plan_guard!(OokPlan, sys::lrc_ook, sys::lrc_ook_destroy);
+plan_guard!(OokStreamPlan, sys::lrc_ook_stream, sys::lrc_ook_stream_destroy);
 
 /// Drop-in for `rtlsdr::data_to_samples` as a block (src/rtlsdr/src/rtlsdr.rs:160-162; wired in bitfount.rs:24-28):
 /// bytes pairwise to `Complex<f32>`, bit-exact `i2f`.  An odd length panics like the reference's `i[1]`.
@@ -386,6 +387,44 @@ pub fn ook_decode(gpu: &Gpu, u: Receiver<Vec<u8>>, v: Sender<OokPacket>, n_strea
         for p in &pk[..n] {
             let bits = p.bits[..p.nbits as usize].iter().map(|&b| b as usize).collect();
             v.send(OokPacket { stream: p.stream, proto: p.proto, bits }).unwrap();
+        }
+    }
+}
+
+/// The streaming form of [`ook_decode`], for a live receiver: every message holds the NEXT `k` blocks of each of the
+/// `n_streams` streams, stream-major (`n_streams * k * 1024` bytes), `k` free to change from message to message.  The state
+/// of the reference's `trigger` .. `shaper_optional` blocks stays on the device between messages, so the packets sent after
+/// a message are exactly those the reference sends on all the bytes so far.  The carry is the exact one (the trigger's OOM
+/// guard + 1 blocks per stream).
+pub fn ook_decode_stream(gpu: &Gpu, u: Receiver<Vec<u8>>, v: Sender<OokPacket>, n_streams: usize, s_rate: u32) {
+    let (max_push, max_carry, max_runs, max_packets) = (1024usize, 0usize, 1usize << 16, 256usize);
+    let mut ook = ptr::null_mut();
+    check(unsafe { sys::lrc_ook_stream_create(gpu.0, n_streams, max_push, s_rate, max_carry, max_runs, max_packets, &mut ook) },
+          "lrc_ook_stream_create");
+    let ook = OokStreamPlan(ook);
+    let st = Stream::new(gpu);
+    let mut inp = Slot::new(gpu);
+    let mut pk = vec![sys::lrc_ook_packet { stream: 0, proto: 0, seq: 0, nbits: 0, bits: [0u8; 40] }; n_streams * 2 * max_packets];
+    loop {
+        let msg = u.recv().unwrap();
+        assert!(!msg.is_empty() && msg.len() % (n_streams * 1024) == 0, "ook_decode_stream: message is not n_streams * k * 1024 bytes");
+        let k = msg.len() / (n_streams * 1024);
+        inp.reserve(msg.len());
+        inp.put(0, &msg);
+        inp.h2d(msg.len(), &st);
+        let mut b = 0usize;
+        while b < k {
+            let n = max_push.min(k - b);
+            check(unsafe { sys::lrc_ook_stream_push(ook.0, (inp.d as *const u8).add(b * 1024), n, k * 1024, st.0) },
+                  "lrc_ook_stream_push");
+            let mut np = 0usize;
+            check(unsafe { sys::lrc_ook_stream_fetch_packets(ook.0, pk.as_mut_ptr(), pk.len(), &mut np) },
+                  "lrc_ook_stream_fetch_packets");
+            for p in &pk[..np] {
+                let bits = p.bits[..p.nbits as usize].iter().map(|&b| b as usize).collect();
+                v.send(OokPacket { stream: p.stream, proto: p.proto, bits }).unwrap();
+            }
+            b += n;
         }
     }
 }

@@ -15,7 +15,8 @@ pub const LRC_WINDOW_NONE: c_int = 0;
 pub const LRC_WINDOW_HANN: c_int = 1;
 
 macro_rules! opaque { ($($n:ident),*) => { $( #[repr(C)] pub struct $n { _p: [u8; 0] } )* } }
-opaque!(lrc_ctx, lrc_fir, lrc_fir_stream, lrc_fft, lrc_rfft, lrc_psd, lrc_chain, lrc_fastfir, lrc_resampler, lrc_fmrx, lrc_ook, lrc_gather);
+opaque!(lrc_ctx, lrc_fir, lrc_fir_stream, lrc_fft, lrc_rfft, lrc_psd, lrc_chain, lrc_fastfir, lrc_resampler, lrc_fmrx, lrc_ook,
+        lrc_ook_stream, lrc_gather);
 
 #[repr(C)]
 #[derive(Clone, Copy)]
@@ -138,6 +139,17 @@ extern "C" {
     pub fn lrc_ook_fetch_packets(ook: *mut lrc_ook, h_packets: *mut lrc_ook_packet, cap: size_t, n_packets: *mut size_t) -> c_int;
     pub fn lrc_ook_debug_ptrs(ook: *mut lrc_ook, d_block_sums: *mut *const c_float, d_run_counts: *mut *const u32,
                               d_runs: *mut *const u32, d_n_bits: *mut *const u32) -> c_int;
+    pub fn lrc_ook_stream_create(ctx: *mut lrc_ctx, n_streams: size_t, max_push_blocks: size_t, sample_rate: c_uint,
+                                 max_carry_blocks: size_t, max_runs_per_push: size_t, max_packets_per_fetch: size_t,
+                                 st: *mut *mut lrc_ook_stream) -> c_int;
+    pub fn lrc_ook_stream_destroy(st: *mut lrc_ook_stream) -> c_int;
+    pub fn lrc_ook_stream_reset(st: *mut lrc_ook_stream) -> c_int;
+    pub fn lrc_ook_stream_push(st: *mut lrc_ook_stream, d_iq: *const u8, n_blocks: size_t, stream_stride_bytes: size_t,
+                               stream: *mut c_void) -> c_int;
+    pub fn lrc_ook_stream_fetch_packets(st: *mut lrc_ook_stream, h_packets: *mut lrc_ook_packet, cap: size_t,
+                                        n_packets: *mut size_t) -> c_int;
+    pub fn lrc_ook_stream_debug_ptrs(st: *mut lrc_ook_stream, d_block_sums: *mut *const c_float, d_run_counts: *mut *const u32,
+                                     d_runs: *mut *const u32, d_n_bits: *mut *const u32) -> c_int;
     pub fn lrc_eat(bits: *const u8, nbits: size_t, widths: *const size_t, n_widths: size_t, out: *mut size_t) -> c_int;
     pub fn lrc_ook_envelope_table(ctx: *mut lrc_ctx, d_table: *mut c_float, stream: *mut c_void) -> c_int;
 
