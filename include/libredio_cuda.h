@@ -302,8 +302,7 @@ int lrc_ook_debug_ptrs(lrc_ook *ook, const float **d_block_sums, const uint32_t 
  * whatever the push sizes.  The blocks of a burst still open at the end of a push are kept in a per-stream carry of
  * max_carry_blocks blocks (0 = the trigger's OOM guard + 1 = 50 001 blocks, 51 MB per stream: exact for every
  * input); a smaller carry is a memory choice, and a burst that outgrows it is reported (LRC_ERR_CAPACITY naming the
- * stream, no packet from it), never decoded wrongly.  LRC_OOK_TEST_GUARD_BLOCKS is read at create, as for lrc_ook.
- * The slicer always runs in its split form here (LRC_OOK_KC is not read). */
+ * stream, no packet from it), never decoded wrongly.  LRC_OOK_TEST_GUARD_BLOCKS is read at create, as for lrc_ook. */
 typedef struct lrc_ook_stream lrc_ook_stream;
 int lrc_ook_stream_create(lrc_ctx *ctx, size_t n_streams, size_t max_push_blocks, unsigned sample_rate,
                           size_t max_carry_blocks, size_t max_runs_per_push, size_t max_packets_per_fetch,

@@ -17,22 +17,33 @@
 //                              the masks into per-block tags (the burst a block is collected into, -1 = none)
 //   K-B2 ook_burst_kernel    : per sent burst its maximum (fold of the tagged blocks' maxima), max/2 (discretize
 //                              :90-91) and that threshold as a rank among the distinct envelope values
-//   K-C  the slicer + rle, in one of two forms with identical output (the split form is the default, LRC_OOK_KC=0 selects the
-//        walk); neither reads a collected block whose maximum does not exceed the burst's max/2 (512 zeros):
-//        ook_rle_kernel      : one warp per stream re-reads the collected blocks, slices them against the burst's
-//                              rank threshold into bit masks and emits the positions where the continuous bit stream
-//                              changes value (rle: runs span burst boundaries, the last run is never flushed)
-//        ook_slice_kernel + ook_scan_kernel + ook_scatter_kernel: every (stream, 32 blocks) sliced independently into
-//                              stored bit masks, a per-stream scan over per-block summaries places every block in the
-//                              bit stream and the transition list, every block writes its transitions in place
+//   K-C  ook_slice_kernel + ook_scan_kernel + ook_scatter_kernel: the slicer + rle.  Every (stream, 32 blocks) is sliced
+//                              independently against the burst's rank threshold into stored bit masks, a per-stream scan over
+//                              per-block summaries places every block in the bit stream and the transition list, every block
+//                              writes the positions where the continuous bit stream changes value in place (rle: runs span
+//                              burst boundaries, the last run is never flushed).  A collected block whose maximum does not
+//                              exceed the burst's max/2 is not read (512 zeros)
 //   K-D  ook_match_kernel    : per stream: run lengths -> seconds (dle, IEEE f32 division) -> matcher A and B ->
 //                              shaper_optional -> packed packets
 //
 // Two plans run these kernels.  lrc_ook decodes finite captures, every stream from the reference's initial state.
-// lrc_ook_stream decodes endless streams pushed a few blocks at a time: K-B, K-B2, the split K-C and K-D take a per-stream
+// lrc_ook_stream decodes endless streams pushed a few blocks at a time: K-B, K-B2, K-C and K-D take a per-stream
 // OokSeam (null for lrc_ook) with what the reference's blocks hold between two messages, and ook_carry_kernel keeps the
 // blocks of the burst still open at the end of a push, which the slicer reads in place, in front of the push's blocks, when
 // that burst is sent.  The packets after any push are those of the reference on everything pushed so far.
+//
+// Measured and rejected (round 2, one B200 at its 1 kW power cap; whole chain, tools/bench_kernels.py --only ook; every form
+// produced the same bits):
+//   - K-A as the round-1 ook_block_kernel: a triangular envelope table (32896 sorted pairs, rows padded) and cp.async slabs,
+//     13.6 issued instructions per sample, 5.5 of them table index work and ~4 slab bookkeeping
+//     (profiles/r1_s3_ookA3_ncu_keys.txt): 0.893 ms against 0.825 for the TMA kernel with the folded table (tools/runs/r2n.sh);
+//   - K-A with the table skew k2 + (k2 >> 5) as mad.hi by 2^27 + 1, to move it from the ALU pipe (LEA.HI) to the FMA pipe:
+//     IMAD.HI adds into a 64-bit register pair whose low half has to be zeroed for every use, one more instruction per sample
+//     in a kernel bound by issue slots (81 % busy): 0.913 ms, and 1.001 ms with 8 warps x 4 stages (tools/runs/r2n.sh);
+//   - K-C as ook_rle_kernel, one warp per stream walking its collected blocks in order: with quiet blocks skipped the split
+//     form won at every size, whole chain in ms, one warp / split: 4096 streams 0.596 / 0.571, 3072 0.493 / 0.452,
+//     2048 0.391 / 0.335, 1024 0.292 / 0.220, 512 (one GPU's share of 4096 over eight) 0.253 / 0.163
+//     (profiles/r2_bb_ook_forms.txt).
 #include "common.cuh"
 #include "unpack.cuh"
 #include <cuda.h>
@@ -52,62 +63,25 @@ __device__ __forceinline__ float lr_envelope(uint32_t b0, uint32_t b1)
     return __double2float_rn(__dsqrt_rn(s));
 }
 
-// The envelope depends on the two bytes only and is symmetric in them (the f64 add commutes), so the hot
-// kernels read it from a triangular table (32896 entries, rows padded: 139.7 KB) held in shared memory.
-// The table is filled ON THE DEVICE by lr_envelope above when the plan is created; the u8 domain being
+// The envelope depends on the two bytes only and is symmetric in them (the f64 add commutes), so the block-sum
+// kernel reads it from a table of the 32896 sorted pairs {lo <= hi} (the folded table below, 135.7 KB) held in shared
+// memory.  The table is filled ON THE DEVICE by lr_envelope above when the plan is created; the u8 domain being
 // finite, table == formula for all 65536 pairs is a proof of equivalence, checked exhaustively by
 // tests/test_gpu_ook_fastfir.py::test_envelope_exhaustive_65536_pairs_bit_exact (formula vs CPU) and by the
 // bit-exact block sums of every OOK test (table vs CPU).
-// Row hi of the triangle starts at hi (hi + 17) / 2 = tri(hi) + 8 hi: eight unused words per row, so that
-// consecutive rows start ~8 banks apart.  (With the plain tri(hi) the rows next to hi = 127 -- where a noise
-// floor lives -- start 0 or 1 bank apart and a warp's 32 lookups pile onto a handful of banks.)
-constexpr int OOK_LUT_N = 255 * (255 + 17) / 2 + 256;         // 34936 floats
-constexpr int OOK_LUT_BYTES = OOK_LUT_N * 4;
-static_assert(OOK_LUT_N % 4 == 0, "table is copied as float4");
-
-__device__ __forceinline__ uint32_t lut_index(uint32_t hi, uint32_t lo) { return ((hi * (hi + 17u)) >> 1) + lo; }
-
-__device__ __forceinline__ float lut_envelope(const float *lut, uint32_t b0, uint32_t b1)
-{
-    return lut[lut_index(max(b0, b1), min(b0, b1))];
-}
-
-// The block-sum kernel is bound by the ALU pipe (byte extraction, max/min, index and address arithmetic run
-// there at half the FMA pipe's rate), so its lookup is written to keep that pipe short: one PRMT per byte,
-// max, min, and the byte address  lut + 4 (hi (hi + 17) / 2 + lo)  =  lut + hi (2 hi + 34) + 4 lo  as two
-// integer multiply-adds (FMA pipe) and one scaled add.
-__device__ __forceinline__ float lut_envelope_s(uint32_t lut_s, uint32_t b0, uint32_t b1)
-{
-    const uint32_t hi = max(b0, b1), lo = min(b0, b1);
-    uint32_t a, b;
-    asm("mad.lo.u32 %0, %1, 2, 34;" : "=r"(a) : "r"(hi));
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(b) : "r"(hi), "r"(a), "r"(lut_s));
-    float e;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(e) : "r"(b + 4u * lo));
-    return e;
-}
-
-__device__ __forceinline__ void lut_load(float *s_lut, const float *__restrict__ g_lut)
-{
-    for (int i = threadIdx.x; i < OOK_LUT_N / 4; i += blockDim.x)
-        reinterpret_cast<float4 *>(s_lut)[i] = __ldg(reinterpret_cast<const float4 *>(g_lut) + i);
-    __syncthreads();
-}
-
-// ---- folded table (round 2, the block-sum kernel's default) -----------------------------------------------
-// ncu on the triangular lookup (profiles/r1_s3_ookA3_ncu_keys.txt): ALU pipe 89.5 %, 13.6 issued instructions per
-// sample of which 5.5 are ALU-pipe index work (PRMT x2, IMNMX x2, LEA) and ~4 are the cp.async slab bookkeeping.
-// The folded table needs no byte extraction and no per-byte max/min:
+// The lookup is most of the block-sum kernel's instructions, and byte extraction, max/min, index and address arithmetic run on
+// the ALU pipe at half the FMA pipe's rate, so the folded table is laid out for a lookup with no byte extraction and no
+// per-byte max/min:
 //   * a 32-bit word holds two samples {b0, b1} {b2, b3}; ONE PRMT swaps the bytes of both halfwords and ONE
 //     VIMNMX.U16x2 (__vmaxu2) takes the per-halfword maximum  max(b0 | b1 << 8, b1 | b0 << 8) = hi << 8 | lo,
 //     the sorted pair as a 16-bit key -- two ALU instructions for two samples;
 //   * the triangle {lo <= hi} is folded into the 129 x 256 rectangle of rows 127..255: rows hi >= 128 stay where they
 //     are (columns 0..hi), a row hi <= 127 goes to row 254 - hi, columns 255 - lo (the free columns hi' + 1 .. 255 of
 //     that row): key2 = max(key, 65279 - key), one integer multiply-add (FMA pipe) and one signed max;
-//   * rows are skewed 8 banks apart like the triangular table's: index = key2 + (key2 >> 5) = 264 row + col + col / 32
-//     (one LEA.HI), injective because col + col / 32 <= 262 < 264.
-// 3.5 ALU-pipe instructions per sample instead of 5.5.  The table is filled by the same lr_envelope as before, so
-// table == formula for all 65536 pairs is still checked by the bit-exact block sums of every OOK test.
+//   * rows are skewed 8 banks apart: index = key2 + (key2 >> 5) = 264 row + col + col / 32 (one LEA.HI), injective
+//     because col + col / 32 <= 262 < 264.  (With a pitch of 256 every row starts in the same bank, and the pairs of a
+//     noise floor -- a few codes around 127 / 127, in neighbouring rows -- pile a warp's 32 lookups onto a handful of banks.)
+// 3.5 ALU-pipe instructions per sample (5.5 for the round-1 triangular table, see the rejected forms above).
 constexpr uint32_t OOK_FOLD_C = 65279u;                                  // 254 * 256 + 255
 __host__ __device__ __forceinline__ uint32_t ook_fold_index(uint32_t key)   // key = hi << 8 | lo, lo <= hi
 {
@@ -128,14 +102,6 @@ __global__ void ook_build_flut_kernel(float *__restrict__ flut)
     if (lo <= hi) flut[ook_fold_index(i) - OOK_FOLD_MIN] = lr_envelope(hi, lo);
 }
 
-__global__ void ook_build_lut_kernel(float *__restrict__ lut)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= 65536u) return;
-    const uint32_t hi = i >> 8, lo = i & 0xffu;
-    if (lo <= hi) lut[lut_index(hi, lo)] = lr_envelope(hi, lo);
-}
-
 struct lrc_ook {
     lrc_ctx *ctx;
     size_t   n_streams, n_blocks, max_runs, max_packets, max_bursts;
@@ -153,11 +119,10 @@ struct lrc_ook {
     unsigned long long *d_packets;    // [n_streams][2][max_packets] packets packed MSB-first
     uint32_t *d_npackets;             // [n_streams][2]
     uint32_t *d_runs_dbg;             // [n_streams][max_runs] (value << 31 | length), filled by K-D
-    float    *d_lut;                  // triangular envelope table, OOK_LUT_N floats (LRC_OOK_KA=0 variant)
-    float    *d_flut;                 // folded envelope table, OOK_FLUT_N floats (default block-sum kernel)
+    float    *d_flut;                 // folded envelope table, OOK_FLUT_N floats (the block-sum kernel's)
     void     *encode_tiled;           // cuTensorMapEncodeTiled (driver entry point, fetched once)
-    uint16_t *d_mask;                 // [n_streams][n_blocks][32] slicer output of collected blocks, 512 bits each (split K-C)
-    uint32_t *d_hrank;                // [n_streams][max_bursts] rank threshold of a sent burst (split K-C)
+    uint16_t *d_mask;                 // [n_streams][n_blocks][32] slicer output of collected blocks, 512 bits each (K-C)
+    uint32_t *d_hrank;                // [n_streams][max_bursts] rank threshold of a sent burst (K-C)
     uint32_t *d_next;                 // [1] next (stream, group) the slice kernel hands out
     uint32_t *d_bsum;                 // [n_streams][n_blocks] {inner transitions, first bit, last bit} of a collected block
     uint4    *d_binfo;                // [n_streams][n_blocks] place of a collected block in the bit stream and the transition list
@@ -212,110 +177,26 @@ struct OokCarry {
 // ---------------------------------------------------------------------------------------------
 // K-A: envelope, sequential block sum, block max.  One warp handles 32 consecutive blocks of one
 // stream and lane b owns block b: its 512 envelopes must be added one after the other (bitfount.rs:48),
-// so the lane walks its own 1024 bytes.  The bytes reach it through shared memory: the warp copies
-// 64-byte slabs of its 32 block rows with cp.async (16 bytes per lane, 4 lanes per row: coalesced, no
-// registers, the next slab in flight while this one is summed) into rows of pitch 80 bytes, which lane b
-// then reads back with LDS.128 -- 5 x 16 bytes between lanes, so the eight lanes of a quarter-warp phase
-// hit eight different bank groups.  No envelope is ever written back to shared memory.
-// ---------------------------------------------------------------------------------------------
-constexpr int KA_WARPS = 16;
-constexpr int KA_SLAB = 32;                          // samples per block row per slab (64 bytes)
-constexpr int KA_PITCH = KA_SLAB * 2 + 16;           // bytes between block rows in the staging tile
-constexpr int KA_STAGE_BYTES = 32 * KA_PITCH;
-constexpr int KA_STAGES = 2;
-constexpr int KA_SMEM_BYTES = OOK_LUT_BYTES + KA_WARPS * KA_STAGES * KA_STAGE_BYTES;
-
-__global__ void __launch_bounds__(KA_WARPS * 32, 1)
-ook_block_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_streams, size_t n_blocks,
-                 const float *__restrict__ g_lut, float *__restrict__ d_sum, float *__restrict__ d_max)
-{
-    extern __shared__ __align__(16) float ka_smem[];
-    float *lut = ka_smem;
-    lut_load(lut, g_lut);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint8_t *stg = reinterpret_cast<uint8_t *>(ka_smem + OOK_LUT_N) + warp * (KA_STAGES * KA_STAGE_BYTES);
-    const uint32_t stg_s = smem_u32(stg);
-    const uint32_t lut_s = smem_u32(lut);
-    const size_t groups_per_stream = (n_blocks + 31) / 32;
-    const size_t n_groups = groups_per_stream * n_streams;
-    const size_t warps_total = (size_t)gridDim.x * KA_WARPS;
-    constexpr int N_SLABS = OOK_BLOCK / KA_SLAB;
-    for (size_t grp = (size_t)blockIdx.x * KA_WARPS + warp; grp < n_groups; grp += warps_total) {
-        const size_t st = grp / groups_per_stream, b0 = (grp % groups_per_stream) * 32;
-        const int nb = (int)((n_blocks - b0) < 32 ? (n_blocks - b0) : 32);
-        const uint8_t *base = iq + st * stream_stride + b0 * (size_t)(OOK_BLOCK * 2);
-        auto issue = [&](int slab) {
-            const uint32_t dst0 = stg_s + (slab & 1) * KA_STAGE_BYTES;
-#pragma unroll
-            for (int it = 0; it < 4; ++it) {
-                const int row = it * 8 + (lane >> 2), col = lane & 3;
-                if (row < nb)
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;"
-                                 :: "r"(dst0 + row * KA_PITCH + col * 16),
-                                    "l"(base + (size_t)row * (OOK_BLOCK * 2) + slab * (KA_SLAB * 2) + col * 16) : "memory");
-            }
-            asm volatile("cp.async.commit_group;" ::: "memory");
-        };
-        float s = 0.0f, mx = 0.0f;
-        issue(0);
-        for (int slab = 0; slab < N_SLABS; ++slab) {
-            if (slab + 1 < N_SLABS) {
-                issue(slab + 1);
-                asm volatile("cp.async.wait_group 1;" ::: "memory");
-            } else {
-                asm volatile("cp.async.wait_group 0;" ::: "memory");
-            }
-            __syncwarp();                                   // every lane's copies of this slab have landed
-            if (lane < nb) {
-                const uint4 *r = reinterpret_cast<const uint4 *>(stg + (slab & 1) * KA_STAGE_BYTES + lane * KA_PITCH);
-#pragma unroll
-                for (int q = 0; q < KA_SLAB * 2 / 16; ++q) {
-                    const uint4 v = r[q];
-                    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        const float e0 = lut_envelope_s(lut_s, __byte_perm(w[k], 0, 0x4440), __byte_perm(w[k], 0, 0x4441));
-                        const float e1 = lut_envelope_s(lut_s, __byte_perm(w[k], 0, 0x4442), __byte_perm(w[k], 0, 0x4443));
-                        s = __fadd_rn(s, e0);                // samples.iter().sum(): left to right from 0.0
-                        s = __fadd_rn(s, e1);
-                        mx = fmaxf(mx, fmaxf(e0, e1));
-                    }
-                }
-            }
-            __syncwarp();                                   // the stage is rewritten two slabs from now
-        }
-        if (lane < nb) {
-            d_sum[st * n_blocks + b0 + lane] = s;
-            d_max[st * n_blocks + b0 + lane] = mx;
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// K-A, round 2 (default): the same lane-owns-block walk with
-//   * the folded table above (3.5 instead of 5.5 ALU-pipe instructions per sample), and
-//   * the staging done by the TMA engine: the capture is described to it as a 3-D byte tensor
-//     [stream][block][1024 B]; ONE cp.async.bulk.tensor per slab (issued by lane 0) brings the box
-//     {64 B, 32 blocks, 1 stream} into a 2 KB stage with the 64-byte hardware swizzle, i.e. 16-byte chunk c of
-//     row r lands at chunk c ^ ((r >> 1) & 3).  Lane r then reads its row with four LDS.128 and the eight lanes of
-//     a quarter-warp phase hit eight distinct bank groups (4 r + (c ^ f(r)) mod 8 takes all values 0..7) -- the
-//     transposition costs no padding, no per-lane address arithmetic and no LDGSTS instructions (the cp.async
-//     version spent ~4 of its 13.6 instructions per sample on slab bookkeeping).  Blocks past the end of the
-//     capture are zero-filled by the TMA (out-of-bounds rows of the box).
+// so the lane walks its own 1024 bytes, through the folded table above.  The bytes reach it through shared
+// memory, staged by the TMA engine: the capture is described to it as a 3-D byte tensor
+// [stream][block][1024 B]; ONE cp.async.bulk.tensor per slab (issued by lane 0) brings the box
+// {64 B, 32 blocks, 1 stream} into a 2 KB stage with the 64-byte hardware swizzle, i.e. 16-byte chunk c of
+// row r lands at chunk c ^ ((r >> 1) & 3).  Lane r then reads its row with four LDS.128 and the eight lanes of
+// a quarter-warp phase hit eight distinct bank groups (4 r + (c ^ f(r)) mod 8 takes all values 0..7) -- the
+// transposition costs no padding, no per-lane address arithmetic and no LDGSTS instructions.  Blocks past the
+// end of the capture are zero-filled by the TMA (out-of-bounds rows of the box).  No envelope is ever written
+// back to shared memory.
 // Every warp runs its own ring of KA2_STAGES stages with one mbarrier per stage and treats all its (group, slab)
 // pairs as one flat sequence, so the prefetch runs across group boundaries.
 // ---------------------------------------------------------------------------------------------
 constexpr int KA2_SLAB_BYTES = 64;
 constexpr int KA2_STAGE_BYTES = 32 * KA2_SLAB_BYTES;
 constexpr int KA2_SLABS = OOK_BLOCK * 2 / KA2_SLAB_BYTES;     // 16 slabs per block row
-
-template <int WARPS, int STAGES>
-struct Ka2Cfg {
-    static constexpr int STG_OFF = (OOK_FLUT_BYTES + 1023) / 1024 * 1024;
-    static constexpr int BAR_OFF = STG_OFF + WARPS * STAGES * KA2_STAGE_BYTES;
-    static constexpr int SMEM_BYTES = BAR_OFF + WARPS * STAGES * 8 + 1024;     // + slack to align the base to 1024
-    static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
-};
+constexpr int KA2_WARPS = 16, KA2_STAGES = 2;
+constexpr int KA2_STG_OFF = (OOK_FLUT_BYTES + 1023) / 1024 * 1024;
+constexpr int KA2_BAR_OFF = KA2_STG_OFF + KA2_WARPS * KA2_STAGES * KA2_STAGE_BYTES;
+constexpr int KA2_SMEM_BYTES = KA2_BAR_OFF + KA2_WARPS * KA2_STAGES * 8 + 1024;     // + slack to align the base to 1024
+static_assert(KA2_SMEM_BYTES <= 227 * 1024, "shared memory budget");
 
 __device__ __forceinline__ void tma_load_box3(uint32_t dst_s, const CUtensorMap *tm, int c0, int c1, int c2, uint32_t bar_s)
 {
@@ -324,31 +205,23 @@ __device__ __forceinline__ void tma_load_box3(uint32_t dst_s, const CUtensorMap 
 }
 
 // envelope of one sorted 16-bit key through the folded table; flut_adj = shared address of the table minus
-// 4 OOK_FOLD_MIN.  The negation runs on the FMA pipe (IMAD.MOV), the fused add-max (VIADDMNMX) and the address LEA on the ALU
-// pipe.  The skew k2 + (k2 >> 5) has two forms: SKEW_FMA writes it as mad.hi by 2^27 + 1 (floor(k2 (2^27 + 1) / 2^32) = k2 >> 5
-// for k2 < 2^16; with the plain 2^27 ptxas turns it into an LEA.HI) to keep it on the FMA pipe, but IMAD.HI adds into a 64-bit
-// register pair whose low half has to be zeroed for every use -- one more instruction per sample, and the kernel is bound by
-// issue slots (81 % busy), not by the ALU pipe alone: the plain LEA.HI form measured 10 % faster and is the default.
-template <bool SKEW_FMA>
+// 4 OOK_FOLD_MIN.  The negation runs on the FMA pipe (IMAD.MOV), the fused add-max (VIADDMNMX), the skew (LEA.HI) and
+// the address LEA on the ALU pipe.
 __device__ __forceinline__ float flut_envelope(uint32_t flut_adj, uint32_t key)
 {
     int alt;
     asm("mad.lo.s32 %0, %1, -1, 65279;" : "=r"(alt) : "r"((int)key));
     const uint32_t k2 = (uint32_t)max(alt, (int)key);
-    uint32_t idx;
-    if (SKEW_FMA) asm("mad.hi.u32 %0, %1, 134217729, %1;" : "=r"(idx) : "r"(k2));   // IMAD.HI (+ a zeroed pair register)
-    else idx = k2 + (k2 >> 5);                                                       // LEA.HI
+    const uint32_t idx = k2 + (k2 >> 5);
     float e;
     asm volatile("ld.shared.f32 %0, [%1];" : "=f"(e) : "r"(flut_adj + 4u * idx));
     return e;
 }
 
-template <int WARPS, int STAGES, bool SKEW_FMA>
-__global__ void __launch_bounds__(WARPS * 32, 1)
+__global__ void __launch_bounds__(KA2_WARPS * 32, 1)
 ook_block_tma_kernel(const __grid_constant__ CUtensorMap tmap, size_t n_streams, size_t n_blocks,
                      const float *__restrict__ g_flut, float *__restrict__ d_sum, float *__restrict__ d_max)
 {
-    using Cfg = Ka2Cfg<WARPS, STAGES>;
     extern __shared__ __align__(1024) uint8_t ka2_smem[];
     // the 64-byte swizzle pattern is a function of the shared ADDRESS: stages must sit on 512-byte boundaries
     const uint32_t base_s = (smem_u32(ka2_smem) + 1023u) & ~1023u;
@@ -359,11 +232,11 @@ ook_block_tma_kernel(const __grid_constant__ CUtensorMap tmap, size_t n_streams,
     // warp index through a shuffle: the compiler then knows it (and every stage, barrier and box coordinate derived
     // from it) is warp-uniform and keeps the TMA operands in uniform registers
     const int lane = threadIdx.x & 31, warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-    const uint32_t stg_s = base_s + Cfg::STG_OFF + warp * (STAGES * KA2_STAGE_BYTES);
-    const uint32_t bar_s = base_s + Cfg::BAR_OFF + warp * (STAGES * 8);
+    const uint32_t stg_s = base_s + KA2_STG_OFF + warp * (KA2_STAGES * KA2_STAGE_BYTES);
+    const uint32_t bar_s = base_s + KA2_BAR_OFF + warp * (KA2_STAGES * 8);
     if (lane == 0) {
 #pragma unroll
-        for (int s = 0; s < STAGES; ++s)
+        for (int s = 0; s < KA2_STAGES; ++s)
             asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(bar_s + 8 * s), "r"(1));
         mbar_fence_init();
     }
@@ -371,24 +244,24 @@ ook_block_tma_kernel(const __grid_constant__ CUtensorMap tmap, size_t n_streams,
     const uint32_t flut_adj = base_s - 4u * OOK_FOLD_MIN;
     const size_t groups_per_stream = (n_blocks + 31) / 32;
     const size_t n_groups = groups_per_stream * n_streams;
-    const size_t warps_total = (size_t)gridDim.x * WARPS;
-    size_t grp = (size_t)blockIdx.x * WARPS + warp;
+    const size_t warps_total = (size_t)gridDim.x * KA2_WARPS;
+    size_t grp = (size_t)blockIdx.x * KA2_WARPS + warp;
     if (grp >= n_groups) return;
     // lane's read offsets inside a stage: row = lane, chunk q at (q ^ ((lane >> 1) & 3))
     const uint32_t row_s = stg_s + lane * KA2_SLAB_BYTES;
     const uint32_t f16 = ((uint32_t)(lane >> 1) & 3u) << 4;
-    // stage = slab % STAGES and parity = (slab / STAGES) & 1 come from the slab counter alone: a group has 16 slabs, a
-    // multiple of 2 STAGES, so every group starts with all barriers back in phase 0
-    static_assert(KA2_SLABS % (2 * STAGES) == 0, "phase bookkeeping");
+    // stage = slab % KA2_STAGES and parity = (slab / KA2_STAGES) & 1 come from the slab counter alone: a group has 16 slabs, a
+    // multiple of 2 KA2_STAGES, so every group starts with all barriers back in phase 0
+    static_assert(KA2_SLABS % (2 * KA2_STAGES) == 0, "phase bookkeeping");
     auto issue = [&](int st, int b0, int slab) {                 // lane 0
-        const uint32_t bar = bar_s + 8 * (slab % STAGES);
+        const uint32_t bar = bar_s + 8 * (slab % KA2_STAGES);
         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"(KA2_STAGE_BYTES) : "memory");
-        tma_load_box3(stg_s + (slab % STAGES) * KA2_STAGE_BYTES, &tmap, slab * KA2_SLAB_BYTES, b0, st, bar);
+        tma_load_box3(stg_s + (slab % KA2_STAGES) * KA2_STAGE_BYTES, &tmap, slab * KA2_SLAB_BYTES, b0, st, bar);
     };
     int st = (int)(grp / groups_per_stream), b0 = (int)(grp % groups_per_stream) * 32;
     if (lane == 0) {
 #pragma unroll
-        for (int k = 0; k < STAGES - 1; ++k) issue(st, b0, k);
+        for (int k = 0; k < KA2_STAGES - 1; ++k) issue(st, b0, k);
     }
     while (true) {
         const size_t grp_n = grp + warps_total;
@@ -396,14 +269,14 @@ ook_block_tma_kernel(const __grid_constant__ CUtensorMap tmap, size_t n_streams,
         const int st_n = (int)(grp_n / groups_per_stream), b0_n = (int)(grp_n % groups_per_stream) * 32;
         float s = 0.0f, mx = 0.0f;
 #pragma unroll 1
-        for (int so = 0; so < KA2_SLABS; so += STAGES) {
-            const uint32_t parity = (uint32_t)(so / STAGES) & 1u;
+        for (int so = 0; so < KA2_SLABS; so += KA2_STAGES) {
+            const uint32_t parity = (uint32_t)(so / KA2_STAGES) & 1u;
 #pragma unroll
-            for (int h = 0; h < STAGES; ++h) {
+            for (int h = 0; h < KA2_STAGES; ++h) {
                 const int slab = so + h;
                 // the stage this issue overwrites was read one slab ago (closed by its __syncwarp)
                 {
-                    const int nx = slab + STAGES - 1;
+                    const int nx = slab + KA2_STAGES - 1;
                     const bool wrap = nx >= KA2_SLABS;           // the prefetch runs into the warp's next group
                     if (lane == 0 && (!wrap || has_n)) issue(wrap ? st_n : st, wrap ? b0_n : b0, wrap ? nx - KA2_SLABS : nx);
                 }
@@ -427,8 +300,8 @@ ook_block_tma_kernel(const __grid_constant__ CUtensorMap tmap, size_t n_streams,
                     for (int k = 0; k < 4; ++k) {
                         // both samples of the word at once: per halfword max(b0 | b1 << 8, b1 | b0 << 8) = hi << 8 | lo
                         const uint32_t K = __vmaxu2(w[k], __byte_perm(w[k], 0, 0x2301));
-                        const float e0 = flut_envelope<SKEW_FMA>(flut_adj, K & 0xffffu);
-                        const float e1 = flut_envelope<SKEW_FMA>(flut_adj, __umulhi(K, 65536u));    // K >> 16 on the FMA pipe
+                        const float e0 = flut_envelope(flut_adj, K & 0xffffu);
+                        const float e1 = flut_envelope(flut_adj, __umulhi(K, 65536u));    // K >> 16 on the FMA pipe
                         s = __fadd_rn(s, e0);                    // samples.iter().sum(): left to right from 0.0
                         s = __fadd_rn(s, e1);
                         mx = fmaxf(mx, fmaxf(e0, e1));
@@ -784,21 +657,26 @@ ook_trigger_kernel(const float *__restrict__ d_sum, size_t n_streams, size_t n_b
 }
 
 // ---------------------------------------------------------------------------------------------
-// K-C: discretize + rle as bit masks, one warp per stream.  Lane l owns samples [16 l, 16 l + 16) of a
-// collected block (32 contiguous bytes).  The positions (in the flattened bit stream) where the value
-// changes are appended to the stream's transition list in order.
+// K-C: discretize + rle as bit masks.  A warp slices a collected block at a time, lane l owns samples
+// [16 l, 16 l + 16) of it (32 contiguous bytes).  The positions (in the flattened bit stream) where the value
+// changes make up the stream's transition list, in order.
 //
 // The slicer `x > max/2` (bitfount.rs:91) never needs the envelope VALUE here, only its order against the
 // threshold: the plan holds rank[b0 | b1 << 8] = index of the pair's envelope among the 32 k distinct
 // envelope values in ascending order (a 128 KB u16 table indexed by the raw byte pair -- no max/min, no
 // triangular index); a burst's max/2 becomes the rank threshold #{values <= max/2} by a warp-wide 32-ary
-// search of the sorted values when the walk enters the burst; then x > max/2  <=>  rank(x) >= threshold,
+// search of the sorted values (ook_burst_kernel); then x > max/2  <=>  rank(x) >= threshold,
 // exactly, for every byte pair.  Neighbouring byte pairs (a noise floor sits within a few codes of 127/127)
 // would all fall into the banks of byte0 >> 1 with a pitch of 256 entries, so a byte1 row is 264 entries long:
-// 132 words = 4 banks further per row, which spreads an 8 x 8 neighbourhood over all 32 banks.  Like the
-// block-sum kernel this one is ALU-pipe bound, so the per-sample work is kept to two PRMT, one integer
-// multiply-add (FMA pipe) and one scaled add for the address, one subtraction and one funnel shift that
-// moves the comparison's sign bit into the mask (bits arrive reversed; one BREV per 16 samples).
+// 132 words = 4 banks further per row, which spreads an 8 x 8 neighbourhood over all 32 banks.  The per-sample
+// work is six instructions: the raw halfword (LOP3, or IMAD.HI on the FMA pipe), its slot and address (LEA.HI,
+// IADD3), the load, one subtraction and one funnel shift that moves the comparison's sign bit into the mask
+// (bits arrive reversed; one BREV per 16 samples).
+//
+// QUIET BLOCKS.  The block-sum kernel left every block's maximum; a collected block whose maximum does not exceed the burst's
+// max/2 slices to 512 zeros (x <= block max <= max/2 for each of its samples: `x > max/2` is false, bitfount.rs:91) -- without
+// being read.  That is the noise the trigger keeps collecting for 49 blocks after a burst and most of the gaps between the
+// pulses of a packet: the slicer's share of the capture drops from the collected half to the blocks that hold a pulse.
 // ---------------------------------------------------------------------------------------------
 constexpr int OOK_RANK_PITCH = 264;                           // u16 entries per byte1 row (256 used)
 constexpr int OOK_RANK_N = 256 * OOK_RANK_PITCH;
@@ -831,173 +709,10 @@ __device__ __forceinline__ uint32_t warp_upper_bound(const float *__restrict__ u
     return lo;
 }
 
-constexpr int KC_THREADS = 896;              // at most 28 streams per CTA, one CTA per SM (the table fills its shared memory).  The launch
-                                             // uses ceil(n_streams / n_sm) warps per CTA so that every SM gets the same number of streams
-                                             // (4096 streams: 147 CTAs of 28 warps instead of 128 CTAs of 32 with 20 SMs idle)
-
-__global__ void __launch_bounds__(KC_THREADS, 1)
-ook_rle_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_streams, size_t n_blocks,
-               size_t max_bursts, size_t max_runs, const uint16_t *__restrict__ g_rank,
-               const int32_t *__restrict__ d_tag,
-               const uint32_t *__restrict__ d_hrank, const float *__restrict__ d_half, const float *__restrict__ d_max,
-               const uint8_t *__restrict__ d_bflags, const uint32_t *__restrict__ d_nbursts,
-               uint32_t *__restrict__ d_trans, uint32_t *__restrict__ d_ntrans, uint32_t *__restrict__ d_nbits)
-{
-    extern __shared__ __align__(16) uint16_t kc_rank[];
-    for (int i = threadIdx.x; i < OOK_RANK_BYTES / 16; i += blockDim.x)
-        reinterpret_cast<uint4 *>(kc_rank)[i] = __ldg(reinterpret_cast<const uint4 *>(g_rank) + i);
-    __syncthreads();
-    const int lane = threadIdx.x & 31;
-    const uint32_t rank_s = smem_u32(kc_rank);
-    const size_t st = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (st >= n_streams) return;
-    const int32_t *tag = d_tag + st * n_blocks;
-    const uint32_t *hrank = d_hrank + st * max_bursts;
-    const float *half = d_half + st * max_bursts;
-    const float *bmax = d_max + st * n_blocks;
-    const uint8_t *flags = d_bflags + st * max_bursts;
-    uint32_t *trans = d_trans + st * max_runs;
-    const uint8_t *base = iq + st * stream_stride;
-    // QUIET BLOCKS.  The block-sum kernel left every block's maximum; a collected block whose maximum does not exceed the burst's
-    // max/2 slices to 512 zeros (x <= block max <= max/2 for each of its samples: `x > max/2` is false, bitfount.rs:91) -- without
-    // being read.  That is the noise the trigger keeps collecting for 49 blocks after a burst and most of the gaps between the
-    // pulses of a packet: the slicer's share of the capture drops from the collected half to the blocks that hold a pulse.
-    float half_cur = -1.0f;      // max/2 of the current burst (no block maximum is below 0: nothing is quiet before a burst is entered)
-    uint32_t pos = 0;            // length of the bit stream so far
-    uint32_t ntr = 0;            // transitions so far
-    uint32_t prev = 0;           // value of the last bit (meaningful once pos > 0)
-    int32_t cur_burst = -1;
-    uint32_t h = 0;              // rank threshold of the current burst
-    // one collected block: 16 samples per lane -> bit mask -> transitions appended in order
-    // a burst that was SENT without a single collected block: the OOM guard (:52-54) reset the buffer to [0.0] on the block where
-    // the trigger counter stood at 1, nothing was pushed, and the next block sent that lone 0.0 (:78-81) -- one 0 bit
-    // (0.0 > 0.0 / 2 is false).  No tag points at such a burst, so the walk picks them up from the flags of the burst indices
-    // it steps over (flags == 3: sent, leading 0.0; an abandoned burst has bit 0 clear and contributes nothing).
-    auto lone_zero_bursts = [&](int32_t from, int32_t to) {
-        for (int32_t j = from; j < to; ++j) {
-            if ((flags[j] & 3u) == 3u) {
-                if (pos > 0 && prev != 0u) { if (lane == 0 && ntr < max_runs) trans[ntr] = pos; ntr++; }
-                prev = 0u; pos += 1;
-            }
-        }
-    };
-    auto process = [&](int32_t tg, float mxk, const uint4 &q0, const uint4 &q1) {
-        if (tg != cur_burst) {
-            lone_zero_bursts(cur_burst + 1, tg);
-            cur_burst = tg;
-            h = hrank[tg];                                                    // ook_burst_kernel: #{values <= max/2}
-            half_cur = half[tg];
-            if (flags[tg] & 2u) {
-                // the burst starts with the literal 0.0 of vec!(0.0): 0.0 > max/2 is false -> bit 0
-                if (pos > 0 && prev != 0u) { if (lane == 0 && ntr < max_runs) trans[ntr] = pos; ntr++; }
-                prev = 0u; pos += 1;
-            }
-        }
-        if (mxk <= half_cur) {                                                // quiet: 512 zeros (its samples were not even fetched
-            if (pos > 0 && prev != 0u) { if (lane == 0 && ntr < max_runs) trans[ntr] = pos; ntr++; }   // when the burst was known)
-            prev = 0u; pos += OOK_BLOCK;
-            return;
-        }
-        const uint32_t w[8] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w};
-        uint32_t m = 0;
-        const uint32_t hm1 = h - 1u;                                         // rank >= h  <=>  (h - 1) - rank < 0
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const uint32_t raw0 = w[i] & 0xffffu, raw1 = __umulhi(w[i], 65536u);        // w >> 16 on the FMA pipe
-            const uint32_t a0 = rank_s + 2u * (raw0 + (raw0 >> 5)), a1 = rank_s + 2u * (raw1 + (raw1 >> 5));
-            unsigned short r0, r1;
-            asm volatile("ld.shared.u16 %0, [%1];" : "=h"(r0) : "r"(a0));
-            asm volatile("ld.shared.u16 %0, [%1];" : "=h"(r1) : "r"(a1));
-            m = __funnelshift_l(hm1 - (uint32_t)r0, m, 1);                   // (x > max/2f32) as usize  :91
-            m = __funnelshift_l(hm1 - (uint32_t)r1, m, 1);
-        }
-        m = __brev(m) >> 16;                                                 // sample i -> bit i
-        // previous bit of this lane's first sample
-        uint32_t pb = __shfl_up_sync(0xffffffffu, m >> 15, 1) & 1u;
-        const bool has_prev = (lane > 0) || (pos > 0);
-        if (lane == 0) pb = prev;
-        uint32_t tm = (m ^ ((m << 1) | pb)) & 0xffffu;                       // bit i set: sample i differs from i-1
-        if (!has_prev) tm &= ~1u;                                            // very first bit of the stream
-        // most collected blocks are the noise that follows a burst (the trigger holds for 49 blocks) or the inside of a long
-        // pulse: no transition anywhere in the block, nothing to scan or append
-        if (__ballot_sync(0xffffffffu, tm != 0u) != 0u) {
-            const uint32_t cnt = __popc(tm);
-            uint32_t off = cnt;                                              // inclusive warp scan
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const uint32_t v = __shfl_up_sync(0xffffffffu, off, d);
-                if (lane >= d) off += v;
-            }
-            const uint32_t total = __shfl_sync(0xffffffffu, off, 31);
-            uint32_t o = ntr + off - cnt;
-            while (tm) {
-                const int i = __ffs(tm) - 1;
-                tm &= tm - 1;
-                if (o < max_runs) trans[o] = pos + lane * 16 + i;
-                ++o;
-            }
-            ntr += total;
-        }
-        prev = __shfl_sync(0xffffffffu, m >> 15, 31) & 1u;
-        pos += OOK_BLOCK;
-    };
-    // collected blocks are fetched PF at a time, one batch ahead of the one being sliced: a warp keeps
-    // 2 x PF KB in flight instead of one block (the walk along a stream is sequential)
-    constexpr int PF = 2;
-    int32_t tg_next = lane < (int)n_blocks ? tag[lane] : -1;
-    float mx_next = lane < (int)n_blocks ? bmax[lane] : 0.0f;
-    for (size_t b0 = 0; b0 < n_blocks; b0 += 32) {
-        const int32_t tg_l = tg_next;
-        const float mx_l = mx_next;
-        {
-            const size_t bn = b0 + 32 + lane;                                 // the next group's tags and maxima are on their way
-            tg_next = bn < n_blocks ? tag[bn] : -1;
-            mx_next = bn < n_blocks ? bmax[bn] : 0.0f;
-        }
-        unsigned rem = __ballot_sync(0xffffffffu, tg_l >= 0);
-        int kA[PF], kB[PF];
-        uint4 dA[PF][2], dB[PF][2];
-        // a block is fetched unless it is known to be quiet already: same burst as the one being sliced (its max/2 is at hand) and a
-        // maximum that does not exceed it.  Tags do not decrease along a stream, so the burst cannot change between this decision
-        // and the block's turn; a block of a burst not entered yet is fetched and judged when its turn comes.
-        auto take = [&](int (&ks)[PF], uint4 (&d)[PF][2]) {
-#pragma unroll
-            for (int i = 0; i < PF; ++i) {
-                ks[i] = rem ? __ffs(rem) - 1 : -1;
-                if (rem) rem &= rem - 1;
-                if (ks[i] >= 0) {
-                    const int32_t tgk = __shfl_sync(0xffffffffu, tg_l, ks[i]);
-                    const float mxk = __shfl_sync(0xffffffffu, mx_l, ks[i]);
-                    if (!(tgk == cur_burst && mxk <= half_cur)) {
-                        const uint4 *p = reinterpret_cast<const uint4 *>(base + (b0 + ks[i]) * (size_t)(OOK_BLOCK * 2) + lane * 32);
-                        d[i][0] = ldg_stream_u4(p); d[i][1] = ldg_stream_u4(p + 1);
-                    }
-                }
-            }
-        };
-        take(kA, dA);
-        while (kA[0] >= 0) {
-            take(kB, dB);
-#pragma unroll
-            for (int i = 0; i < PF; ++i)
-                if (kA[i] >= 0)
-                    process(__shfl_sync(0xffffffffu, tg_l, kA[i]), __shfl_sync(0xffffffffu, mx_l, kA[i]), dA[i][0], dA[i][1]);
-#pragma unroll
-            for (int i = 0; i < PF; ++i) { kA[i] = kB[i]; dA[i][0] = dB[i][0]; dA[i][1] = dB[i][1]; }
-        }
-    }
-    {
-        const uint32_t nbu = d_nbursts[st];
-        lone_zero_bursts(cur_burst + 1, (int32_t)(nbu < max_bursts ? nbu : max_bursts));
-    }
-    if (lane == 0) { d_ntrans[st] = ntr; d_nbits[st] = pos; }
-}
-
 // ---------------------------------------------------------------------------------------------
-// K-C, split form (default): the same slicer + rle as ook_rle_kernel in three kernels, so that nothing heavy is tied to the walk
-// along a stream.  ook_rle_kernel gives a stream to ONE warp, which reads and slices its collected blocks one after the other:
-// 4096 streams keep 28 warps per SM busy, but the kernel is bound by the latency of that walk (long-scoreboard 2.7 per issue),
-// and a shard of 512 streams (4096 streams over 8 GPUs) leaves three warps per SM walking for just as long.  Here
+// K-C in three kernels, so that nothing heavy is tied to the walk along a stream (a warp that reads and slices a stream's
+// collected blocks one after the other is bound by the latency of that walk, and a shard of 512 streams leaves three such warps
+// per SM: see the rejected forms at the top of the file):
 //   C1 ook_slice_kernel   : every (stream, group of 32 blocks) is an independent unit of work (grid-stride, one CTA per SM beside
 //                           the rank table): collected blocks -> 512-bit masks (64 B per block) and a summary word per block
 //                           {transitions between its own bits, first bit, last bit};
@@ -1006,7 +721,6 @@ ook_rle_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_st
 //                           index of its first entry in the transition list, transition at its first bit -- 20 bytes per block in,
 //                           16 out, no sample is touched;
 //   C3 ook_scatter_kernel : every (stream, group) independent again: blocks that hold a transition write them at their place.
-// Same transition list, bit for bit, as ook_rle_kernel (LRC_OOK_KC=0 keeps that kernel for A/B runs).
 // ---------------------------------------------------------------------------------------------
 constexpr int KC1_WARPS = 28;
 constexpr uint32_t KC_SUM_FIRST = 1u << 30, KC_SUM_LAST = 1u << 31, KC_SUM_CNT = 0x3ffu;
@@ -1041,7 +755,7 @@ __device__ __forceinline__ uint32_t kc_inner_transitions(uint32_t m, int lane)
 
 // K-B2: what the trigger kernel leaves open about a sent burst, one warp per (stream, burst): its maximum (bitfount.rs:90 fold(0.0,
 // max) -- order-free, so the per-block maxima of the blocks that carry its tag can be reduced in any order), max/2 (:91), and that
-// threshold in the rank domain  #{distinct envelope values <= max/2}  (see ook_rle_kernel).  The burst's blocks lie between the
+// threshold in the rank domain  #{distinct envelope values <= max/2}  (see K-C above).  The burst's blocks lie between the
 // block that ended the previous burst and the one that ended this one (d_bend).
 // Stream plans (STREAM): burst 0 is the one that was open when the push started; its carried blocks' running maximum is folded
 // in, and the carried blocks take part in this push's slicing (live = their number) only if it is sent here.
@@ -1125,7 +839,7 @@ ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_
     auto thr_of = [&](uint32_t g, int32_t tg) -> uint32_t {
         return tg >= 0 ? d_hrank[(size_t)(g / gps) * max_bursts + tg] - 1u : 0u;           // rank >= h  <=>  (h - 1) - rank < 0
     };
-    // quiet block (see ook_rle_kernel): its maximum does not exceed the burst's max/2, it slices to 512 zeros without being read
+    // quiet block (see QUIET BLOCKS above): its maximum does not exceed the burst's max/2, it slices to 512 zeros without being read
     auto quiet_of = [&](uint32_t g, int32_t tg) -> bool {
         if (tg < 0) return false;
         const size_t st = g / gps, b = (size_t)(g % gps) * 32 + lane;
@@ -1185,7 +899,7 @@ ook_slice_kernel(const uint8_t *__restrict__ iq, size_t stream_stride, size_t n_
             // was measured slower: slice 254 us against 225 for 4096 streams, 0.185 against 0.184 ms for a 512-stream chain.  The
             // kernel is not bound by its instruction count.  Nor by the data in flight: three batches in turn on 20 warps x 102
             // registers measured 232 us; nor by the L2 being asked for every 32-byte sector twice -- the two 128-bit loads of a
-            // lane share a sector -- since loads that allocate in L1 changed nothing, here and in ook_rle_kernel: tools/runs/r2ao.sh.)
+            // lane share a sector -- since loads that allocate in L1 changed nothing: tools/runs/r2ao.sh.)
             take(kA, dA);
             while (true) {
                 take(kB, dB);
@@ -1593,24 +1307,17 @@ static int ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, size_t cp
     OOK_ALLOC(d_packets, n_streams * 2 * o->max_packets); OOK_ALLOC(d_npackets, n_streams * 2);
     OOK_ALLOC(d_runs_dbg, n_streams * o->max_runs);
     OOK_ALLOC(d_mask, sr * 32); OOK_ALLOC(d_bsum, sr); OOK_ALLOC(d_binfo, sr); OOK_ALLOC(d_hrank, n_streams * o->max_bursts); OOK_ALLOC(d_next, 1);
-    OOK_ALLOC(d_lut, (size_t)OOK_LUT_N);
     OOK_ALLOC(d_flut, (size_t)OOK_FLUT_N);
     OOK_ALLOC(d_rank, (size_t)OOK_RANK_N); OOK_ALLOC(d_uniq, (size_t)65536);
 #undef OOK_ALLOC
     if (e == cudaSuccess) {
-        e = cudaMemsetAsync(o->d_lut, 0, OOK_LUT_BYTES, ctx->stream);           // the row padding is never read
-        ook_build_lut_kernel<<<256, 256, 0, ctx->stream>>>(o->d_lut);
-        e = cudaGetLastError();
-        if (e == cudaSuccess) e = cudaMemsetAsync(o->d_flut, 0, OOK_FLUT_BYTES, ctx->stream);   // the row skew gaps are never read
+        e = cudaMemsetAsync(o->d_flut, 0, OOK_FLUT_BYTES, ctx->stream);   // the row skew gaps are never read
         if (e == cudaSuccess) {
             ook_build_flut_kernel<<<256, 256, 0, ctx->stream>>>(o->d_flut);
             e = cudaGetLastError();
         }
         if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, KA_SMEM_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_block_tma_kernel<16, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Ka2Cfg<16, 2>::SMEM_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_block_tma_kernel<16, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Ka2Cfg<16, 2>::SMEM_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_block_tma_kernel<8, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Ka2Cfg<8, 4>::SMEM_BYTES);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_block_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, KA2_SMEM_BYTES);
         if (e == cudaSuccess) {
             cudaDriverEntryPointQueryResult qr;
             e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &o->encode_tiled, cudaEnableDefault, &qr);
@@ -1620,7 +1327,6 @@ static int ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, size_t cp
                 return LRC_ERR_UNSUPPORTED;
             }
         }
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_rle_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, OOK_RANK_BYTES);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_slice_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, OOK_RANK_BYTES);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(ook_slice_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, OOK_RANK_BYTES);
     }
@@ -1666,7 +1372,7 @@ extern "C" int lrc_ook_destroy(lrc_ook *o)
     cudaSetDevice(o->ctx->device);
     cudaFree(o->d_sum); cudaFree(o->d_max); cudaFree(o->d_tag); cudaFree(o->d_half); cudaFree(o->d_bflags); cudaFree(o->d_bend);
     cudaFree(o->d_nbursts); cudaFree(o->d_trans); cudaFree(o->d_ntrans); cudaFree(o->d_nbits);
-    cudaFree(o->d_packets); cudaFree(o->d_npackets); cudaFree(o->d_runs_dbg); cudaFree(o->d_lut); cudaFree(o->d_flut);
+    cudaFree(o->d_packets); cudaFree(o->d_npackets); cudaFree(o->d_runs_dbg); cudaFree(o->d_flut);
     cudaFree(o->d_rank); cudaFree(o->d_uniq); cudaFree(o->d_mask); cudaFree(o->d_bsum); cudaFree(o->d_binfo); cudaFree(o->d_hrank); cudaFree(o->d_next);
     delete o;
     return LRC_OK;
@@ -1690,50 +1396,27 @@ static int ook_launch(lrc_ook *o, const uint8_t *d_iq, size_t n_blocks, size_t s
 {
     const size_t groups = ((n_blocks + 31) / 32) * o->n_streams;
     const size_t cap = (size_t)o->ctx->n_sm;           // one persistent CTA per SM (the table fills its shared memory)
-    // LRC_OOK_KA: 3 (default) = folded table + TMA slabs, 16 warps x 2 stages, table skew as one LEA.HI (ALU pipe): 0.825 ms for the
-    // whole chain; 1 = the same with the skew as IMAD.HI (FMA pipe, needs a zeroed pair register per use: 0.913 ms); 2 = like 1 with
-    // 8 warps x 4 stages (1.001 ms); 0 = the round-1 kernel (triangular table, cp.async slabs: 0.893 ms).  A/B knob; identical bits.
-    static const int ka = getenv("LRC_OOK_KA") ? atoi(getenv("LRC_OOK_KA")) : 3;
-    if (ka == 0) {
-        size_t blocks = ceil_div(groups, (size_t)KA_WARPS);
-        if (blocks > cap) blocks = cap;
-        ook_block_kernel<<<(unsigned)blocks, KA_WARPS * 32, KA_SMEM_BYTES, s>>>(d_iq, stream_stride_bytes, o->n_streams,
-                                                                               n_blocks, o->d_lut, o->d_sum, o->d_max);
-    } else {
-        // the capture as a byte tensor [stream][block][1024]: one box = 64 bytes of 32 consecutive blocks of one stream
-        typedef CUresult (*encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                      const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-        CUtensorMap tm;
-        const cuuint64_t dims[3] = {(cuuint64_t)OOK_BLOCK * 2, (cuuint64_t)n_blocks, (cuuint64_t)o->n_streams};
-        const cuuint64_t strides[2] = {(cuuint64_t)OOK_BLOCK * 2, (cuuint64_t)stream_stride_bytes};
-        const cuuint32_t box[3] = {KA2_SLAB_BYTES, 32, 1};
-        const cuuint32_t estr[3] = {1, 1, 1};
-        const CUresult cr = reinterpret_cast<encode_fn>(o->encode_tiled)(
-            &tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<uint8_t *>(d_iq), dims, strides, box, estr,
-            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (cr != CUDA_SUCCESS) {
-            lrc_set_error("lrc_ook_decode: cuTensorMapEncodeTiled -> CUresult %d (n_blocks %zu, n_streams %zu, stride %zu)",
-                          (int)cr, n_blocks, o->n_streams, stream_stride_bytes);
-            return LRC_ERR_CUDA;
-        }
-        if (ka == 2) {
-            size_t blocks = ceil_div(groups, (size_t)8);
-            if (blocks > cap) blocks = cap;
-            ook_block_tma_kernel<8, 4, true><<<(unsigned)blocks, 8 * 32, Ka2Cfg<8, 4>::SMEM_BYTES, s>>>(
-                tm, o->n_streams, n_blocks, o->d_flut, o->d_sum, o->d_max);
-        } else {
-            size_t blocks = ceil_div(groups, (size_t)16);
-            if (blocks > cap) blocks = cap;
-            if (ka == 3)
-                ook_block_tma_kernel<16, 2, false><<<(unsigned)blocks, 16 * 32, Ka2Cfg<16, 2>::SMEM_BYTES, s>>>(
-                    tm, o->n_streams, n_blocks, o->d_flut, o->d_sum, o->d_max);
-            else
-                ook_block_tma_kernel<16, 2, true><<<(unsigned)blocks, 16 * 32, Ka2Cfg<16, 2>::SMEM_BYTES, s>>>(
-                    tm, o->n_streams, n_blocks, o->d_flut, o->d_sum, o->d_max);
-        }
+    // the capture as a byte tensor [stream][block][1024]: one box = 64 bytes of 32 consecutive blocks of one stream
+    typedef CUresult (*encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
+                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+    CUtensorMap tm;
+    const cuuint64_t dims[3] = {(cuuint64_t)OOK_BLOCK * 2, (cuuint64_t)n_blocks, (cuuint64_t)o->n_streams};
+    const cuuint64_t strides[2] = {(cuuint64_t)OOK_BLOCK * 2, (cuuint64_t)stream_stride_bytes};
+    const cuuint32_t box[3] = {KA2_SLAB_BYTES, 32, 1};
+    const cuuint32_t estr[3] = {1, 1, 1};
+    const CUresult cr = reinterpret_cast<encode_fn>(o->encode_tiled)(
+        &tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<uint8_t *>(d_iq), dims, strides, box, estr,
+        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (cr != CUDA_SUCCESS) {
+        lrc_set_error("lrc_ook_decode: cuTensorMapEncodeTiled -> CUresult %d (n_blocks %zu, n_streams %zu, stride %zu)",
+                      (int)cr, n_blocks, o->n_streams, stream_stride_bytes);
+        return LRC_ERR_CUDA;
     }
+    const size_t ka_blocks = std::min(ceil_div(groups, (size_t)KA2_WARPS), cap);
+    ook_block_tma_kernel<<<(unsigned)ka_blocks, KA2_WARPS * 32, KA2_SMEM_BYTES, s>>>(tm, o->n_streams, n_blocks, o->d_flut,
+                                                                                   o->d_sum, o->d_max);
     LRC_CUDA(cudaGetLastError());
     ook_trigger_kernel<STREAM><<<(unsigned)ceil_div(o->n_streams, (size_t)KB_STREAMS), KB_THREADS, 0, s>>>(
         o->d_sum, o->n_streams, n_blocks, o->max_bursts, o->guard_samples, o->d_tag, o->d_bend, o->d_bflags, o->d_nbursts,
@@ -1747,35 +1430,17 @@ static int ook_launch(lrc_ook *o, const uint8_t *d_iq, size_t n_blocks, size_t s
         o->n_streams, n_blocks, o->max_bursts, o->d_max, o->d_tag, o->d_bend, o->d_bflags, o->d_nbursts, o->d_uniq, o->n_uniq,
         o->d_half, o->d_hrank, o->d_next, (uint32_t)(3 * kc1_blocks * KC1_WARPS), seam, sl ? sl->d_live : nullptr);
     LRC_CUDA(cudaGetLastError());
-    // Which K-C.  Until quiet blocks were skipped the one-warp-per-stream kernel won where an SM had 20 or more streams to itself (its
-    // walk's latency covered by 28 warps); with them skipped the split form wins at every size measured -- whole chain, ms,
-    // one-warp-per-stream / split: 4096 streams 0.596 / 0.571, 3072 0.493 / 0.452, 2048 0.391 / 0.335, 1024 0.292 / 0.220, 512 -- one
-    // GPU's share of 4096 over eight -- 0.253 / 0.163 (profiles/r2_bb_ook_forms.txt) -- and is the default.  LRC_OOK_KC = 0 / 1 forces
-    // one or the other for A/B runs and for the tests that put both through the same cases; identical transition lists.  A stream
-    // plan always runs the split form (the one-warp walk has no carry).
-    const char *kc_s = getenv("LRC_OOK_KC");                              // read at every call: a test runs both forms in one process
-    const int kc_env = kc_s && *kc_s ? atoi(kc_s) : -1;
-    const int kc = STREAM ? 1 : kc_env >= 0 ? kc_env : 1;
-    if (kc == 0) {
-        size_t kc_warps = ceil_div(o->n_streams, (size_t)o->ctx->n_sm);
-        if (kc_warps > KC_THREADS / 32) kc_warps = KC_THREADS / 32;
-        ook_rle_kernel<<<(unsigned)ceil_div(o->n_streams, kc_warps), (unsigned)(kc_warps * 32), OOK_RANK_BYTES, s>>>(
-            d_iq, stream_stride_bytes, o->n_streams, n_blocks, o->max_bursts, o->max_runs, o->d_rank, o->d_tag, o->d_hrank,
-            o->d_half, o->d_max, o->d_bflags, o->d_nbursts, o->d_trans, o->d_ntrans, o->d_nbits);
-        LRC_CUDA(cudaGetLastError());
-    } else {
-        ook_slice_kernel<STREAM><<<(unsigned)kc1_blocks, KC1_WARPS * 32, OOK_RANK_BYTES, s>>>(
-            d_iq, stream_stride_bytes, o->n_streams, n_blocks, o->max_bursts, o->d_rank, o->d_tag, o->d_hrank, o->d_half,
-            o->d_max, o->d_next, o->d_mask, o->d_bsum, carry);
-        LRC_CUDA(cudaGetLastError());
-        ook_scan_kernel<STREAM><<<(unsigned)ceil_div(o->n_streams, (size_t)KC2_WARPS), KC2_WARPS * 32, 0, s>>>(
-            o->n_streams, n_blocks, o->max_bursts, o->max_runs, o->d_tag, o->d_bsum, o->d_bflags, o->d_nbursts, o->d_binfo,
-            o->d_trans, o->d_ntrans, o->d_nbits, carry, seam);
-        LRC_CUDA(cudaGetLastError());
-        ook_scatter_kernel<STREAM><<<(unsigned)ceil_div(slice_groups, (size_t)KC3_WARPS), KC3_WARPS * 32, 0, s>>>(
-            o->n_streams, n_blocks, o->max_runs, o->d_tag, o->d_bsum, o->d_binfo, o->d_mask, o->d_trans, carry);
-        LRC_CUDA(cudaGetLastError());
-    }
+    ook_slice_kernel<STREAM><<<(unsigned)kc1_blocks, KC1_WARPS * 32, OOK_RANK_BYTES, s>>>(
+        d_iq, stream_stride_bytes, o->n_streams, n_blocks, o->max_bursts, o->d_rank, o->d_tag, o->d_hrank, o->d_half,
+        o->d_max, o->d_next, o->d_mask, o->d_bsum, carry);
+    LRC_CUDA(cudaGetLastError());
+    ook_scan_kernel<STREAM><<<(unsigned)ceil_div(o->n_streams, (size_t)KC2_WARPS), KC2_WARPS * 32, 0, s>>>(
+        o->n_streams, n_blocks, o->max_bursts, o->max_runs, o->d_tag, o->d_bsum, o->d_bflags, o->d_nbursts, o->d_binfo,
+        o->d_trans, o->d_ntrans, o->d_nbits, carry, seam);
+    LRC_CUDA(cudaGetLastError());
+    ook_scatter_kernel<STREAM><<<(unsigned)ceil_div(slice_groups, (size_t)KC3_WARPS), KC3_WARPS * 32, 0, s>>>(
+        o->n_streams, n_blocks, o->max_runs, o->d_tag, o->d_bsum, o->d_binfo, o->d_mask, o->d_trans, carry);
+    LRC_CUDA(cudaGetLastError());
     if constexpr (STREAM) {
         // after the slicer has read the carried blocks of a burst sent in this push: the carry may start over
         ook_carry_kernel<<<(unsigned)ceil_div(o->n_streams, (size_t)KCY_WARPS), KCY_WARPS * 32, 0, s>>>(

@@ -528,11 +528,11 @@ def test_trigger_bookkeeping_from_masks_equals_the_blockwise_statements():
     assert n_events > 1000
 
 
-def test_split_slicer_model_equals_the_sequential_walk_and_the_flattened_bit_stream():
+def test_split_slicer_model_equals_the_flattened_bit_stream():
     """ook_slice_kernel / ook_scan_kernel / ook_scatter_kernel place every collected block in the bit stream and in the transition
-    list from per-block summaries and prefix sums, 32 blocks per step; ook_rle_kernel walks the blocks in order.  Both are restated
-    in tools/models/index_models.py and compared with the plainest statement there is: flatten the sent bursts (leading 0.0 bit,
-    lone [0.0] bursts of the OOM guard, abandoned bursts contributing nothing) and record where the value changes (kpn.rs:17-29)."""
+    list from per-block summaries and prefix sums, 32 blocks per step.  That is restated in tools/models/index_models.py and
+    compared with the plainest statement there is: flatten the sent bursts (leading 0.0 bit, lone [0.0] bursts of the OOM guard,
+    abandoned bursts contributing nothing) and record where the value changes (kpn.rs:17-29)."""
     import sys
     import random
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools", "models"))
@@ -587,7 +587,6 @@ def test_split_slicer_model_equals_the_sequential_walk_and_the_flattened_bit_str
     for it in range(120):
         blocks, flags, nb = stream(random.randint(1, 300), random.choice([0, 0.2, 0.5]), it % 3 == 0)
         want = flattened(blocks, flags, nb)
-        assert im.rle_walk(blocks, flags, nb) == want
         assert im.rle_split(blocks, flags, nb) == want
         n_tr += len(want[0])
     assert n_tr > 100_000

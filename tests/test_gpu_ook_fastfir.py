@@ -72,7 +72,7 @@ def check_against_oracle(caps, pk, dbg):
             assert np.array_equal(x, y)
 
 
-def test_ook_decodes_known_packets_bit_exact(ctx, slicer_form):
+def test_ook_decodes_known_packets_bit_exact(ctx):
     caps, sent = [], []
     for s in range(16):
         iq, snt = synth.ook_capture_u8(800, seed=4 + s, n_packets=3)
@@ -90,20 +90,9 @@ def test_ook_decodes_known_packets_bit_exact(ctx, slicer_form):
     assert sum(len(x) for x in sent) == len(pk) > 16
 
 
-@pytest.fixture(params=["default", "one_warp_per_stream", "split"])
-def slicer_form(request, monkeypatch):
-    """the slicer has two forms with identical transition lists (k_ook.cu: ook_rle_kernel / ook_slice + scan + scatter); the split
-    form is the default, LRC_OOK_KC forces one or the other: the edge cases run through both (and through whatever the default is)"""
-    if request.param == "default":
-        monkeypatch.delenv("LRC_OOK_KC", raising=False)
-    else:
-        monkeypatch.setenv("LRC_OOK_KC", "0" if request.param == "one_warp_per_stream" else "1")
-    return request.param
-
-
 @pytest.mark.parametrize("case", ["noise_only", "loud_noise", "ragged_blocks", "all_zero", "saturated", "burst_at_end",
                                   "long_gapped_burst_at_end", "gapped_bursts_sent"])
-def test_ook_edge_cases_match_oracle(ctx, case, slicer_form):
+def test_ook_edge_cases_match_oracle(ctx, case):
     rng = np.random.default_rng(hash(case) % 1000)
     if case == "noise_only":
         caps = [np.clip(np.rint(127 + 1.5 * rng.standard_normal(300 * 1024)), 0, 255).astype(np.uint8) for _ in range(3)]
@@ -142,7 +131,7 @@ def test_ook_edge_cases_match_oracle(ctx, case, slicer_form):
     check_against_oracle(caps, pk, dbg)
 
 
-def test_ook_oom_guard_path_matches_oracle_with_the_guard_shrunk_on_both_sides(ctx, monkeypatch, slicer_form):
+def test_ook_oom_guard_path_matches_oracle_with_the_guard_shrunk_on_both_sides(ctx, monkeypatch):
     """bitfount.rs:52-54: a buffer longer than 1000*50*512 samples is thrown away and collection restarts from [0.0].  The real
     constant needs 100 s of capture per stream, so the test shrinks it to 120 blocks in the oracle AND in the plan (test hooks on
     both sides) and drives every way through the guard: a long loud stretch cut into abandoned pieces whose remainder is sent with
@@ -172,12 +161,12 @@ def test_ook_oom_guard_path_matches_oracle_with_the_guard_shrunk_on_both_sides(c
     check_against_oracle(caps[:6], pk, dbg)
 
 
-def test_ook_quiet_block_boundary_block_maximum_equal_to_half_the_burst_maximum(ctx, slicer_form):
+def test_ook_quiet_block_boundary_block_maximum_equal_to_half_the_burst_maximum(ctx):
     """The slicer does not read a collected block whose maximum does not exceed the burst's max/2 (k_ook.cu, quiet blocks): such a
     block is 512 zeros because `x > max/2` (bitfount.rs:91) is false for x <= max/2 -- INCLUDING equality.  Byte pairs whose envelope
     is exactly half of another pair's exist (2229 of the distinct values): (78, 115) is 0.3972283, (29, 103) twice that.  A burst
     whose maximum is the latter gets one block that peaks exactly at max/2 (all zeros, not read) and one that peaks at the next
-    envelope value above it (one 1 bit: must be read); everything against the oracle, through both slicer forms."""
+    envelope value above it (one 1 bit: must be read); everything against the oracle."""
     env = lambda b0, b1: oracle.norm(oracle.i2f(b0), oracle.i2f(b1))
     top, mid = (29, 103), (78, 115)
     assert np.float32(env(*top)) / np.float32(2) == np.float32(env(*mid))

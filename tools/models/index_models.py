@@ -3,7 +3,7 @@ checked exhaustively on the CPU (tests/test_cpu_oracle.py):
 
 * `ook_fold_index` / `sorted_key_pair` -- the block-sum kernel's folded envelope table (k_ook.cu): one PRMT + VIMNMX.U16x2 sort
   the byte pairs of two samples, `max(key, 65279 - key)` folds the triangle {lo <= hi} into rows 127..255, `k2 + (k2 >> 5)` skews
-  the rows 8 banks apart; the skew is computed as mad.hi by 2^27 + 1.
+  the rows 8 banks apart.
 * `ook_rank_slot` -- the slicer's rank table indexed from the raw halfword.
 * `gen_tile_offsets` / `chunk_plan` -- the padded-chunk tile of the generic fused chain and FIR tile kernel
   (chain_generic.cuh: GenTile, load_sub): where sample j of a thread window lives, which bulk copies a tile takes, and that
@@ -27,9 +27,7 @@ def sorted_key_pair(w: int) -> tuple[int, int]:
 def ook_fold_index(key: int) -> int:
     alt = OOK_FOLD_C - key                                               # negative for hi = 255: loses the SIGNED max
     k2 = max(alt, key)
-    skew = (k2 * ((1 << 27) + 1)) >> 32                                  # mad.hi.u32 by 2^27 + 1
-    assert skew == k2 >> 5
-    return k2 + skew
+    return k2 + (k2 >> 5)                                                # LEA.HI
 
 
 def ook_rank_slot(raw: int) -> int:
@@ -125,44 +123,12 @@ def keeper_send_to_send(tiles, guard_samples, max_bursts):
     return tags, events, state
 
 
-# ---- OOK slicer, split form: summaries -> scan -> scatter against the sequential walk ---------------------------------------
+# ---- OOK slicer: summaries -> scan -> scatter ---------------------------------------------------------------------------------
 # A stream is a list of blocks (tag, bits): tag = index of the burst the block is collected into (-1: not collected), bits = its
 # 512 slicer outputs.  flags[j] of burst j: bit 0 sent, bit 1 the burst starts with the 0.0 of vec!(0.0) (one 0 bit); a burst with
-# flags 3 and no tagged block is the lone [0.0] the OOM guard leaves behind (bitfount.rs:52-54, :78-81).  rle_walk is what
-# ook_rle_kernel does (and kpn::rle on the flattened bit stream, kpn.rs:17-29: a position is recorded where the value changes);
-# rle_split restates ook_slice_kernel's summaries, ook_scan_kernel's 32-block steps with their carry and ook_scatter_kernel.
-def rle_walk(blocks, flags, n_bursts):
-    pos, prev, trans, cur = 0, 0, [], -1
-
-    def zero_bit():
-        nonlocal pos, prev
-        if pos > 0 and prev != 0:
-            trans.append(pos)
-        prev = 0
-        pos += 1
-
-    def lone(frm, to):
-        for j in range(frm, to):
-            if flags[j] & 3 == 3:
-                zero_bit()
-
-    for tag, bits in blocks:
-        if tag < 0:
-            continue
-        if tag != cur:
-            lone(cur + 1, tag)
-            cur = tag
-            if flags[tag] & 2:
-                zero_bit()
-        for b in bits:
-            if pos > 0 and b != prev:
-                trans.append(pos)
-            prev = b
-            pos += 1
-    lone(cur + 1, n_bursts)
-    return trans, pos
-
-
+# flags 3 and no tagged block is the lone [0.0] the OOM guard leaves behind (bitfount.rs:52-54, :78-81).  rle_split restates
+# ook_slice_kernel's summaries, ook_scan_kernel's 32-block steps with their carry and ook_scatter_kernel; the result is kpn::rle on
+# the flattened bit stream (kpn.rs:17-29: a position is recorded where the value changes).
 def rle_split(blocks, flags, n_bursts):
     # C1: per collected block {transitions between its own bits, first bit, last bit}
     summ = [None if t < 0 else (sum(1 for i in range(1, len(b)) if b[i] != b[i - 1]), b[0], b[-1]) for t, b in blocks]
