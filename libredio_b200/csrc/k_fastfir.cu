@@ -7,9 +7,12 @@
 // One CTA owns one block at a time: forward FFT, spectrum multiply and inverse FFT all happen in
 // registers/shared memory (the forward output layout "thread t holds bin t + e*T" is exactly the
 // inverse input layout), so HBM sees nfft reads and ngood writes per block and nothing else.
+//
+// Measured and rejected (round 1, one B200, 4096 taps): fastfir_kernel<13>, the register-resident CTA-level kernel, for
+// 8192-point blocks: 50 300 Msamples/s against 99 400 for fastfir8k_kernel (DESIGN.md, overlap-save rows; SASS in
+// profiles/sass/r1_fastfir_8192.sass and r1_fastfir8k.sass).
 #include "fft_core.cuh"
 #include <cmath>
-#include <cstdlib>
 #include <utility>
 #include <vector>
 
@@ -472,7 +475,6 @@ extern "C" int lrc_fastfir_run(lrc_fastfir *f, const float *d_in, size_t n_in, f
     cudaStream_t s = lrc_stream(f->ctx, stream);
     const float2 *in = (const float2 *)d_in;
     float2 *out = (float2 *)d_out;
-    static const int variant = getenv("LRC_FASTFIR_VARIANT") ? atoi(getenv("LRC_FASTFIR_VARIANT")) : 1;
     if (f->compute16k) {
         // the same full * ngood + keep outputs, cut into 16384-point blocks: every output k < n_total only needs
         // x[k .. k + nh - 1], which the call holds; the last block keeps the remainder and reads zeros past the input
@@ -481,7 +483,7 @@ extern "C" int lrc_fastfir_run(lrc_fastfir *f, const float *d_in, size_t n_in, f
         return lrc_fastfir16k_launch(f->ctx->n_sm, in, n_in, out, full16, full16 + (keep16 ? 1 : 0), ngood16, keep16, f->d_tw,
                                      f->d_tw1k, f->d_Hc, s);
     }
-    if (f->d_Hc && variant == 1) {
+    if (f->log2n == 13) {                 // 8192-point blocks: the plan holds d_Hc for fastfir8k_kernel
         size_t blocks = (size_t)f->ctx->n_sm * 2;
         if (blocks > nblk) blocks = nblk;
         fastfir8k_kernel<<<(unsigned)blocks, ff8k::NT, ff8k::SMEM_BYTES, s>>>(in, n_in, out, full, nblk, f->ngood, keep,
@@ -492,7 +494,7 @@ extern "C" int lrc_fastfir_run(lrc_fastfir *f, const float *d_in, size_t n_in, f
     switch (f->log2n) {
 #define FF_CASE(L) case L: return launch_fastfir<L>(f, in, n_in, out, full, nblk, keep, s);
         FF_CASE(1) FF_CASE(2) FF_CASE(3) FF_CASE(4) FF_CASE(5) FF_CASE(6) FF_CASE(7)
-        FF_CASE(8) FF_CASE(9) FF_CASE(10) FF_CASE(11) FF_CASE(12) FF_CASE(13)
+        FF_CASE(8) FF_CASE(9) FF_CASE(10) FF_CASE(11) FF_CASE(12)
 #undef FF_CASE
     }
     return LRC_ERR_UNSUPPORTED;

@@ -35,6 +35,8 @@ using namespace lrfft;
 
 namespace ff16k {
 constexpr int N = 16384, NPAIR = 512, ROWS = 16;
+constexpr int NT = NPAIR;                        // one column pair per thread, one row per warp
+static_assert(NT / 32 == ROWS, "one row per warp");
 constexpr int LP = 34;                          // entries per lane slab (32 used)
 constexpr int RP = 32 * LP;                     // entries per row
 constexpr int DATA_CPX = ROWS * RP;
@@ -100,21 +102,19 @@ __device__ __forceinline__ void warp_fft1024(float2 *v, float2 *row, const float
 //   - staging the next block's first column in shared memory with cp.async during P2 (P1 twiddles factorised into two
 //     small tables to make room): 121 Gsamples/s against 140 -- 8192 LDGSTS per CTA sit in the LSU queue in front of the
 //     barrier (lg_throttle 0.12 -> 0.79, barrier 0.63 -> 1.07 per issue), profiles/r2_ff16k_staged_ncu_phases.txt;
-//   - a CTA-uniform fast path with unpredicated loads: 133 against 140.
+//   - a CTA-uniform fast path with unpredicated loads: 133 against 140;
+//   - 256 threads with two column pairs and two rows each at 255 registers, room to request a whole pair of the next block
+//     before P2 and the other at the head of the P1 phase, with half the warps to hide everything else: timed against
+//     512 threads in tools/runs/r2c.sh, whose 512-thread captures are profiles/r2_r2c_ff16k_512_ncu_keys.txt and
+//     r2_r2c_ff16k_512_ncu_phases.txt.
 // A TMA tensor copy would take the loads off the LSU, but block starts (multiples of ngood = 12289 samples) are only
 // 8-byte aligned every other block.
-//
-// NT = 512: one column pair and one row per thread / warp, 128 registers.  NT = 256: two pairs and two rows, 255 registers --
-// room to request a whole pair of the next block BEFORE P2 and the other pair at the head of the P1 phase, so no load is
-// ever waited for; half the warps to hide everything else.  Chosen by measurement (lrc_fastfir16k_launch).
-template <int NT>
-__global__ void __launch_bounds__(NT, 1)
+__global__ void __launch_bounds__(ff16k::NT, 1)
 fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict__ out, size_t n_blocks_full,
                   size_t n_blocks, size_t ngood, size_t flush_keep, const float2 *__restrict__ tw /* W_16384^k */,
                   const float2 *__restrict__ tw1k /* W_1024^k */, const float4 *__restrict__ Hq)
 {
     using namespace ff16k;
-    constexpr int NW = NT / 32, PAIRS = NPAIR / NT, RPW = ROWS / NW;          // warps, pairs per thread, rows per warp
     extern __shared__ __align__(16) float2 ff16k_smem[];
     float2 *sd = ff16k_smem;                         // [16][RP]
     float2 *tw1 = sd + DATA_CPX;                     // [512 pairs][T1P]
@@ -131,13 +131,12 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
     }
     __syncthreads();
 
-    // pair p of this thread: pair index pr = t + NT p = lane + 32 j, columns ca = lane + 64 j and ca + 32,
-    // cells (row q) at sd[q RP + lane LP + 2 j] (.lo = column ca, .hi = column ca + 32)
-    auto col_a = [&](int p) { return lane + 64 * (warp + NW * p); };
-    auto twp_of = [&](int p) { return reinterpret_cast<const float4 *>(tw1 + (t + NT * p) * T1P); };
-    auto cell_of = [&](int p) { return reinterpret_cast<float4 *>(sd + lane * LP + 2 * (warp + NW * p)); };
+    // this thread's pair: pair index t = lane + 32 warp, columns ca = lane + 64 warp and ca + 32,
+    // cells (row q) at sd[q RP + lane LP + 2 warp] (.lo = column ca, .hi = column ca + 32)
+    auto twp_of = [&]() { return reinterpret_cast<const float4 *>(tw1 + t * T1P); };
+    auto cell_of = [&]() { return reinterpret_cast<float4 *>(sd + lane * LP + 2 * warp); };
 
-    // the 2 x 16 inputs of a column pair of block `blk`; volatile loads: they stay where they are written
+    // the 2 x 16 inputs of the column pair of block `blk`; volatile loads: they stay where they are written
     auto p1_load = [&](size_t blk, int ca, float2 *va, float2 *vb) {
         const size_t s0 = blk * ngood;
         const float2 *src = in + s0 + ca;
@@ -156,10 +155,10 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
             }
         }
     };
-    // forward butterflies of a column pair; results into the pair's 16 shared cells
-    auto p1_forward = [&](int p, float2 *va, float2 *vb) {
-        const float4 *twp = twp_of(p);
-        float4 *cell = cell_of(p);
+    // forward butterflies of the column pair; results into the pair's 16 shared cells
+    auto p1_forward = [&](float2 *va, float2 *vb) {
+        const float4 *twp = twp_of();
+        float4 *cell = cell_of();
         RegFFT<16, false>::run(va);
         RegFFT<16, false>::run(vb);
 #pragma unroll
@@ -176,9 +175,9 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
         }
     };
     // inverse side of a pair, part 1: cells -> registers, conjugated twiddles
-    auto p1_unload = [&](int p, float2 *ua, float2 *ub) {
-        const float4 *twp = twp_of(p);
-        const float4 *cell = cell_of(p);
+    auto p1_unload = [&](float2 *ua, float2 *ub) {
+        const float4 *twp = twp_of();
+        const float4 *cell = cell_of();
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
             const float4 w = twp[i];
@@ -203,12 +202,9 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
 
     size_t b = blockIdx.x;
     if (b < n_blocks) {
-#pragma unroll
-        for (int p = 0; p < PAIRS; ++p) {
-            float2 va[16], vb[16];
-            p1_load(b, col_a(p), va, vb);
-            p1_forward(p, va, vb);
-        }
+        float2 va[16], vb[16];
+        p1_load(b, lane + 64 * warp, va, vb);
+        p1_forward(va, vb);
     }
     for (; b < n_blocks; b += gridDim.x) {
         const size_t nb = b + gridDim.x;
@@ -222,13 +218,10 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
                 if (nb * ngood * 8 + off < n_in * 8) asm volatile("prefetch.global.L2 [%0];" :: "l"(nsrc + off));
             }
         }
-        float2 nxa[16], nxb[16];
-        if (NT == 256 && more) p1_load(nb, col_a(0), nxa, nxb);   // in flight across the whole of P2
         __syncthreads();
-        // ---- P2: a warp transforms its rows, multiplies by its slice of H, transforms back -------------------
-#pragma unroll 1
-        for (int rr = 0; rr < RPW; ++rr) {
-            const int k1 = warp + NW * rr;
+        // ---- P2: warp k1 transforms row k1, multiplies by its slice of H, transforms back ----------------------
+        {
+            const int k1 = warp;
             float2 *row = sd + RP * k1;
             float4 *slab4 = reinterpret_cast<float4 *>(row + lane * LP);
             float2 v[32];
@@ -255,47 +248,26 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
         // ---- P1 inverse of this block fused with P1 forward of the CTA's next block -----------------------
         const int keep = (int)((b < n_blocks_full) ? ngood : flush_keep);
         float2 *dstg = out + b * ngood;
-        if (NT == 256) {
-            // pair 1 of the next block is requested now and used after all of pair 0's butterflies
-            float2 nya[16], nyb[16];
-            if (more) p1_load(nb, col_a(1), nya, nyb);
-            asm volatile("" ::: "memory");
-            {
-                float2 ua[16], ub[16];
-                p1_unload(0, ua, ub);
-                p1_emit(ua, dstg + col_a(0), col_a(0), keep);
-                p1_emit(ub, dstg + col_a(0) + 32, col_a(0) + 32, keep);
-            }
-            if (more) p1_forward(0, nxa, nxb);
-            {
-                float2 ua[16], ub[16];
-                p1_unload(1, ua, ub);
-                p1_emit(ua, dstg + col_a(1), col_a(1), keep);
-                p1_emit(ub, dstg + col_a(1) + 32, col_a(1) + 32, keep);
-            }
-            if (more) p1_forward(1, nya, nyb);
-        } else {
-            // 128 registers: ua, ub, nxa, nxb are 32 each, so a column of the next block is requested only once a
-            // column of this block has left
-            const int ca = col_a(0);
-            const float2 *src = in + nb * ngood + ca;
-            // (one predicated form for whole and ragged blocks: splitting it into a CTA-uniform fast path with
-            // unpredicated loads measured 5 % SLOWER, 133 vs 140 Gsamples/s -- the phase waits on memory, not on issue)
-            const bool whole = more && n_in - nb * ngood >= (size_t)N;
-            const int avail = more ? (whole ? N : (int)(n_in - nb * ngood)) : 0;
-            float2 ua[16], ub[16];
-            p1_unload(0, ua, ub);
-            p1_emit(ua, dstg + ca, ca, keep);
-            asm volatile("" ::: "memory");
+        // 128 registers: ua, ub, nxa, nxb are 32 each, so a column of the next block is requested only once a
+        // column of this block has left
+        const int ca = lane + 64 * warp;
+        const float2 *src = in + nb * ngood + ca;
+        // (one predicated form for whole and ragged blocks: splitting it into a CTA-uniform fast path with
+        // unpredicated loads measured 5 % SLOWER, 133 vs 140 Gsamples/s -- the phase waits on memory, not on issue)
+        const bool whole = more && n_in - nb * ngood >= (size_t)N;
+        const int avail = more ? (whole ? N : (int)(n_in - nb * ngood)) : 0;
+        float2 ua[16], ub[16], nxa[16], nxb[16];
+        p1_unload(ua, ub);
+        p1_emit(ua, dstg + ca, ca, keep);
+        asm volatile("" ::: "memory");
 #pragma unroll
-            for (int r = 0; r < 16; ++r) nxa[r] = (whole || ca + 1024 * r < avail) ? ldg_nc_f2(src + 1024 * r) : make_float2(0.f, 0.f);
-            p1_emit(ub, dstg + ca + 32, ca + 32, keep);
-            asm volatile("" ::: "memory");
+        for (int r = 0; r < 16; ++r) nxa[r] = (whole || ca + 1024 * r < avail) ? ldg_nc_f2(src + 1024 * r) : make_float2(0.f, 0.f);
+        p1_emit(ub, dstg + ca + 32, ca + 32, keep);
+        asm volatile("" ::: "memory");
 #pragma unroll
-            for (int r = 0; r < 16; ++r)
-                nxb[r] = (whole || ca + 32 + 1024 * r < avail) ? ldg_nc_f2(src + 1024 * r + 32) : make_float2(0.f, 0.f);
-            if (more) p1_forward(0, nxa, nxb);
-        }
+        for (int r = 0; r < 16; ++r)
+            nxb[r] = (whole || ca + 32 + 1024 * r < avail) ? ldg_nc_f2(src + 1024 * r + 32) : make_float2(0.f, 0.f);
+        if (more) p1_forward(nxa, nxb);
     }
 }
 
@@ -312,8 +284,7 @@ void lrc_fastfir16k_permute_H(const float2 *H, float2 *Hq)
 
 int lrc_fastfir16k_prepare(void)
 {
-    LRC_CUDA(cudaFuncSetAttribute(fastfir16k_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, ff16k::SMEM_BYTES));
-    LRC_CUDA(cudaFuncSetAttribute(fastfir16k_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, ff16k::SMEM_BYTES));
+    LRC_CUDA(cudaFuncSetAttribute(fastfir16k_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ff16k::SMEM_BYTES));
     return LRC_OK;
 }
 
@@ -322,12 +293,8 @@ int lrc_fastfir16k_launch(int n_sm, const float2 *in, size_t n_in, float2 *out, 
 {
     size_t blocks = (size_t)n_sm;                    // one CTA per SM (216.5 KB of shared memory)
     if (blocks > nblk) blocks = nblk;
-    static const int nt = getenv("LRC_FASTFIR16K_THREADS") ? atoi(getenv("LRC_FASTFIR16K_THREADS")) : 512;
-    const float4 *hq = reinterpret_cast<const float4 *>(d_Hq);
-    if (nt == 256)
-        fastfir16k_kernel<256><<<(unsigned)blocks, 256, ff16k::SMEM_BYTES, s>>>(in, n_in, out, full, nblk, ngood, keep, d_tw16k, d_tw1k, hq);
-    else
-        fastfir16k_kernel<512><<<(unsigned)blocks, 512, ff16k::SMEM_BYTES, s>>>(in, n_in, out, full, nblk, ngood, keep, d_tw16k, d_tw1k, hq);
+    fastfir16k_kernel<<<(unsigned)blocks, ff16k::NT, ff16k::SMEM_BYTES, s>>>(in, n_in, out, full, nblk, ngood, keep, d_tw16k,
+                                                                          d_tw1k, reinterpret_cast<const float4 *>(d_Hq));
     LRC_CUDA(cudaGetLastError());
     return LRC_OK;
 }

@@ -2,9 +2,19 @@
 //
 // Replaces: kissfft::fft block + kiss_fft_alloc/kiss_fft (src/kissfft/src/kissfft.rs:11-31,
 // libkissfft/kiss_fft.c:339-388); |X|^2 averaging after tools/psdpng.c:157-178.
+//
+// Measured and rejected at 1024 points (Gsamples/s, one B200):
+//   - the CTA-level TMA-ring kernels (fft_tma_kernel, psd_tma_kernel) that the warp-per-transform kernels replaced:
+//     FFT 357.6 and PSD 547.2 (profiles/r1_s3_kernels_table.jsonl) against 422.1 and 657.1 (r1_s8_kernels_table.jsonl);
+//   - psd1024_warp_kernel without the L2 prefetch of the next frame (644.0 against 657.0), with an L1 prefetch (657.9,
+//     no gain) and bounded for 4 CTAs per SM (624.8 / 623.4) (profiles/r1_s8_grid_sweeps.txt);
+//   - psd1024_warp_db_kernel, the next frame double-buffered in registers: 589.0 at 2 CTAs x 4 warps, 566.8 at 1 x 8
+//     (r1_s8_grid_sweeps.txt), 519.2 at 3 x 4 (r1_s6_psd_variants.txt);
+//   - the folded window and shared-memory accumulators of profiles/r2_psd_variants.txt.
+// psd_tma_kernel (512 and 2048 points) also had 2-stage rings at 3 or 4 CTAs per SM and (re^2, im^2) accumulated apart with
+// one FFMA2 per bin at 2 CTAs per SM; no recorded measurement put them ahead of 3 stages at 3 CTAs.
 #include "fft_core.cuh"
 #include <cmath>
-#include <cstdlib>
 #include <vector>
 
 using namespace lrfft;
@@ -180,28 +190,29 @@ fft1024_warp_kernel(const float2 *__restrict__ in, float2 *__restrict__ out, siz
     }
 }
 
+// N = 1024 always runs the warp kernel, so launch_fft is never instantiated for it
+template <bool INV>
+static int launch_fft1024(const lrc_fft *p, const float2 *in, float2 *out, size_t batch, cudaStream_t s)
+{
+    auto kern = fft1024_warp_kernel<INV>;
+    LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, FFTW_SMEM_BYTES));
+    int occ = 1;
+    LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, FFTW_WARPS * 32, FFTW_SMEM_BYTES));
+    if (occ < 1) occ = 1;
+    size_t blocks = ceil_div(batch, (size_t)FFTW_WARPS);
+    static const size_t gm = lrc_grid_mult("LRC_FFT_GRID", 32);
+    const size_t max_blocks = (size_t)p->ctx->n_sm * occ * gm;
+    if (blocks > max_blocks) blocks = max_blocks;
+    kern<<<(unsigned)blocks, FFTW_WARPS * 32, FFTW_SMEM_BYTES, s>>>(in, out, batch, p->d_tw);
+    LRC_CUDA(cudaGetLastError());
+    return LRC_OK;
+}
+
 template <int LOG2N, bool INV>
 static int launch_fft(const lrc_fft *p, const float2 *in, float2 *out, size_t batch, cudaStream_t s)
 {
     using F = CtaFFT<LOG2N, INV>;
     constexpr int T = F::T;
-    if constexpr (LOG2N == 10) {
-        static const int variant = getenv("LRC_FFT_VARIANT") ? atoi(getenv("LRC_FFT_VARIANT")) : 0;
-        if (variant == 0) {
-            auto kern = fft1024_warp_kernel<INV>;
-            LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, FFTW_SMEM_BYTES));
-            int occ = 1;
-            LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, FFTW_WARPS * 32, FFTW_SMEM_BYTES));
-            if (occ < 1) occ = 1;
-            size_t blocks = ceil_div(batch, (size_t)FFTW_WARPS);
-            static const size_t gm = lrc_grid_mult("LRC_FFT_GRID", 32);
-            const size_t max_blocks = (size_t)p->ctx->n_sm * occ * gm;
-            if (blocks > max_blocks) blocks = max_blocks;
-            kern<<<(unsigned)blocks, FFTW_WARPS * 32, FFTW_SMEM_BYTES, s>>>(in, out, batch, p->d_tw);
-            LRC_CUDA(cudaGetLastError());
-            return LRC_OK;
-        }
-    }
     if constexpr (T >= 32 && T <= 128) {
         // in-place calls are safe here too: a frame is fully in shared memory before its slot is written
         if (((uintptr_t)in & 15) == 0 && batch >= 64) {
@@ -245,7 +256,7 @@ static int dispatch_fft(const lrc_fft *p, const float2 *in, float2 *out, size_t 
         case 7:  return launch_fft<7, INV>(p, in, out, batch, s);
         case 8:  return launch_fft<8, INV>(p, in, out, batch, s);
         case 9:  return launch_fft<9, INV>(p, in, out, batch, s);
-        case 10: return launch_fft<10, INV>(p, in, out, batch, s);
+        case 10: return launch_fft1024<INV>(p, in, out, batch, s);
         case 11: return launch_fft<11, INV>(p, in, out, batch, s);
         case 12: return launch_fft<12, INV>(p, in, out, batch, s);
         case 13: return launch_fft<13, INV>(p, in, out, batch, s);
@@ -388,11 +399,11 @@ psd_kernel(const float2 *__restrict__ in, const float2 *__restrict__ tw, const f
 // Same work, frames staged by the TMA engine: every transform group owns a PSD_STAGES-deep ring of frame
 // buffers in shared memory; its leader thread keeps PSD_STAGES-1 bulk copies in flight while the group
 // transforms the current frame, so HBM latency is hidden inside the group instead of by occupancy alone.
-// Used for N = 512..2048 (T = 32..128 threads per transform) when the input is 16-byte aligned.
+// Used for N = 512 and 2048 (T = 32 and 128 threads per transform) when the input is 16-byte aligned.
+constexpr int PSD_STAGES = 3;
 
-template <int LOG2N, int PSD_STAGES>
+template <int LOG2N>
 struct PsdTmaCfg {
-    static constexpr int STAGES = PSD_STAGES;
     using F = CtaFFT<LOG2N, false>;
     static constexpr int THREADS = F::T > 128 ? F::T : 128;
     static constexpr int G = THREADS / F::T;
@@ -401,12 +412,12 @@ struct PsdTmaCfg {
     static constexpr int SMEM_BYTES = G * GROUP_BYTES;
 };
 
-template <int LOG2N, int PSD_STAGES, int MINB, bool PACKACC>
-__global__ void __launch_bounds__(PsdTmaCfg<LOG2N, PSD_STAGES>::THREADS, MINB)
+template <int LOG2N>
+__global__ void __launch_bounds__(PsdTmaCfg<LOG2N>::THREADS, 3)
 psd_tma_kernel(const float2 *__restrict__ in, const float2 *__restrict__ tw, const float *__restrict__ win,
                float *__restrict__ partial, size_t k_avg, size_t fpi, size_t ipr, size_t n_items)
 {
-    using Cfg = PsdTmaCfg<LOG2N, PSD_STAGES>;
+    using Cfg = PsdTmaCfg<LOG2N>;
     using F = CtaFFT<LOG2N, false>;
     constexpr int N = F::N, E = F::E, T = F::T, G = Cfg::G;
     extern __shared__ __align__(128) uint8_t psd_smem[];
@@ -458,11 +469,9 @@ psd_tma_kernel(const float2 *__restrict__ in, const float2 *__restrict__ tw, con
     if (t == 0)
         for (int i = 0; i < PSD_STAGES - 1 && ahead.item < n_items; ++i) request();
 
-    // PACKACC: (sum re^2, sum im^2) kept apart, one FFMA2 per bin per frame (fewer issue slots, 16 more
-    // registers); otherwise one float per bin, two FFMA (same FP32-pipe cycles)
-    float2 acc[E];
+    float acc[E];
 #pragma unroll
-    for (int e = 0; e < E; ++e) acc[e] = make_float2(0.f, 0.f);
+    for (int e = 0; e < E; ++e) acc[e] = 0.f;
     for (int i = 0; cur.item < n_items; ++i) {
         const int stage = i % PSD_STAGES;
         // the stage being refilled now was read (into registers) one iteration ago, and every thread has
@@ -478,14 +487,11 @@ psd_tma_kernel(const float2 *__restrict__ in, const float2 *__restrict__ tw, con
         }
         F::run_twreg(v, sm, twr, t, SyncNamed{1 + g, T});
 #pragma unroll
-        for (int e = 0; e < E; ++e) {
-            if constexpr (PACKACC) acc[e] = fma2(v[e], v[e], acc[e]);
-            else acc[e].x = fmaf(v[e].x, v[e].x, fmaf(v[e].y, v[e].y, acc[e].x));
-        }
+        for (int e = 0; e < E; ++e) acc[e] = fmaf(v[e].x, v[e].x, fmaf(v[e].y, v[e].y, acc[e]));
         if (cur.f + 1 == cur.f1) {                        // last frame of the item: hand the partial spectrum out
             float *dst = partial + cur.item * N + t;
 #pragma unroll
-            for (int e = 0; e < E; ++e) { dst[e * T] = PACKACC ? acc[e].x + acc[e].y : acc[e].x; acc[e] = make_float2(0.f, 0.f); }
+            for (int e = 0; e < E; ++e) { dst[e * T] = acc[e]; acc[e] = 0.f; }
         }
         advance(cur);
     }
@@ -503,13 +509,7 @@ __device__ __forceinline__ void prefetch_l2(const void *p)
     asm volatile("prefetch.global.L2 [%0];" :: "l"(p));
 }
 
-__device__ __forceinline__ void prefetch_l1(const void *p)
-{
-    asm volatile("prefetch.global.L1 [%0];" :: "l"(p));
-}
-
-template <int MINB, int PF>
-__global__ void __launch_bounds__(PSDW_WARPS * 32, MINB)
+__global__ void __launch_bounds__(PSDW_WARPS * 32, 3)
 psd1024_warp_kernel(const float2 *__restrict__ in, const float2 *__restrict__ tw, const float *__restrict__ win,
                     float *__restrict__ partial, size_t k_avg, size_t fpi, size_t ipr, size_t n_items)
 {
@@ -550,8 +550,7 @@ psd1024_warp_kernel(const float2 *__restrict__ in, const float2 *__restrict__ tw
                 const bool more = f + 1 < f1;
                 if (more || has_next) {
                     const char *nx = reinterpret_cast<const char *>(in + (more ? f + 1 : fnext_item) * N) + lane * 256;
-                    if (PF == 1) { prefetch_l2(nx); prefetch_l2(nx + 128); }
-                    if (PF == 2) { prefetch_l1(nx); prefetch_l1(nx + 128); }
+                    prefetch_l2(nx); prefetch_l2(nx + 128);
                 }
             }
 #pragma unroll
@@ -566,83 +565,6 @@ psd1024_warp_kernel(const float2 *__restrict__ in, const float2 *__restrict__ tw
         float *dst = partial + item * N + lane;
 #pragma unroll
         for (int e = 0; e < 32; ++e) dst[32 * e] = acc[e];
-    }
-}
-
-// Same transform, frames double-buffered in REGISTERS: the 32 loads of the warp's next frame are issued before
-// the current frame is transformed, so a full frame of arithmetic (~760 issue slots) covers the HBM latency and
-// no warp ever sits in a pure load phase.  Costs 64 more registers (2 CTAs of 4 warps per SM instead of 3).
-// The frame loop is unrolled by two so the buffers ping-pong without register moves.
-template <int MINB, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-psd1024_warp_db_kernel(const float2 *__restrict__ in, const float2 *__restrict__ tw, const float *__restrict__ win,
-                       float *__restrict__ partial, size_t k_avg, size_t fpi, size_t ipr, size_t n_items)
-{
-    using F = WarpFFT1024<false>;
-    constexpr int N = 1024;
-    extern __shared__ __align__(16) float2 psdw_sm[];
-    float2 *tws = psdw_sm + WARPS * F::SMEM_CPX;
-    float *wsm = reinterpret_cast<float *>(tws + F::TW_CPX);
-    for (int i = threadIdx.x; i < N; i += blockDim.x) wsm[i] = win[i];
-    F::fill_twiddles(tw, tws);
-    __syncthreads();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    float2 *xb = psdw_sm + warp * F::SMEM_CPX;
-    const float *wl = wsm + lane;
-    const size_t stride = (size_t)gridDim.x * WARPS;
-
-    struct Cur { size_t item, f, f1; bool valid; };
-    auto setup = [&](size_t item) -> Cur {
-        Cur c;
-        c.item = item;
-        c.valid = item < n_items;
-        const size_t row = item / ipr, col = item % ipr;
-        c.f = row * k_avg + col * fpi;
-        c.f1 = c.f + fpi;
-        if (c.f1 > (row + 1) * k_avg) c.f1 = (row + 1) * k_avg;
-        return c;
-    };
-    auto next_of = [&](const Cur &c) -> Cur {
-        if (c.f + 1 < c.f1) { Cur n = c; n.f = c.f + 1; return n; }
-        return setup(c.item + stride);
-    };
-    auto load = [&](float2 *b, const Cur &c) {
-        if (c.valid) {
-            const float2 *src = in + c.f * N + lane;
-#pragma unroll
-            for (int e = 0; e < 32; ++e) b[e] = __ldcs(src + 32 * e);
-        }
-    };
-    float acc[32];
-#pragma unroll
-    for (int e = 0; e < 32; ++e) acc[e] = 0.f;
-    auto compute = [&](float2 *v, const Cur &c) {
-#pragma unroll
-        for (int e = 0; e < 32; ++e) {
-            const float w = wl[32 * e];
-            v[e] = mul2(v[e], make_float2(w, w));
-        }
-        F::run(v, xb, tws, lane);
-#pragma unroll
-        for (int e = 0; e < 32; ++e) acc[e] = fmaf(v[e].x, v[e].x, fmaf(v[e].y, v[e].y, acc[e]));
-        if (c.f + 1 == c.f1) {
-            float *dst = partial + c.item * N + lane;
-#pragma unroll
-            for (int e = 0; e < 32; ++e) { dst[32 * e] = acc[e]; acc[e] = 0.f; }
-        }
-    };
-
-    float2 a[32], b[32];
-    Cur cur = setup((size_t)blockIdx.x * WARPS + warp);
-    load(a, cur);
-    while (cur.valid) {
-        const Cur nxt = next_of(cur);
-        load(b, nxt);
-        compute(a, cur);
-        if (!nxt.valid) break;
-        cur = next_of(nxt);
-        load(a, cur);
-        compute(b, nxt);
     }
 }
 
@@ -667,9 +589,22 @@ static int launch_psd(lrc_psd *p, const float2 *in, size_t k_avg, size_t fpi, si
     constexpr int T = F::T;
     if constexpr (T >= 32 && T <= 128) {            // N = 512 .. 2048: the ring fits several CTAs per SM
         if (((uintptr_t)in & 15) == 0) {
-            static const int variant = getenv("LRC_PSD_VARIANT") ? atoi(getenv("LRC_PSD_VARIANT")) : 0;
-            auto go = [&](auto kern, auto cfg) -> int {
-                using Cfg = decltype(cfg);
+            if constexpr (LOG2N == 10) {
+                auto kern = psd1024_warp_kernel;
+                LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, PSDW_SMEM_BYTES));
+                int occ = 1;
+                LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, PSDW_WARPS * 32, PSDW_SMEM_BYTES));
+                if (occ < 1) occ = 1;
+                size_t blocks = ceil_div(n_items, (size_t)PSDW_WARPS);
+                static const size_t gm = lrc_grid_mult("LRC_PSD_GRID", 16);
+                const size_t max_blocks = (size_t)p->ctx->n_sm * occ * gm;
+                if (blocks > max_blocks) blocks = max_blocks;
+                kern<<<(unsigned)blocks, PSDW_WARPS * 32, PSDW_SMEM_BYTES, s>>>(in, p->d_tw, p->d_win, p->d_partial, k_avg, fpi, ipr, n_items);
+                LRC_CUDA(cudaGetLastError());
+                return LRC_OK;
+            } else {
+                using Cfg = PsdTmaCfg<LOG2N>;
+                auto kern = psd_tma_kernel<LOG2N>;
                 LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
                 int occ = 1;
                 LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, Cfg::THREADS, Cfg::SMEM_BYTES));
@@ -680,40 +615,6 @@ static int launch_psd(lrc_psd *p, const float2 *in, size_t k_avg, size_t fpi, si
                 kern<<<(unsigned)blocks, Cfg::THREADS, Cfg::SMEM_BYTES, s>>>(in, p->d_tw, p->d_win, p->d_partial, k_avg, fpi, ipr, n_items);
                 LRC_CUDA(cudaGetLastError());
                 return LRC_OK;
-            };
-            if constexpr (LOG2N == 10) {
-                if (variant == 0 || variant >= 10) {
-                    auto launch_w = [&](auto kern, int warps = PSDW_WARPS) -> int {
-                        const int smem = (warps * WarpFFT1024<false>::SMEM_CPX + WarpFFT1024<false>::TW_CPX) * 8 + 1024 * 4;
-                        LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-                        int occ = 1;
-                        LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, warps * 32, smem));
-                        if (occ < 1) occ = 1;
-                        size_t blocks = ceil_div(n_items, (size_t)warps);
-                        static const size_t gm = lrc_grid_mult("LRC_PSD_GRID", 16);
-                        const size_t max_blocks = (size_t)p->ctx->n_sm * occ * gm;
-                        if (blocks > max_blocks) blocks = max_blocks;
-                        kern<<<(unsigned)blocks, warps * 32, smem, s>>>(in, p->d_tw, p->d_win, p->d_partial, k_avg, fpi, ipr, n_items);
-                        LRC_CUDA(cudaGetLastError());
-                        return LRC_OK;
-                    };
-                    switch (variant) {
-                        case 10: return launch_w(psd1024_warp_kernel<3, 0>);
-                        case 11: return launch_w(psd1024_warp_kernel<4, 1>);
-                        case 12: return launch_w(psd1024_warp_kernel<3, 2>);
-                        case 13: return launch_w(psd1024_warp_kernel<4, 2>);
-                        case 14: return launch_w(psd1024_warp_db_kernel<2, 4>, 4);
-                        case 15: return launch_w(psd1024_warp_db_kernel<1, 8>, 8);
-                        case 16: return launch_w(psd1024_warp_db_kernel<3, 4>, 4);
-                        default: return launch_w(psd1024_warp_kernel<3, 1>);
-                    }
-                }
-            }
-            switch (variant) {      // tuning variants (tools/bench_kernels.py); 0 is the shipped one
-                case 1: return go(psd_tma_kernel<LOG2N, 2, 4, false>, PsdTmaCfg<LOG2N, 2>{});
-                case 2: return go(psd_tma_kernel<LOG2N, 3, 2, true>, PsdTmaCfg<LOG2N, 3>{});
-                case 3: return go(psd_tma_kernel<LOG2N, 2, 3, false>, PsdTmaCfg<LOG2N, 2>{});
-                default: return go(psd_tma_kernel<LOG2N, 3, 3, false>, PsdTmaCfg<LOG2N, 3>{});   // also variant 4
             }
         }
     }
@@ -807,10 +708,9 @@ extern "C" int lrc_psd_run(lrc_psd *p, const float *d_in, size_t n_frames, size_
     LRC_REQUIRE(d_in && d_rows, LRC_ERR_INVALID, "lrc_psd_run: null buffer");
     LRC_REQUIRE(((uintptr_t)d_in & 7) == 0, LRC_ERR_INVALID, "lrc_psd_run: input must be 8-byte aligned");
     cudaStream_t s = lrc_stream(p->ctx, stream);
-    size_t fpi = lrc_psd_frames_per_item(k_avg);
     // the grouping of frames into items is a function of k_avg alone, so results do not depend on the launch
     // or on how a stream is sharded (finer items were measured slower: 16 -> 8 costs 2 %, -> 4 costs 9 %)
-    if (const char *e = getenv("LRC_PSD_FPI")) { const size_t v = (size_t)atoi(e); if (v >= 1 && v <= k_avg) fpi = v; }
+    const size_t fpi = lrc_psd_frames_per_item(k_avg);
     const size_t ipr = ceil_div(k_avg, fpi);
     const size_t n_items = n_rows * ipr;
     int rc = lrc_psd_ensure_partial(&p->d_partial, &p->partial_cap, n_items * (size_t)p->nfft);

@@ -7,6 +7,11 @@
 //     ratio = L/M;  prototype h: ntaps = 2*32*max(L,M)+1, sinc(2 fc (i-c)) * kaiser(beta=12),
 //     fc = 0.45/max(L,M), sum(h) = L;
 //     y[m] = sum_j h[(mM mod L) + jL] * x[floor(mM/L) - j],  x[<0] = 0   (streaming-causal).
+//
+// Measured and rejected for the packed decimator at M = 5 (the BASELINE 240 kHz -> 48 kHz shape, 1024 channels x 240 k
+// samples, profiles/r1_s8_rs_configs.txt, Gsamples/s): 128 threads (380), and a second cp.async stage that fills the next
+// tile pair while this one is filtered, at 64 threads (359) and at 128 (351), against 64 threads and one stage (387).
+// The second stage halves the resident CTAs and loses more than the hidden fill gains.
 #include "fm_core.cuh"
 #include <cmath>
 #include <cstdlib>
@@ -354,14 +359,14 @@ struct RsTileSrc {
     }
 };
 
-template <int M, int R, int NT, int STAGES>
+template <int M, int R, int NT>
 __global__ void __launch_bounds__(NT)
 resample_dec2_kernel(const float *__restrict__ carry, const float *__restrict__ in, size_t n_in, size_t in_stride,
                      size_t n_ch, size_t s0, size_t n_out,
                      float *__restrict__ out, size_t out_stride, const __grid_constant__ RsTaps<2 * RS_ZERO_CROSSINGS * M + 1> taps)
 {
     using Cfg = RsDec2Cfg<M, R, NT>;
-    extern __shared__ __align__(16) float2 rs_tile2[];           // STAGES buffers of TILE_IN pairs
+    extern __shared__ __align__(16) float2 rs_tile2[];           // TILE_IN pairs
     const int t = threadIdx.x;
     const size_t tiles_per_ch = (n_out + Cfg::TILE_OUT - 1) / Cfg::TILE_OUT;
     const size_t n_tiles = tiles_per_ch * n_ch;
@@ -375,7 +380,7 @@ resample_dec2_kernel(const float *__restrict__ carry, const float *__restrict__ 
         s.row = RsRow{carry + *c * (size_t)Cfg::TPP, (size_t)(Cfg::TPP - 1), in + *c * in_stride, n_in};
         return s;
     };
-    // Fill one stage with the tile pair `pair`: asynchronous 4-byte copies (LDGSTS) straight into the interleaved
+    // Fill the tile with the tile pair `pair`: asynchronous 4-byte copies (LDGSTS) straight into the interleaved
     // tile, zero-filled past the end of a row, one commit group per fill.  All loads of a thread are in flight at
     // once and nothing is staged in registers (a register-staged fill exposed one HBM round trip per 16 loads and
     // took 27-60 % of the kernel).  Three paths, cheapest first: both windows inside their rows (no predicates),
@@ -411,24 +416,14 @@ resample_dec2_kernel(const float *__restrict__ carry, const float *__restrict__ 
         cp_async_commit();
     };
 
-    if (STAGES == 2 && blockIdx.x < n_pairs) fill(blockIdx.x, rs_tile2);
-    int k = 0;
-    for (size_t pair = blockIdx.x; pair < n_pairs; pair += gridDim.x, ++k) {
-        float2 *buf = rs_tile2 + (STAGES == 2 ? (k & 1) * Cfg::TILE_IN : 0);
-        if (STAGES == 2) {
-            // the other stage was consumed one iteration ago (trailing barrier): refill it while this one is filtered
-            const size_t next = pair + gridDim.x;
-            if (next < n_pairs) { fill(next, rs_tile2 + ((k & 1) ^ 1) * Cfg::TILE_IN); cp_async_wait_group<1>(); }
-            else cp_async_wait_group<0>();
-        } else {
-            fill(pair, buf);
-            cp_async_wait_group<0>();
-        }
+    for (size_t pair = blockIdx.x; pair < n_pairs; pair += gridDim.x) {
+        fill(pair, rs_tile2);
+        cp_async_wait_group<0>();
         __syncthreads();
         float2 acc[R];
 #pragma unroll
         for (int r = 0; r < R; ++r) acc[r] = make_float2(0.f, 0.f);
-        const float2 *sx = buf + t * Cfg::STEP;
+        const float2 *sx = rs_tile2 + t * Cfg::STEP;
         RsDec2Steps<M, R, Cfg::TPP, 0, Cfg::WIN2>::run(sx, taps, acc);
         size_t cA, oA, cB, oB;
         tile_src(2 * pair, &cA, &oA);
@@ -445,17 +440,17 @@ resample_dec2_kernel(const float *__restrict__ carry, const float *__restrict__ 
             for (int r = 0; r < R; ++r)
                 if ((size_t)(t * R + r) < leftB) dB[r] = acc[r].y;
         }
-        __syncthreads();                                       // stage consumed before it is refilled
+        __syncthreads();                                       // tile consumed before it is refilled
     }
 }
 
-template <int M, int R, int NT, int STAGES>
+template <int M, int R, int NT>
 static int launch_resample_dec2(lrc_resampler *r, const float *d_in, size_t n_in, size_t in_stride, size_t no, float *d_out,
                                 size_t out_stride, cudaStream_t s)
 {
     using Cfg = RsDec2Cfg<M, R, NT>;
-    constexpr int SMEM = Cfg::SMEM_BYTES * STAGES;
-    auto kern = resample_dec2_kernel<M, R, NT, STAGES>;
+    constexpr int SMEM = Cfg::SMEM_BYTES;
+    auto kern = resample_dec2_kernel<M, R, NT>;
     LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
     int occ = 1;
     LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, SMEM));
@@ -586,21 +581,12 @@ extern "C" int lrc_resampler_process(lrc_resampler *r, const float *d_in, size_t
         static const int variant = getenv("LRC_RS_VARIANT") ? atoi(getenv("LRC_RS_VARIANT")) : 1;
         if (r->L == 1 && variant == 1) {       // packed (FFMA2) two-tile decimators
             switch (r->M) {
-                case 2: rc = launch_resample_dec2<2, 7, 128, 1>(r, d_in, n_in, in_stride, no, d_out, out_stride, s); break;
-                case 3: rc = launch_resample_dec2<3, 6, 128, 1>(r, d_in, n_in, in_stride, no, d_out, out_stride, s); break;
-                case 5: {
-                    // tuning configurations of the BASELINE shape (240 kHz -> 48 kHz), LRC_RS_CFG = threads*10 + stages.
-                    // Measured on 1024 channels x 240 k samples (profiles/r1_s8_rs_configs.txt): 64 threads x 1 stage
-                    // 387 Gsamples/s, 128 x 1: 380, 64 x 2: 359, 128 x 2: 351 (a second stage halves the resident CTAs and
-                    // loses more than the hidden fill gains), scalar one-tile kernel 333.
-                    static const int cfg = getenv("LRC_RS_CFG") ? atoi(getenv("LRC_RS_CFG")) : 641;
-                    if (cfg == 1282)      rc = launch_resample_dec2<5, 6, 128, 2>(r, d_in, n_in, in_stride, no, d_out, out_stride, s);
-                    else if (cfg == 1281) rc = launch_resample_dec2<5, 6, 128, 1>(r, d_in, n_in, in_stride, no, d_out, out_stride, s);
-                    else if (cfg == 642)  rc = launch_resample_dec2<5, 6, 64, 2>(r, d_in, n_in, in_stride, no, d_out, out_stride, s);
-                    else                  rc = launch_resample_dec2<5, 6, 64, 1>(r, d_in, n_in, in_stride, no, d_out, out_stride, s);
-                    break;
-                }
-                case 6: rc = launch_resample_dec2<6, 5, 128, 1>(r, d_in, n_in, in_stride, no, d_out, out_stride, s); break;
+                case 2: rc = launch_resample_dec2<2, 7, 128>(r, d_in, n_in, in_stride, no, d_out, out_stride, s); break;
+                case 3: rc = launch_resample_dec2<3, 6, 128>(r, d_in, n_in, in_stride, no, d_out, out_stride, s); break;
+                // 64 threads at M = 5, the BASELINE shape: 387 Gsamples/s against 380 at 128 and 333 for the scalar
+                // one-tile kernel (profiles/r1_s8_rs_configs.txt)
+                case 5: rc = launch_resample_dec2<5, 6, 64>(r, d_in, n_in, in_stride, no, d_out, out_stride, s); break;
+                case 6: rc = launch_resample_dec2<6, 5, 128>(r, d_in, n_in, in_stride, no, d_out, out_stride, s); break;
                 default: break;                // M = 4: no conflict-free R, the scalar tile kernel below
             }
         }

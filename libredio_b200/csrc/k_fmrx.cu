@@ -19,6 +19,11 @@
 //              of having more work items than CTA slots; a segment is sized so that it stays near 5 %).
 // Every audio sample is the same operation sequence wherever it falls in a tile, segment or call, so the stream is
 // bit-identical however it is chunked; the carried state between calls is just raw input: the last <= 6.7 k samples.
+//
+// Measured and rejected (one B200): the three stand-alone stages for this shape, 752 200 Msamples/s in round 1 against
+// 765 400 for this kernel in round 2 (DESIGN.md, config 3); they stay the path for every other shape.  fmrx_kernel bounded
+// for 2 CTAs per SM (128 registers) instead of 3, timed against it in tools/runs/r2h.sh; the 3-CTA captures of that run are
+// profiles/r2_r2h_fmrx3_ncu_keys.txt and r2_r2h_fmrx3_ncu_phases.txt.
 #include "fir_core.cuh"
 #include "fm_core.cuh"
 #include <cmath>
@@ -91,8 +96,7 @@ struct RoundIter {
 };
 }  // namespace fmrx
 
-template <int MIN_CTAS>
-__global__ void __launch_bounds__(fmrx::NT, MIN_CTAS)
+__global__ void __launch_bounds__(fmrx::NT, 3)
 fmrx_kernel(const __grid_constant__ fmrx::Args a, const __grid_constant__ FirTaps<fmrx::NTAPS> taps127,
             const __grid_constant__ RsTaps<fmrx::TPP> rtaps)
 {
@@ -298,8 +302,7 @@ extern "C" int lrc_fmrx_create(lrc_ctx *ctx, const float *h_taps, int ntaps, int
     f->ctx = ctx; f->n_ch = n_ch; f->max_chunk = max_chunk; f->decim = decim; f->ntaps = ntaps;
     f->d_carry[0] = f->d_carry[1] = nullptr; f->cur = 0; f->carry_stride = 0; f->held = f->n_raw = f->m_next = 0;
     f->fir = nullptr; f->fs = nullptr; f->rs = nullptr; f->d_bb = f->d_fm = f->d_state = nullptr; f->bb_cap = 0;
-    static const int variant = getenv("LRC_FMRX_VARIANT") ? atoi(getenv("LRC_FMRX_VARIANT")) : 1;   // 0: always the composition (A/B)
-    f->fused = variant == 1 && ntaps == fmrx::NTAPS && decim == fmrx::DECIM && fabs(ratio - 0.2) < 1e-15;
+    f->fused = ntaps == fmrx::NTAPS && decim == fmrx::DECIM && fabs(ratio - 0.2) < 1e-15;
     // both forms need the plans: the fused one takes its taps from them (one designer, one rounding)
     int rc = lrc_fir_create(ctx, h_taps, ntaps, decim, &f->fir);           // validates the taps (finite)
     const size_t bb_max = (ntaps + max_chunk) / decim + 2;
@@ -325,8 +328,7 @@ extern "C" int lrc_fmrx_create(lrc_ctx *ctx, const float *h_taps, int ntaps, int
                 return LRC_ERR_CUDA;
             }
         }
-        cudaError_t e = cudaFuncSetAttribute(fmrx_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, fmrx::SMEM_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(fmrx_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, fmrx::SMEM_BYTES);
+        cudaError_t e = cudaFuncSetAttribute(fmrx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fmrx::SMEM_BYTES);
         if (e != cudaSuccess) { lrc_set_error("lrc_fmrx_create: %s", cudaGetErrorString(e)); lrc_fmrx_destroy(f); return LRC_ERR_CUDA; }
     } else {
         rc = lrc_fir_stream_create(f->fir, n_ch, max_chunk, 1, &f->fs);
@@ -412,15 +414,13 @@ extern "C" int lrc_fmrx_push(lrc_fmrx *f, const uint8_t *d_iq, size_t n, size_t 
         a.tiles_per_pair = (no + TILE_A - 1) / TILE_A;
         const long long outs_last = no - (a.tiles_per_pair - 1) * TILE_A;         // outputs of a pair's last tile
         a.last_rounds = (int)((M * (outs_last - 1) + 1 + ROUND_Z - 1) / ROUND_Z);
-        static const int occ = getenv("LRC_FMRX_OCC") ? atoi(getenv("LRC_FMRX_OCC")) : 3;      // CTAs per SM (A/B: 2 = 128 registers)
-        const long long pairs = ((long long)f->n_ch + 1) / 2, slots = (long long)f->ctx->n_sm * (occ == 2 ? 2 : 3);
+        const long long pairs = ((long long)f->n_ch + 1) / 2, slots = (long long)f->ctx->n_sm * 3;    // 3 CTAs per SM
         a.total_tiles = pairs * a.tiles_per_pair;
         // TMA needs 16-byte aligned rows and piece boundaries: held and n multiples of 8 samples, aligned bases / strides
         a.use_tma = (f->held % 8 == 0) && (n % 8 == 0) && (((uintptr_t)d_iq & 15) == 0) && (a.chunk_stride % 16 == 0) &&
                     (a.row_abs0 % 8 == 0);
         long long blocks = slots < a.total_tiles ? slots : a.total_tiles;
-        if (occ == 2) fmrx_kernel<2><<<(unsigned)blocks, NT, SMEM_BYTES, s>>>(a, f->taps127, f->rtaps);
-        else          fmrx_kernel<3><<<(unsigned)blocks, NT, SMEM_BYTES, s>>>(a, f->taps127, f->rtaps);
+        fmrx_kernel<<<(unsigned)blocks, NT, SMEM_BYTES, s>>>(a, f->taps127, f->rtaps);
         LRC_CUDA(cudaGetLastError());
     }
     // carry for the next call: everything from the start of the next segment's priming round, floored to 8 samples

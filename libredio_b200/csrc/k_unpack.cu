@@ -2,19 +2,19 @@
 // (src/rtlsdr/src/rtlsdr.rs:159-162):  i2f(b) = fl(fl(b)/127) - 1.
 //
 // HBM-bound: 2 B in, 8 B out per sample; 6 full-rate instructions per value (unpack.cuh).
+//
+// Measured and rejected (round 1, profiles/r1_s8_grid_sweeps.txt, grid capped at 16 CTAs per SM, Gsamples/s): the
+// streaming st.global.L1::no_allocate store (562.6) and st.global.cs (563.1) against plain stores (571.1), and a register
+// bound for 8 resident CTAs per SM (539.7 / 542.5 / 540.5 for the three store forms) against 4.
 #include "common.cuh"
 #include "unpack.cuh"
-#include <cstdlib>
 
 // One 32-bit word (two samples) per lane per step: the warp reads 128 contiguous bytes and writes 512
 // contiguous bytes with one STG.128 per lane, so both directions are perfectly coalesced; UNROLL steps are
 // issued back to back to keep enough loads in flight.
 constexpr int UNPACK_UNROLL = 8;
 
-// STORE: 0 = st.global.L1::no_allocate (streaming), 1 = plain st.global, 2 = st.global.cs;  MINB: resident CTAs per
-// SM the register allocation is bounded for (tuning knobs, LRC_UNPACK_VARIANT = STORE * 10 + MINB)
-template <int STORE, int MINB>
-__global__ void __launch_bounds__(256, MINB)
+__global__ void __launch_bounds__(256, 4)
 unpack_kernel(const uint8_t *__restrict__ in, float *__restrict__ out, size_t n_bytes)
 {
     const size_t n_words = n_bytes / 4;
@@ -34,9 +34,7 @@ unpack_kernel(const uint8_t *__restrict__ in, float *__restrict__ out, size_t n_
             if (i < n_words) {
                 const float4 v = make_float4(lr_i2f_byte(w[u], 0), lr_i2f_byte(w[u], 1),
                                              lr_i2f_byte(w[u], 2), lr_i2f_byte(w[u], 3));
-                if (STORE == 0) stg_stream_f4(dst + i, v);
-                else if (STORE == 1) dst[i] = v;
-                else __stcs(dst + i, v);
+                dst[i] = v;
             }
         }
     }
@@ -67,21 +65,12 @@ extern "C" int lrc_unpack_u8_cf32(lrc_ctx *ctx, const uint8_t *d_iq, size_t n_by
         if (vec_bytes) {
             size_t blocks = ceil_div(vec_bytes / 4, (size_t)256 * UNPACK_UNROLL);
             // one 8 KB-in / 32 KB-out chunk per CTA and no grid cap: 0.87 -> 1.04 of the copy bandwidth against 16
-            // looping CTAs per SM; plain stores are marginally ahead of the streaming hint (profiles/r1_s8_grid_sweeps.txt).
-            // LRC_UNPACK_VARIANT = store mode * 10 + CTAs/SM of the register bound, LRC_UNPACK_CAP = CTAs per SM cap
-            static const int variant = getenv("LRC_UNPACK_VARIANT") ? atoi(getenv("LRC_UNPACK_VARIANT")) : 14;
+            // looping CTAs per SM (profiles/r1_s8_grid_sweeps.txt).  LRC_UNPACK_CAP = CTAs per SM cap
             static const size_t capf = lrc_grid_mult("LRC_UNPACK_CAP", (size_t)1 << 20);
             const size_t cap = (size_t)ctx->n_sm * capf;
             if (blocks > cap) blocks = cap;
             if (blocks > 0x7fffffffu) blocks = 0x7fffffffu;
-            switch (variant) {
-                case 8:  unpack_kernel<0, 8><<<(unsigned)blocks, 256, 0, s>>>(d_iq, d_out, vec_bytes); break;
-                case 14: unpack_kernel<1, 4><<<(unsigned)blocks, 256, 0, s>>>(d_iq, d_out, vec_bytes); break;
-                case 18: unpack_kernel<1, 8><<<(unsigned)blocks, 256, 0, s>>>(d_iq, d_out, vec_bytes); break;
-                case 24: unpack_kernel<2, 4><<<(unsigned)blocks, 256, 0, s>>>(d_iq, d_out, vec_bytes); break;
-                case 28: unpack_kernel<2, 8><<<(unsigned)blocks, 256, 0, s>>>(d_iq, d_out, vec_bytes); break;
-                default: unpack_kernel<0, 4><<<(unsigned)blocks, 256, 0, s>>>(d_iq, d_out, vec_bytes); break;
-            }
+            unpack_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_iq, d_out, vec_bytes);
             LRC_CUDA(cudaGetLastError());
         }
     }

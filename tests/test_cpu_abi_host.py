@@ -83,6 +83,27 @@ def test_product_package_never_imports_the_oracle():
                     assert "liboracle" not in txt and "restated.h" not in txt, f
 
 
+def test_library_reads_only_the_documented_environment_switches():
+    """Every stage compiles one kernel per shape; an environment variable may size a grid, select the reference a test
+    compares against, or be a test hook, but not pick a second kernel form.  The list is DESIGN.md's "Tuning knobs"."""
+    documented = {
+        # grid multipliers
+        "LRC_UNPACK_CAP", "LRC_FM_CAP", "LRC_FIR_GRID", "LRC_FIRU8_GRID", "LRC_FFT_GRID", "LRC_PSD_GRID", "LRC_RS_GRID",
+        "LRC_CHAIN_GRID",
+        # reference switches that tests compare against
+        "LRC_RS_VARIANT", "LRC_CHAIN_NO_GENERIC", "LRC_CHAIN_GENERIC_ALL", "LRC_FIR_NO_GENTILE",
+        # test hook
+        "LRC_OOK_TEST_GUARD_BLOCKS",
+        # device of the kissfft / libsamplerate ABI shims
+        "LIBREDIO_DEVICE",
+    }
+    csrc = os.path.join(ROOT, "libredio_b200", "csrc")
+    found = set()
+    for f in os.listdir(csrc):
+        found |= set(re.findall(r'"((?:LRC|LIBREDIO)_[A-Z0-9_]+)"', open(os.path.join(csrc, f)).read()))
+    assert found == documented, f"undocumented: {sorted(found - documented)}, no longer read: {sorted(documented - found)}"
+
+
 def test_split_units_covers_everything():
     from libredio_b200 import shard
     for n in (0, 1, 7, 8, 4096, 4099):
