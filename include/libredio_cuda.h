@@ -200,6 +200,7 @@ int    lrc_chain_run_host_u8(lrc_chain *chain, const uint8_t *h_iq, size_t n_in,
  * (libkissfft/tools/kiss_fastfir.c:65-245): true convolution with the nh-1 transient removed,
  *     y[k] = sum_j h[j] * x[k + nh - 1 - j].
  * nfft = 0 -> next power of two >= 2*nh, at least 1024 (:81-93).  Blocks advance by ngood = nfft-nh+1.
+ * nfft fixes the output length; the library chooses the block size it computes in.
  * lrc_fastfir_run processes every full block of the n samples (kff_nocopy :192-206) and, if flush,
  * the zero-padded remainder (kff_flush :208-226); *n_out receives the number of outputs.
  * ---------------------------------------------------------------------------------------------- */

@@ -1,5 +1,5 @@
-// k_fastfir16k.cu -- overlap-save with nfft = 16384 (the default block size for 2048 < nh <= 8192 on request, and the
-// size lrc_fastfir_create picks itself for the config-5 shape when the caller does not insist on kiss_fastfir's).
+// k_fastfir16k.cu -- overlap-save in 16384-point blocks: the compute block lrc_fastfir_create picks for every plan with
+// nh > 1024 or nfft >= 8192, whatever output length the plan's nfft fixes (the config-5 shape among them).
 //
 // Why: with nh = 4096 an 8192-point block keeps 4097 of 8192 outputs (50 %), a 16384-point block keeps 12289 of 16384
 // (75 %): 1.39x fewer butterflies per output sample (kiss_fastfir.c:81-93 picks the block size by a cost model of

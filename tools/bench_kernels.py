@@ -189,21 +189,18 @@ def main():
         x = torch.view_as_complex(torch.randn(n, 2, device=dev, generator=g))
         rng = np.random.default_rng(6)
         h = ((rng.standard_normal(4096) + 1j * rng.standard_normal(4096)) / 64).astype(np.complex64)
-        flop16 = (2 * 5 * 16384 * 14 + 6 * 16384) / 12289.0
-        for nfft, label, flop in ((0, "overlap-save FIR 4096 taps, 16384-point blocks (config 5, K4)", flop16),
-                                  (8192, "overlap-save FIR 4096 taps, explicit nfft 8192 (fastfir8k_kernel)", 272.0)):
-            ff = blocks.FastFir(ctx, h, nfft)
-            out = torch.empty(ff.out_len(n) + 1, dtype=torch.complex64, device=dev)
-            ms, _ = timeit(lambda: ff.run(x, out=out), iters=5)
-            extra = {"flop_per_sample_nominal": flop, "TFLOP/s_nominal": n * flop / (ms * 1e-3) / 1e12}
-            if a.cpu and oracle.have_ref() and nfft == 0:
-                hx = synth.cf32_noise_tones(1 << 20, seed=5)
-                extra.update(cpu_rate(lambda: oracle.ref_fastfir(h, hx), hx.size))
-                extra["cpu_what"] = "vendored tools/kiss_fastfir.c (-O3, tools/Makefile:43), 2^20-sample buffers"
-            report(label, n, n * 16, ms, extra)
-            del out
-            ff.close()
-        del x
+        flop = (2 * 5 * 16384 * 14 + 6 * 16384) / 12289.0
+        ff = blocks.FastFir(ctx, h, 0)
+        out = torch.empty(ff.out_len(n) + 1, dtype=torch.complex64, device=dev)
+        ms, _ = timeit(lambda: ff.run(x, out=out), iters=5)
+        extra = {"flop_per_sample_nominal": flop, "TFLOP/s_nominal": n * flop / (ms * 1e-3) / 1e12}
+        if a.cpu and oracle.have_ref():
+            hx = synth.cf32_noise_tones(1 << 20, seed=5)
+            extra.update(cpu_rate(lambda: oracle.ref_fastfir(h, hx), hx.size))
+            extra["cpu_what"] = "vendored tools/kiss_fastfir.c (-O3, tools/Makefile:43), 2^20-sample buffers"
+        report("overlap-save FIR 4096 taps, 16384-point blocks (config 5, K4)", n, n * 16, ms, extra)
+        del out, x
+        ff.close()
 
     if want("firg"):
         # stand-alone FIR for shapes without a dedicated instance: the padded-chunk tile kernel vs the one-thread-per-output kernel

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """One-process check + timing of the 16384-point overlap-save kernel: windows of the output (incl. block seams and
-the flush block) against an f64 direct convolution, then the throughput of the three plans on the same input:
-nfft = 0 (kiss_fastfir's output length, computed in 16384-point blocks), explicit 16384, explicit 8192 (fastfir8k_kernel)."""
+the flush block) against an f64 direct convolution, then the throughput of the two plans on the same input:
+nfft = 0 (kiss_fastfir's output length, computed in 16384-point blocks) and explicit 16384."""
 import json
 import os
 import sys
@@ -19,7 +19,7 @@ h = ((rng.standard_normal(nh) + 1j * rng.standard_normal(nh)) / 64).astype(np.co
 hr = h[::-1].astype(np.complex128)
 g = torch.Generator(device=ctx.tdev).manual_seed(5)
 res = {}
-for nfft in (0, 16384, 8192):
+for nfft in (0, 16384):
     ff = blocks.FastFir(ctx, h, nfft)
     worst = 0.0
     for n, flush in ((16384, False), (70_001, True), (1 << 22, False)):
