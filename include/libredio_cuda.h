@@ -212,6 +212,31 @@ size_t lrc_fastfir_out_len(const lrc_fastfir *ff, size_t n_in, int flush);
 int    lrc_fastfir_run(lrc_fastfir *ff, const float *d_in, size_t n_in, float *d_out, int flush,
                        size_t *n_out, void *stream);
 
+/* Streaming form of lrc_fastfir_run over n_ch channels (kiss_fastfir(cfg, inbuf, outbuf, n_new, &offset), :228-245):
+ * every channel carries its own history on the device, and all channels of a push go through one launch.
+ * Outputs come in whole compute blocks: a push emits every output whose compute block is complete.  Blocks sit at
+ * multiples of the compute block's ngood from the start of the stream, and the compute block is nfft points
+ * (ngood = nfft - nh + 1) for plans with nh <= 1024 and nfft < 8192, 16384 points (ngood = 16385 - nh) otherwise.  So for
+ * the first kind the per-push counts are kiss_fastfir's; for the second they come in units of 16385 - nh, while the
+ * values and the flushed total are the same.  For every channel and every way of cutting the input into pushes, the
+ * outputs concatenated, with flush on the last push, equal lrc_fastfir_run(whole input, flush = 1) bit for bit; after a
+ * push without flush they are a bitwise prefix of it.  The carried history is always shorter than one compute block. */
+typedef struct lrc_fastfir_stream lrc_fastfir_stream;
+/* n_ch channels through the plan `ff` (borrowed: it must outlive the stream), each from the initial state (no history) */
+int    lrc_fastfir_stream_create(lrc_fastfir *ff, size_t n_ch, lrc_fastfir_stream **st);
+int    lrc_fastfir_stream_destroy(lrc_fastfir_stream *st);
+int    lrc_fastfir_stream_reset(lrc_fastfir_stream *st);
+/* outputs per channel that the next push of n samples (and flush) will write; host arithmetic */
+size_t lrc_fastfir_stream_next_out_len(const lrc_fastfir_stream *st, size_t n, int flush);
+/* n new samples per channel (n may be 0), channel c at d_chunk + c*chunk_stride (samples, >= n), cf32, 8-byte aligned;
+ * outputs to d_out + c*out_stride (out_stride >= next_out_len, else LRC_ERR_CAPACITY; d_out must not overlap the
+ * chunk); *n_out = outputs per channel (host arithmetic, no readback).  flush: after the chunk, also emit the
+ * zero-padded remainder as kff_flush does (kiss_fastfir with n_new == 0, :228-245); the stream is then back at its
+ * initial state, and a flush with fewer than nh samples held emits nothing more.  Asynchronous on `stream`; the pushes
+ * of one stream must be ordered on the device (one CUDA stream, or synchronised between pushes). */
+int    lrc_fastfir_stream_push(lrc_fastfir_stream *st, const float *d_chunk, size_t n, size_t chunk_stride,
+                               float *d_out, size_t out_stride, int flush, size_t *n_out, void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * (4a) quadrature FM discriminator (north-star stage, absent from the reference):
  *     d[n] = atan2(Im z, Re z), z = x[n] * conj(x[n-1]); x[-1] comes from d_state (one cf32 per

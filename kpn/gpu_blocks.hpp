@@ -9,6 +9,7 @@
 //   kissfft::fft              kissfft.rs:18-31    kpn_gpu::fft
 //   samplerate::resample      samplerate.rs:59    kpn_gpu::resample
 //   dsputils::convolve (+/D)  dsputils.rs:30      kpn_gpu::fir_decimate, fir_decimate_multi (channel ring)
+//   kiss_fastfir (streaming)  kiss_fastfir.c:228  kpn_gpu::fast_fir_multi (channel ring, long FIR by overlap-save)
 //   (north-star) discriminator                    kpn_gpu::fm_demod
 //   (north-star) FIR->FFT->|X|^2 chain            kpn_gpu::chain_psd
 //   (north-star) config-3 FM receiver, N channels  kpn_gpu::fm_receiver_multi (lrc_fmrx: one kernel per batch)
@@ -211,6 +212,62 @@ inline void fir_decimate_multi(Gpu &g, std::vector<Receiver<std::vector<cf32>>> 
     } catch (...) {
         try { drain(ring[0]); drain(ring[1]); } catch (...) {}
         lrc_fir_stream_destroy(fs); lrc_fir_destroy(fir);
+        for (auto &r : ring) { r.in.release(g); r.out.release(g); if (r.done) cudaEventDestroy(r.done); }
+        throw;
+    }
+}
+
+// ---- long FIR by overlap-save over MANY channels: kiss_fastfir with a carried offset ----------------------
+// The channel ring of fir_decimate_multi over lrc_fastfir_stream: one chunk (chunk_len samples) from every channel's port
+// per batch, one push per batch.  Outputs come as whole compute blocks complete (a batch that completes none sends
+// nothing); concatenated per channel they are a prefix of lrc_fastfir_run over the channel's whole input.  The block never
+// flushes: the reference's ports never end (a closed port tears the graph down).
+inline void fast_fir_multi(Gpu &g, std::vector<Receiver<std::vector<cf32>>> u, std::vector<Sender<std::vector<cf32>>> v,
+                           std::vector<cf32> h, size_t nfft, size_t chunk_len)
+{
+    g.bind();
+    const size_t n_ch = u.size();
+    if (v.size() != n_ch || n_ch == 0) throw std::invalid_argument("fast_fir_multi: port count mismatch");
+    lrc_fastfir *ff = nullptr; lrc_fastfir_stream *fs = nullptr;
+    check(lrc_fastfir_create(g.ctx, (const float *)h.data(), h.size(), nfft, &ff), "lrc_fastfir_create");
+    check(lrc_fastfir_stream_create(ff, n_ch, &fs), "lrc_fastfir_stream_create");
+    Stream st;
+    const size_t cap = chunk_len + 16384;                  // the history is shorter than one compute block (<= 16384)
+    struct RingSlot { Slot in, out; cudaEvent_t done = nullptr; size_t n_out = 0; bool busy = false; } ring[2];
+    for (auto &r : ring) {
+        r.in.reserve(g, n_ch * chunk_len * sizeof(cf32)); r.out.reserve(g, n_ch * cap * sizeof(cf32));
+        cuda_check(cudaEventCreateWithFlags(&r.done, cudaEventDisableTiming), "cudaEventCreate");
+    }
+    auto drain = [&](RingSlot &r) {
+        if (!r.busy) return;
+        cuda_check(cudaEventSynchronize(r.done), "cudaEventSynchronize");
+        const cf32 *p = (const cf32 *)r.out.h;
+        if (r.n_out)
+            for (size_t c = 0; c < n_ch; ++c) v[c].send(std::vector<cf32>(p + c * cap, p + c * cap + r.n_out));
+        r.busy = false;
+    };
+    try {
+        for (size_t it = 0;; ++it) {
+            RingSlot &r = ring[it & 1];
+            drain(r);                                          // slot reuse: its previous batch must be out
+            for (size_t c = 0; c < n_ch; ++c) {
+                std::vector<cf32> x = u[c].recv();
+                if (x.size() != chunk_len) throw std::length_error("fast_fir_multi: chunk length != chunk_len");
+                std::memcpy((cf32 *)r.in.h + c * chunk_len, x.data(), chunk_len * sizeof(cf32));
+            }
+            cuda_check(cudaMemcpyAsync(r.in.d, r.in.h, n_ch * chunk_len * sizeof(cf32), cudaMemcpyHostToDevice, st.s), "H2D");
+            check(lrc_fastfir_stream_push(fs, (const float *)r.in.d, chunk_len, chunk_len, (float *)r.out.d, cap, 0, &r.n_out,
+                                          st.s), "lrc_fastfir_stream_push");
+            if (r.n_out)
+                cuda_check(cudaMemcpy2DAsync(r.out.h, cap * sizeof(cf32), r.out.d, cap * sizeof(cf32), r.n_out * sizeof(cf32),
+                                             n_ch, cudaMemcpyDeviceToHost, st.s), "D2H");
+            cuda_check(cudaEventRecord(r.done, st.s), "cudaEventRecord");
+            r.busy = true;
+            drain(ring[(it + 1) & 1]);                         // hand out the batch submitted one step ago
+        }
+    } catch (...) {
+        try { drain(ring[0]); drain(ring[1]); } catch (...) {}
+        lrc_fastfir_stream_destroy(fs); lrc_fastfir_destroy(ff);
         for (auto &r : ring) { r.in.release(g); r.out.release(g); if (r.done) cudaEventDestroy(r.done); }
         throw;
     }

@@ -452,6 +452,41 @@ class FastFir:
             self.h = C.c_void_p()
 
 
+class FastFirStream:
+    """kiss_fastfir with a carried offset (tools/kiss_fastfir.c:228-245) over n_ch channels: each channel keeps its own
+    history on the device and every push is one launch for all channels.  The outputs of the pushes, concatenated, with
+    flush on the last one, equal FastFir.run(whole input, flush=True) bit for bit, whatever the push sizes."""
+
+    def __init__(self, ff: FastFir, n_ch: int):
+        self.ff, self.n_ch = ff, int(n_ch)
+        self.h = C.c_void_p()
+        check(ff.ctx.lib.lrc_fastfir_stream_create(ff.h, self.n_ch, C.byref(self.h)), "lrc_fastfir_stream_create")
+
+    def next_out_len(self, n: int, flush: bool = False) -> int:
+        return int(self.ff.ctx.lib.lrc_fastfir_stream_next_out_len(self.h, n, int(flush)))
+
+    def reset(self):
+        check(self.ff.ctx.lib.lrc_fastfir_stream_reset(self.h), "lrc_fastfir_stream_reset")
+
+    def push(self, x: torch.Tensor, flush: bool = False) -> torch.Tensor:
+        """x: complex64 [n_ch, n] (or [n] when n_ch == 1) -> [n_ch, n_out]"""
+        assert x.dtype == torch.complex64 and x.is_cuda and x.is_contiguous()
+        x2 = x.reshape(self.n_ch, -1)
+        n = x2.shape[1]
+        want = self.next_out_len(n, flush)
+        out = torch.empty((self.n_ch, max(want, 1)), dtype=torch.complex64, device=x.device)
+        no = C.c_size_t()
+        check(self.ff.ctx.lib.lrc_fastfir_stream_push(self.h, _p(x2), n, n, _p(out), out.shape[1], int(flush), C.byref(no),
+                                                      _stream()), "lrc_fastfir_stream_push")
+        assert no.value == want
+        return out[:, :want]
+
+    def close(self):
+        if self.h:
+            self.ff.ctx.lib.lrc_fastfir_stream_destroy(self.h)
+            self.h = C.c_void_p()
+
+
 # ---- (5) OOK ------------------------------------------------------------------------------------------
 class Ook:
     """The OOK chain of ratpak.rs:60-111 over n_streams finite u8-IQ captures of n_blocks*512 samples."""

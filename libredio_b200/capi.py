@@ -91,6 +91,11 @@ SIGNATURES = {
     "lrc_fastfir_nfft": (_sz, [_vp]),
     "lrc_fastfir_out_len": (_sz, [_vp, _sz, _i]),
     "lrc_fastfir_run": (_i, [_vp, _fp, _sz, _fp, _i, _szp, _vp]),
+    "lrc_fastfir_stream_create": (_i, [_vp, _sz, _pp]),
+    "lrc_fastfir_stream_destroy": (_i, [_vp]),
+    "lrc_fastfir_stream_reset": (_i, [_vp]),
+    "lrc_fastfir_stream_next_out_len": (_sz, [_vp, _sz, _i]),
+    "lrc_fastfir_stream_push": (_i, [_vp, _fp, _sz, _sz, _fp, _sz, _i, _szp, _vp]),
     "lrc_fmdemod_run": (_i, [_vp, _fp, _sz, _sz, _sz, _fp, _fp, _sz, _vp]),
     "lrc_resampler_create": (_i, [_vp, C.c_double, _sz, _sz, _pp]),
     "lrc_resampler_destroy": (_i, [_vp]),

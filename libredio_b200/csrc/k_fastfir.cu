@@ -17,6 +17,14 @@
 //     for the 16384-point kernel in the same process (profiles/r1_s8_fastfir16k_check.json), 99.9 against 121.3 in
 //     round 2 (profiles/r2_a_ff16k_v1_check.json); the 16384-point kernel has since reached 145.3.  SASS and ncu keys
 //     in profiles/sass/r1_fastfir8k.sass and profiles/r1_s3_fastfir8k_v4_ncu_keys.txt.
+//
+// Streaming (lrc_fastfir_stream_*): every channel carries the samples of its row that no complete compute block has
+// consumed yet (fewer than one compute block) in a device carry buffer; a push runs the STREAM instance of the plan's
+// kernel over every (channel, block) whose window is complete, reading [carry | chunk] in place (fastfir.cuh), then
+// copies the new tail into the other carry buffer of a ping-pong pair.  Blocks sit at multiples of ngood from the start
+// of the stream and see the same window and zero padding as in one lrc_fastfir_run over the whole stream, so the outputs
+// are bitwise those of that call whatever the push sizes.
+#include "fastfir.cuh"
 #include "fft_core.cuh"
 #include <cmath>
 #include <utility>
@@ -26,11 +34,6 @@ using namespace lrfft;
 
 int lrc_make_twiddles(int nfft, float2 **d_tw);
 int lrc_log2_exact(int n);
-// k_fastfir16k.cu (16384-point blocks)
-void lrc_fastfir16k_permute_H(const float2 *H, float2 *Hq);
-int lrc_fastfir16k_prepare(void);
-int lrc_fastfir16k_launch(int n_sm, const float2 *in, size_t n_in, float2 *out, size_t full, size_t nblk, size_t ngood,
-                          size_t keep, const float2 *d_tw16k, const float2 *d_tw1k, const float2 *d_Hp, cudaStream_t s);
 
 struct lrc_fastfir {
     lrc_ctx *ctx;
@@ -65,25 +68,53 @@ static void host_fft_f64(std::vector<double> &re, std::vector<double> &im)
     }
 }
 
-template <int LOG2N>
+// STREAM: n_blocks counts (channel, block) items of a stream push, n_blocks_full the full blocks per channel (fastfir.cuh)
+template <int LOG2N, bool STREAM>
 __global__ void __launch_bounds__(CtaFFT<LOG2N, false>::T)
 fastfir_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict__ out, size_t n_blocks_full,
                size_t n_blocks, size_t ngood, size_t flush_keep, const float2 *__restrict__ tw,
-               const float2 *__restrict__ H)
+               const float2 *__restrict__ H, FfStreamArgs sa)
 {
     using FF = CtaFFT<LOG2N, false>;
     using FI = CtaFFT<LOG2N, true>;
     constexpr int N = FF::N, E = FF::E, T = FF::T;
     extern __shared__ float2 sm[];
     const int t = threadIdx.x;
-    for (size_t b = blockIdx.x; b < n_blocks; b += gridDim.x) {
+    for (size_t w = blockIdx.x; w < n_blocks; w += gridDim.x) {
+        size_t b = w;
+        const float2 *src = in;
+        float2 *dst = out;
+        if constexpr (STREAM) {
+            const size_t c = (unsigned)w / (unsigned)sa.nblk;
+            b = w - c * sa.nblk;
+            src = in + c * sa.in_stride;
+            dst = out + c * sa.out_stride;
+        }
         const size_t s0 = b * ngood;
         const size_t avail = n_in - s0;              // < N only for the flush block
         float2 v[E];
+        if constexpr (STREAM) {
+            if (s0 >= sa.held) {                     // the block lies in the chunk (CTA-uniform)
+                src += s0 - sa.held;
 #pragma unroll
-        for (int e = 0; e < E; ++e) {
-            const size_t i = (size_t)t + (size_t)e * T;
-            v[e] = (i < avail) ? __ldcs(in + s0 + i) : make_float2(0.f, 0.f);
+                for (int e = 0; e < E; ++e) {
+                    const size_t i = (size_t)t + (size_t)e * T;
+                    v[e] = (i < avail) ? __ldcs(src + i) : make_float2(0.f, 0.f);
+                }
+            } else {                                 // straddles the carried history
+                const float2 *crow = sa.carry + ((unsigned)w / (unsigned)sa.nblk) * sa.carry_pitch;
+#pragma unroll
+                for (int e = 0; e < E; ++e) {
+                    const size_t i = s0 + (size_t)t + (size_t)e * T;
+                    v[e] = i < sa.held ? __ldg(crow + i) : i < n_in ? __ldcs(src + (i - sa.held)) : make_float2(0.f, 0.f);
+                }
+            }
+        } else {
+#pragma unroll
+            for (int e = 0; e < E; ++e) {
+                const size_t i = (size_t)t + (size_t)e * T;
+                v[e] = (i < avail) ? __ldcs(in + s0 + i) : make_float2(0.f, 0.f);
+            }
         }
         FF::run(v, sm, tw, t, SyncCta{});
 #pragma unroll
@@ -96,7 +127,7 @@ fastfir_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict__ 
 #pragma unroll
         for (int e = 0; e < E; ++e) {
             const size_t i = (size_t)t + (size_t)e * T;
-            if (i < keep) __stcs(out + s0 + i, v[e]);
+            if (i < keep) __stcs(dst + s0 + i, v[e]);
         }
     }
 }
@@ -183,21 +214,21 @@ extern "C" size_t lrc_fastfir_out_len(const lrc_fastfir *f, size_t n_in, int flu
     return full * f->ngood + keep;
 }
 
-template <int LOG2N>
+template <int LOG2N, bool STREAM>
 static int launch_fastfir(lrc_fastfir *f, const float2 *in, size_t n_in, float2 *out, size_t full, size_t nblk,
-                          size_t keep, cudaStream_t s)
+                          size_t keep, const FfStreamArgs &sa, cudaStream_t s)
 {
     using FF = CtaFFT<LOG2N, false>;
     const int threads = FF::T;
     const size_t smem = (size_t)FF::SMEM_CPX * sizeof(float2);
-    auto kern = fastfir_kernel<LOG2N>;
+    auto kern = fastfir_kernel<LOG2N, STREAM>;
     if (smem > 48 * 1024) LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 1;
     LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
     if (occ < 1) occ = 1;
     size_t blocks = (size_t)f->ctx->n_sm * occ;
     if (blocks > nblk) blocks = nblk;
-    kern<<<(unsigned)blocks, threads, smem, s>>>(in, n_in, out, full, nblk, f->ngood, keep, f->d_tw, f->d_H);
+    kern<<<(unsigned)blocks, threads, smem, s>>>(in, n_in, out, full, nblk, f->ngood, keep, f->d_tw, f->d_H, sa);
     LRC_CUDA(cudaGetLastError());
     return LRC_OK;
 }
@@ -223,13 +254,160 @@ extern "C" int lrc_fastfir_run(lrc_fastfir *f, const float *d_in, size_t n_in, f
         const size_t n_total = full * f->ngood + keep, ngood16 = 16384 - f->nh + 1;
         const size_t full16 = n_total / ngood16, keep16 = n_total % ngood16;
         return lrc_fastfir16k_launch(f->ctx->n_sm, in, n_in, out, full16, full16 + (keep16 ? 1 : 0), ngood16, keep16, f->d_tw,
-                                     f->d_tw1k, f->d_H, s);
+                                     f->d_tw1k, f->d_H, nullptr, s);
     }
     switch (f->log2n) {
-#define FF_CASE(L) case L: return launch_fastfir<L>(f, in, n_in, out, full, nblk, keep, s);
+#define FF_CASE(L) case L: return launch_fastfir<L, false>(f, in, n_in, out, full, nblk, keep, FfStreamArgs{}, s);
         FF_CASE(1) FF_CASE(2) FF_CASE(3) FF_CASE(4) FF_CASE(5) FF_CASE(6) FF_CASE(7)
         FF_CASE(8) FF_CASE(9) FF_CASE(10) FF_CASE(11) FF_CASE(12)
 #undef FF_CASE
     }
     return LRC_ERR_UNSUPPORTED;
+}
+
+// ---- streaming ---------------------------------------------------------------------------------
+struct lrc_fastfir_stream {
+    lrc_fastfir *ff;
+    size_t       n_ch;
+    size_t       nc, ngood;     // the compute block (nfft, or 16384) and its advance nc - nh + 1
+    size_t       held;          // samples every channel carries, < nc
+    float2      *d_carry[2];    // [n_ch][nc] each, ping-pong; d_carry[cur] holds the history
+    int          cur;
+};
+
+extern "C" int lrc_fastfir_stream_create(lrc_fastfir *f, size_t n_ch, lrc_fastfir_stream **out)
+{
+    LRC_REQUIRE(f && out && n_ch >= 1, LRC_ERR_INVALID, "lrc_fastfir_stream_create: bad arguments");
+    LRC_BIND(f->ctx);
+    lrc_fastfir_stream *st = new (std::nothrow) lrc_fastfir_stream();
+    LRC_REQUIRE(st != nullptr, LRC_ERR_NOMEM, "out of host memory");
+    st->ff = f; st->n_ch = n_ch;
+    st->nc = f->compute16k ? 16384 : f->nfft;
+    st->ngood = st->nc - f->nh + 1;
+    st->held = 0; st->cur = 0;
+    st->d_carry[0] = st->d_carry[1] = nullptr;
+    for (auto &p : st->d_carry) {
+        const cudaError_t e = cudaMalloc(&p, n_ch * st->nc * sizeof(float2));
+        if (e != cudaSuccess) {
+            lrc_set_error("lrc_fastfir_stream_create: %s", cudaGetErrorString(e));
+            lrc_fastfir_stream_destroy(st);
+            return LRC_ERR_CUDA;
+        }
+    }
+    *out = st;
+    return LRC_OK;
+}
+
+extern "C" int lrc_fastfir_stream_destroy(lrc_fastfir_stream *st)
+{
+    if (!st) return LRC_OK;
+    cudaSetDevice(st->ff->ctx->device);
+    cudaFree(st->d_carry[0]); cudaFree(st->d_carry[1]);
+    delete st;
+    return LRC_OK;
+}
+
+extern "C" int lrc_fastfir_stream_reset(lrc_fastfir_stream *st)
+{
+    LRC_REQUIRE(st != nullptr, LRC_ERR_INVALID, "null stream");
+    st->held = 0; st->cur = 0;
+    return LRC_OK;
+}
+
+// complete compute blocks of a row of held + n samples and, with flush, the outputs of the zero-padded remainder
+static void stream_counts(const lrc_fastfir_stream *st, size_t n, int flush, size_t *full, size_t *flush_keep)
+{
+    const size_t total = st->held + n;
+    *full = total >= st->nc ? (total - st->nc) / st->ngood + 1 : 0;
+    const size_t rem = total - *full * st->ngood;
+    *flush_keep = (flush && rem + 1 > st->ff->nh) ? rem + 1 - st->ff->nh : 0;
+}
+
+extern "C" size_t lrc_fastfir_stream_next_out_len(const lrc_fastfir_stream *st, size_t n, int flush)
+{
+    if (!st) return 0;
+    size_t full, keep;
+    stream_counts(st, n, flush, &full, &keep);
+    return full * st->ngood + keep;
+}
+
+// `rows` rows of `width` bytes; one row needs no pitch (a one-channel stream may have any chunk_stride)
+static cudaError_t copy_rows(void *dst, size_t dpitch, const void *src, size_t spitch, size_t width, size_t rows,
+                             cudaStream_t s)
+{
+    if (rows == 1) return cudaMemcpyAsync(dst, src, width, cudaMemcpyDeviceToDevice, s);
+    return cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, cudaMemcpyDeviceToDevice, s);
+}
+
+extern "C" int lrc_fastfir_stream_push(lrc_fastfir_stream *st, const float *d_chunk, size_t n, size_t chunk_stride,
+                                       float *d_out, size_t out_stride, int flush, size_t *n_out, void *stream)
+{
+    LRC_REQUIRE(st && n_out, LRC_ERR_INVALID, "lrc_fastfir_stream_push: null argument");
+    lrc_fastfir *f = st->ff;
+    LRC_BIND(f->ctx);
+    *n_out = 0;
+    const size_t n_ch = st->n_ch, es = sizeof(float2);
+    size_t full, keep;
+    stream_counts(st, n, flush, &full, &keep);
+    const size_t no = full * st->ngood + keep, nblk = full + (keep ? 1 : 0);
+    if (n > 0) {
+        LRC_REQUIRE(d_chunk != nullptr && chunk_stride >= n, LRC_ERR_INVALID, "lrc_fastfir_stream_push: bad chunk");
+        LRC_REQUIRE(((uintptr_t)d_chunk & 7) == 0, LRC_ERR_INVALID, "lrc_fastfir_stream_push: misaligned chunk");
+    }
+    if (no > 0) {
+        LRC_REQUIRE(d_out != nullptr && ((uintptr_t)d_out & 7) == 0, LRC_ERR_INVALID,
+                    "lrc_fastfir_stream_push: null or misaligned output");
+        LRC_REQUIRE(out_stride >= no, LRC_ERR_CAPACITY, "lrc_fastfir_stream_push: out_stride shorter than the outputs");
+        if (n > 0) {
+            const uintptr_t c0 = (uintptr_t)d_chunk, c1 = c0 + ((n_ch - 1) * chunk_stride + n) * es;
+            const uintptr_t o0 = (uintptr_t)d_out, o1 = o0 + ((n_ch - 1) * out_stride + no) * es;
+            LRC_REQUIRE(o1 <= c0 || c1 <= o0, LRC_ERR_INVALID, "lrc_fastfir_stream_push: output overlaps the chunk");
+        }
+        LRC_REQUIRE(n_ch * nblk <= 0xffffffffull, LRC_ERR_UNSUPPORTED, "lrc_fastfir_stream_push: more than 2^32 blocks");
+    }
+    cudaStream_t s = lrc_stream(f->ctx, stream);
+    const float2 *chunk = (const float2 *)d_chunk;
+    float2 *carry = st->d_carry[st->cur];
+    if (nblk > 0) {
+        const FfStreamArgs sa{carry, st->nc, st->held, chunk_stride, out_stride, nblk, 0, 0};
+        const size_t total = st->held + n;
+        float2 *out = (float2 *)d_out;
+        int rc = LRC_ERR_UNSUPPORTED;
+        if (f->compute16k) {
+            rc = lrc_fastfir16k_launch(f->ctx->n_sm, chunk, total, out, full, n_ch * nblk, st->ngood, keep, f->d_tw,
+                                       f->d_tw1k, f->d_H, &sa, s);
+        } else {
+            switch (f->log2n) {
+#define FF_CASE(L) case L: rc = launch_fastfir<L, true>(f, chunk, total, out, full, n_ch * nblk, keep, sa, s); break;
+                FF_CASE(1) FF_CASE(2) FF_CASE(3) FF_CASE(4) FF_CASE(5) FF_CASE(6) FF_CASE(7)
+                FF_CASE(8) FF_CASE(9) FF_CASE(10) FF_CASE(11) FF_CASE(12)
+#undef FF_CASE
+            }
+        }
+        if (rc) return rc;
+    }
+    if (flush) {
+        st->held = 0;                                    // back at the initial state
+    } else if (full == 0) {
+        // no block completed: the chunk goes behind the history
+        if (n > 0)
+            LRC_CUDA(copy_rows(carry + st->held, st->nc * es, chunk, chunk_stride * es, n * es, n_ch, s));
+        st->held += n;
+    } else {
+        // the new history is row[consumed .. held + n), into the other buffer of the pair
+        const size_t consumed = full * st->ngood;
+        float2 *next = st->d_carry[st->cur ^ 1];
+        size_t at = 0;
+        if (consumed < st->held) {
+            at = st->held - consumed;
+            LRC_CUDA(copy_rows(next, st->nc * es, carry + consumed, st->nc * es, at * es, n_ch, s));
+        }
+        const size_t skip = consumed > st->held ? consumed - st->held : 0;
+        if (n > skip)
+            LRC_CUDA(copy_rows(next + at, st->nc * es, chunk + skip, chunk_stride * es, (n - skip) * es, n_ch, s));
+        st->held = st->held + n - consumed;
+        st->cur ^= 1;
+    }
+    *n_out = no;
+    return LRC_OK;
 }

@@ -29,6 +29,13 @@
 //     bins are one coalesced LDG.128.
 // Shared memory: 16 rows x 1088 complex (136 KB) + 512 x 18 P1 twiddles (72 KB) + 32 x 34 warp-transform twiddles
 // (8.5 KB) = 216.5 KB, one 512-thread CTA per SM.
+//
+// STREAM = true (lrc_fastfir_stream_push): a work item is (channel, block) of many channels (fastfir.cuh), the fused
+// P1' / next P1 and the L2 prefetch run across channel boundaries as they do across blocks.  Blocks that start past
+// the carried history read the chunk alone (CTA-uniform branch); only the first blocks of a channel's push start inside
+// it, and those are loaded at the head of their own iteration rather than fused (no registers for a second source).
+// STREAM = false compiles to the instructions of the batch kernel before the stream form existed.
+#include "fastfir.cuh"
 #include "fft_core.cuh"
 
 using namespace lrfft;
@@ -109,10 +116,11 @@ __device__ __forceinline__ void warp_fft1024(float2 *v, float2 *row, const float
 //     r2_r2c_ff16k_512_ncu_phases.txt.
 // A TMA tensor copy would take the loads off the LSU, but block starts (multiples of ngood = 12289 samples) are only
 // 8-byte aligned every other block.
+template <bool STREAM>
 __global__ void __launch_bounds__(ff16k::NT, 1)
 fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict__ out, size_t n_blocks_full,
                   size_t n_blocks, size_t ngood, size_t flush_keep, const float2 *__restrict__ tw /* W_16384^k */,
-                  const float2 *__restrict__ tw1k /* W_1024^k */, const float4 *__restrict__ Hq)
+                  const float2 *__restrict__ tw1k /* W_1024^k */, const float4 *__restrict__ Hq, FfStreamArgs sa)
 {
     using namespace ff16k;
     extern __shared__ __align__(16) float2 ff16k_smem[];
@@ -153,6 +161,30 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
                 va[r] = ca + 1024 * r < avail ? ldg_nc_f2(src + 1024 * r) : make_float2(0.f, 0.f);
                 vb[r] = ca + 32 + 1024 * r < avail ? ldg_nc_f2(src + 1024 * r + 32) : make_float2(0.f, 0.f);
             }
+        }
+    };
+    // STREAM: the 16 inputs of column `col` of block bc of channel c (bounds as lim = bound - col against 1024 r literals,
+    // so that no column index is held across the loop)
+    auto s_load = [&](size_t c, size_t bc, int col, float2 *u) {
+        const size_t s0 = bc * ngood;
+        const float2 *row = in + c * sa.in_stride;
+        const bool whole = n_in - s0 >= (size_t)N;
+        const int lim = (whole ? N : (int)(n_in - s0)) - col;
+        if (s0 >= sa.held) {                                    // the block lies in the chunk (CTA-uniform)
+            const float2 *src = row + (s0 - sa.held) + col;
+#pragma unroll
+            for (int r = 0; r < 16; ++r)
+                u[r] = (whole || 1024 * r < lim) ? ldg_nc_f2(src + 1024 * r) : make_float2(0.f, 0.f);
+        } else {                                                // straddles the carried history (held < N)
+            const int hlim = (int)(sa.held - s0) - col;
+            const float2 *csrc = sa.carry + c * sa.carry_pitch + s0 + col;
+            // row + (1024 r - hlim): integer arithmetic, the address is only formed for 1024 r >= hlim
+            const uintptr_t xsrc = reinterpret_cast<uintptr_t>(row) - (intptr_t)hlim * (intptr_t)sizeof(float2);
+#pragma unroll
+            for (int r = 0; r < 16; ++r)
+                u[r] = 1024 * r < lim ? ldg_nc_f2(1024 * r < hlim ? csrc + 1024 * r
+                                                                  : reinterpret_cast<const float2 *>(xsrc) + 1024 * r)
+                                      : make_float2(0.f, 0.f);          // hlim <= lim
         }
     };
     // forward butterflies of the column pair; results into the pair's 16 shared cells
@@ -201,16 +233,44 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
     };
 
     size_t b = blockIdx.x;
-    if (b < n_blocks) {
+    // STREAM: item b is block bc of channel c, tracked without a division per item (CTA-uniform integer arithmetic)
+    // A straddling block is loaded at the head of its own iteration instead of in the fused phase, where the 128
+    // registers have no room for the second source.
+    size_t c = 0, bc = b;
+    bool loaded = false;                                        // STREAM: item b's P1 forward is done
+    if constexpr (STREAM) {
+        while (bc >= sa.nblk) { bc -= sa.nblk; ++c; }
+    } else if (b < n_blocks) {
         float2 va[16], vb[16];
         p1_load(b, lane + 64 * warp, va, vb);
         p1_forward(va, vb);
     }
     for (; b < n_blocks; b += gridDim.x) {
+        if constexpr (STREAM) {
+            if (!loaded) {
+                float2 va[16], vb[16];
+                s_load(c, bc, lane + 64 * warp, va);
+                s_load(c, bc, lane + 64 * warp + 32, vb);
+                p1_forward(va, vb);
+            }
+        }
         const size_t nb = b + gridDim.x;
         const bool more = nb < n_blocks;
+        size_t nc = c + sa.step_c, nbc = bc + sa.step_b;           // STREAM: item nb
+        if (nbc >= sa.nblk) { nbc -= sa.nblk; ++nc; }
         // the next block's input (1024 lines) is asked into L2 now; its P1 loads come later
-        if (more) {
+        if constexpr (STREAM) {
+            if (more) {                                          // the chunk part of the next item
+                const size_t s0 = nbc * ngood, from = s0 > sa.held ? s0 : sa.held;
+                const char *nsrc = reinterpret_cast<const char *>(in + nc * sa.in_stride + (from - sa.held));
+                const size_t lim = (n_in - from) * 8;
+#pragma unroll
+                for (int k = 0; k < 1024 / NT; ++k) {
+                    const size_t off = (size_t)(t + NT * k) * 128;
+                    if (off < lim) asm volatile("prefetch.global.L2 [%0];" :: "l"(nsrc + off));
+                }
+            }
+        } else if (more) {
             const char *nsrc = reinterpret_cast<const char *>(in + nb * ngood);
 #pragma unroll
             for (int k = 0; k < 1024 / NT; ++k) {
@@ -246,16 +306,32 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
         }
         __syncthreads();
         // ---- P1 inverse of this block fused with P1 forward of the CTA's next block -----------------------
-        const int keep = (int)((b < n_blocks_full) ? ngood : flush_keep);
-        float2 *dstg = out + b * ngood;
         // 128 registers: ua, ub, nxa, nxb are 32 each, so a column of the next block is requested only once a
         // column of this block has left
         const int ca = lane + 64 * warp;
-        const float2 *src = in + nb * ngood + ca;
-        // (one predicated form for whole and ragged blocks: splitting it into a CTA-uniform fast path with
-        // unpredicated loads measured 5 % SLOWER, 133 vs 140 Gsamples/s -- the phase waits on memory, not on issue)
-        const bool whole = more && n_in - nb * ngood >= (size_t)N;
-        const int avail = more ? (whole ? N : (int)(n_in - nb * ngood)) : 0;
+        int keep;
+        float2 *dstg;
+        bool fuse = more;
+        const float2 *src;
+        bool whole;
+        int avail;
+        if constexpr (STREAM) {
+            keep = (int)((bc < n_blocks_full) ? ngood : flush_keep);
+            dstg = out + c * sa.out_stride + bc * ngood;
+            const size_t s0 = nbc * ngood;
+            fuse = more && s0 >= sa.held;                        // the next item lies in the chunk
+            src = fuse ? in + nc * sa.in_stride + (s0 - sa.held) + ca : in;
+            whole = fuse && n_in - s0 >= (size_t)N;
+            avail = fuse ? (whole ? N : (int)(n_in - s0)) : 0;
+        } else {
+            keep = (int)((b < n_blocks_full) ? ngood : flush_keep);
+            dstg = out + b * ngood;
+            src = in + nb * ngood + ca;
+            // (one predicated form for whole and ragged blocks: splitting it into a CTA-uniform fast path with
+            // unpredicated loads measured 5 % SLOWER, 133 vs 140 Gsamples/s -- the phase waits on memory, not on issue)
+            whole = more && n_in - nb * ngood >= (size_t)N;
+            avail = more ? (whole ? N : (int)(n_in - nb * ngood)) : 0;
+        }
         float2 ua[16], ub[16], nxa[16], nxb[16];
         p1_unload(ua, ub);
         p1_emit(ua, dstg + ca, ca, keep);
@@ -267,7 +343,10 @@ fastfir16k_kernel(const float2 *__restrict__ in, size_t n_in, float2 *__restrict
 #pragma unroll
         for (int r = 0; r < 16; ++r)
             nxb[r] = (whole || ca + 32 + 1024 * r < avail) ? ldg_nc_f2(src + 1024 * r + 32) : make_float2(0.f, 0.f);
-        if (more) p1_forward(nxa, nxb);
+        if (fuse) p1_forward(nxa, nxb);
+        c = nc;
+        bc = nbc;
+        loaded = fuse;
     }
 }
 
@@ -284,17 +363,27 @@ void lrc_fastfir16k_permute_H(const float2 *H, float2 *Hq)
 
 int lrc_fastfir16k_prepare(void)
 {
-    LRC_CUDA(cudaFuncSetAttribute(fastfir16k_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ff16k::SMEM_BYTES));
+    LRC_CUDA(cudaFuncSetAttribute(fastfir16k_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ff16k::SMEM_BYTES));
+    LRC_CUDA(cudaFuncSetAttribute(fastfir16k_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ff16k::SMEM_BYTES));
     return LRC_OK;
 }
 
+// nblk: the work items (blocks of the one batch channel, or channels x blocks per channel of a stream push)
 int lrc_fastfir16k_launch(int n_sm, const float2 *in, size_t n_in, float2 *out, size_t full, size_t nblk, size_t ngood,
-                          size_t keep, const float2 *d_tw16k, const float2 *d_tw1k, const float2 *d_Hq, cudaStream_t s)
+                          size_t keep, const float2 *d_tw16k, const float2 *d_tw1k, const float2 *d_Hq,
+                          const FfStreamArgs *sa, cudaStream_t s)
 {
     size_t blocks = (size_t)n_sm;                    // one CTA per SM (216.5 KB of shared memory)
     if (blocks > nblk) blocks = nblk;
-    fastfir16k_kernel<<<(unsigned)blocks, ff16k::NT, ff16k::SMEM_BYTES, s>>>(in, n_in, out, full, nblk, ngood, keep, d_tw16k,
-                                                                          d_tw1k, reinterpret_cast<const float4 *>(d_Hq));
+    FfStreamArgs a{};
+    if (sa) {
+        a = *sa;
+        a.step_c = blocks / a.nblk;
+        a.step_b = blocks % a.nblk;
+    }
+    auto kern = sa ? fastfir16k_kernel<true> : fastfir16k_kernel<false>;
+    kern<<<(unsigned)blocks, ff16k::NT, ff16k::SMEM_BYTES, s>>>(in, n_in, out, full, nblk, ngood, keep, d_tw16k, d_tw1k,
+                                                             reinterpret_cast<const float4 *>(d_Hq), a);
     LRC_CUDA(cudaGetLastError());
     return LRC_OK;
 }

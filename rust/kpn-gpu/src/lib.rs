@@ -14,6 +14,7 @@
 //! |-------------------------------------------------|----------------------------------------|
 //! | `rtlsdr::data_to_samples` rtlsdr.rs:160-162      | [`data_to_samples`]                    |
 //! | `dsputils::convolve` (+ /D) dsputils.rs:30-32    | [`fir_decimate`], [`fir_decimate_multi`] (channel ring) |
+//! | `kiss_fastfir` (streaming) kiss_fastfir.c:228-245 | [`fast_fir_multi`] (channel ring)      |
 //! | `kissfft::fft` kissfft.rs:18-31                  | [`fft`]                                |
 //! | `samplerate::resample` samplerate.rs:59-87       | [`resample`]                           |
 //! | (north-star) discriminator                      | [`fm_demod`]                           |
@@ -113,6 +114,8 @@ macro_rules! plan_guard {
 }
 plan_guard!(FirPlan, sys::lrc_fir, sys::lrc_fir_destroy);
 plan_guard!(FirStreamPlan, sys::lrc_fir_stream, sys::lrc_fir_stream_destroy);
+plan_guard!(FastFirPlan, sys::lrc_fastfir, sys::lrc_fastfir_destroy);
+plan_guard!(FastFirStreamPlan, sys::lrc_fastfir_stream, sys::lrc_fastfir_stream_destroy);
 plan_guard!(FftPlan, sys::lrc_fft, sys::lrc_fft_destroy);
 plan_guard!(ResamplerPlan, sys::lrc_resampler, sys::lrc_resampler_destroy);
 plan_guard!(ChainPlan, sys::lrc_chain, sys::lrc_chain_destroy);
@@ -245,6 +248,50 @@ pub fn fir_decimate_multi(gpu: &Gpu, u: Vec<Receiver<Vec<Cf32>>>, v: Vec<Sender<
         r.inp.h2d(n_ch * chunk_len * 8, &st);
         check(unsafe { sys::lrc_fir_stream_push(fs.0, r.inp.d, chunk_len, chunk_len, r.out.d as *mut f32, cap, &mut r.n_out, st.0) },
               "lrc_fir_stream_push");
+        r.out.d2h(n_ch * cap * 8, &st);
+        r.done.record(&st);
+        r.busy = true;
+        drain(other);                                                    // hand out the batch submitted one step ago
+        it += 1;
+    }
+}
+
+/// Long FIR by overlap-save over MANY channels (`kiss_fastfir` with a carried offset, tools/kiss_fastfir.c:228-245): the
+/// channel ring of [`fir_decimate_multi`] over `lrc_fastfir_stream_push`, one chunk (`chunk_len` samples) per channel per
+/// batch, one push per batch.  Outputs come as whole compute blocks complete (a batch that completes none sends nothing);
+/// per channel they are a prefix of `lrc_fastfir_run` over the channel's whole input.  Never flushes: ports never end.
+pub fn fast_fir_multi(gpu: &Gpu, u: Vec<Receiver<Vec<Cf32>>>, v: Vec<Sender<Vec<Cf32>>>, h: &[Cf32], nfft: usize, chunk_len: usize) {
+    let n_ch = u.len();
+    assert!(v.len() == n_ch && n_ch > 0, "fast_fir_multi: port count mismatch");
+    let mut ff = ptr::null_mut();
+    check(unsafe { sys::lrc_fastfir_create(gpu.0, h.as_ptr() as *const f32, h.len(), nfft, &mut ff) }, "lrc_fastfir_create");
+    let ff = FastFirPlan(ff);
+    let mut fs = ptr::null_mut();
+    check(unsafe { sys::lrc_fastfir_stream_create(ff.0, n_ch, &mut fs) }, "lrc_fastfir_stream_create");
+    let fs = FastFirStreamPlan(fs);
+    let cap = chunk_len + 16384;                                         // the history is shorter than one compute block
+    let st = Stream::new(gpu);
+    let mut ring: Vec<RingSlot> = (0..2).map(|_| RingSlot { inp: Slot::new(gpu), out: Slot::new(gpu), done: Event::new(gpu), n_out: 0, busy: false }).collect();
+    for r in ring.iter_mut() { r.inp.reserve(n_ch * chunk_len * 8); r.out.reserve(n_ch * cap * 8); }
+    let drain = |r: &mut RingSlot| {
+        if !r.busy { return; }
+        r.done.sync();
+        if r.n_out > 0 { for c in 0..n_ch { v[c].send(r.out.take::<Cf32>(c * cap, r.n_out)).unwrap(); } }
+        r.busy = false;
+    };
+    let mut it = 0usize;
+    loop {
+        let (a, b) = ring.split_at_mut(1);
+        let (r, other) = if it & 1 == 0 { (&mut a[0], &mut b[0]) } else { (&mut b[0], &mut a[0]) };
+        drain(r);                                                        // slot reuse: its previous batch must be out
+        for c in 0..n_ch {
+            let x = u[c].recv().unwrap();
+            assert!(x.len() == chunk_len, "fast_fir_multi: chunk length != chunk_len");
+            r.inp.put(c * chunk_len, &x);
+        }
+        r.inp.h2d(n_ch * chunk_len * 8, &st);
+        check(unsafe { sys::lrc_fastfir_stream_push(fs.0, r.inp.d as *const f32, chunk_len, chunk_len, r.out.d as *mut f32, cap, 0,
+                                                    &mut r.n_out, st.0) }, "lrc_fastfir_stream_push");
         r.out.d2h(n_ch * cap * 8, &st);
         r.done.record(&st);
         r.busy = true;

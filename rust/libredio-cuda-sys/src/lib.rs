@@ -15,8 +15,8 @@ pub const LRC_WINDOW_NONE: c_int = 0;
 pub const LRC_WINDOW_HANN: c_int = 1;
 
 macro_rules! opaque { ($($n:ident),*) => { $( #[repr(C)] pub struct $n { _p: [u8; 0] } )* } }
-opaque!(lrc_ctx, lrc_fir, lrc_fir_stream, lrc_fft, lrc_rfft, lrc_psd, lrc_chain, lrc_fastfir, lrc_resampler, lrc_fmrx, lrc_ook,
-        lrc_ook_stream, lrc_gather);
+opaque!(lrc_ctx, lrc_fir, lrc_fir_stream, lrc_fft, lrc_rfft, lrc_psd, lrc_chain, lrc_fastfir, lrc_fastfir_stream, lrc_resampler,
+        lrc_fmrx, lrc_ook, lrc_ook_stream, lrc_gather);
 
 #[repr(C)]
 #[derive(Clone, Copy)]
@@ -106,6 +106,14 @@ extern "C" {
     pub fn lrc_fastfir_out_len(ff: *const lrc_fastfir, n_in: size_t, flush: c_int) -> size_t;
     pub fn lrc_fastfir_run(ff: *mut lrc_fastfir, d_in: *const c_float, n_in: size_t, d_out: *mut c_float, flush: c_int,
                            n_out: *mut size_t, stream: *mut c_void) -> c_int;
+    // streaming overlap-save over many channels (kiss_fastfir with a carried offset, tools/kiss_fastfir.c:228-245)
+    pub fn lrc_fastfir_stream_create(ff: *mut lrc_fastfir, n_ch: size_t, st: *mut *mut lrc_fastfir_stream) -> c_int;
+    pub fn lrc_fastfir_stream_destroy(st: *mut lrc_fastfir_stream) -> c_int;
+    pub fn lrc_fastfir_stream_reset(st: *mut lrc_fastfir_stream) -> c_int;
+    pub fn lrc_fastfir_stream_next_out_len(st: *const lrc_fastfir_stream, n: size_t, flush: c_int) -> size_t;
+    pub fn lrc_fastfir_stream_push(st: *mut lrc_fastfir_stream, d_chunk: *const c_float, n: size_t, chunk_stride: size_t,
+                                   d_out: *mut c_float, out_stride: size_t, flush: c_int, n_out: *mut size_t,
+                                   stream: *mut c_void) -> c_int;
 
     pub fn lrc_fmdemod_run(ctx: *mut lrc_ctx, d_in: *const c_float, n_ch: size_t, n: size_t, in_stride: size_t,
                            d_state: *mut c_float, d_out: *mut c_float, out_stride: size_t, stream: *mut c_void) -> c_int;
