@@ -273,11 +273,8 @@ static int launch_one(const Args &a)
         return -1;
     } else {
         auto kern = chain_gen_kernel<NTAPS, DECIM, LOG2N, R>;
-        LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        int occ = 1;
-        LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, Cfg::NT, Cfg::SMEM_BYTES));
-        if (occ < 1) occ = 1;
-        size_t blocks = (size_t)a.n_sm * occ;
+        size_t blocks;
+        LRC_CUDA(lrc_resident_ctas(kern, Cfg::NT, Cfg::SMEM_BYTES, a.n_sm, &blocks));
         if (blocks > a.n_items) blocks = a.n_items;
         FirTaps<NTAPS> taps;
         for (int i = 0; i < NTAPS; ++i) taps.h[i] = i < a.ntaps ? a.taps[i] : 0.0f;

@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <new>
 #include "../../include/libredio_cuda.h"
+#include "devbuf.h"
 
 // ---------------------------------------------------------------------------------------------
 // context + error plumbing
@@ -65,6 +66,23 @@ static inline size_t lrc_grid_mult(const char *env_name, size_t dflt)
     if (!e) return dflt;
     const long v = atol(e);
     return v > 0 ? (size_t)v : dflt;
+}
+
+// CTAs of `kern` resident on the whole device at `threads` threads and `smem` bytes of dynamic shared memory:
+// n_sm * occupancy, occupancy at least 1.  Raises the kernel's dynamic shared-memory limit to `smem` first; with
+// above_default_only, only when smem exceeds the 48 KB default (kernels whose size follows the plan, launched per call:
+// below the default the limit is left alone and the launch costs no extra driver call).
+template <typename Kernel>
+static inline cudaError_t lrc_resident_ctas(Kernel kern, int threads, size_t smem, int n_sm, size_t *ctas,
+                                            bool above_default_only = false)
+{
+    int occ = 1;
+    cudaError_t e = cudaSuccess;
+    if (!above_default_only || smem > 48 * 1024)
+        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem);
+    *ctas = (size_t)n_sm * (occ < 1 ? 1 : occ);
+    return e;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -107,9 +107,14 @@ extern "C" int lrc_ctx_create(int device, lrc_ctx **out)
     c->n_sm = prop.multiProcessorCount;
     c->numa_node = gpu_numa_node(device);
     c->numa_nodes = online_numa_nodes();
-    LRC_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-    LRC_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-    LRC_CUDA(cudaStreamCreateWithFlags(&c->out_stream, cudaStreamNonBlocking));
+    cudaError_t e = cudaSuccess;
+    for (cudaStream_t *s : {&c->stream, &c->copy_stream, &c->out_stream})
+        if (e == cudaSuccess) e = cudaStreamCreateWithFlags(s, cudaStreamNonBlocking);
+    if (e != cudaSuccess) {
+        lrc_set_error("lrc_ctx_create: cudaStreamCreateWithFlags -> %s", cudaGetErrorString(e));
+        lrc_ctx_destroy(c);
+        return LRC_ERR_CUDA;
+    }
     *out = c;
     return LRC_OK;
 }
@@ -118,9 +123,8 @@ extern "C" int lrc_ctx_destroy(lrc_ctx *c)
 {
     if (!c) return LRC_OK;
     cudaSetDevice(c->device);
-    cudaStreamDestroy(c->stream);
-    cudaStreamDestroy(c->copy_stream);
-    cudaStreamDestroy(c->out_stream);
+    for (cudaStream_t s : {c->stream, c->copy_stream, c->out_stream})
+        if (s) cudaStreamDestroy(s);
     delete c;
     return LRC_OK;
 }

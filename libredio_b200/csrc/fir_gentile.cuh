@@ -91,13 +91,11 @@ static int launch(int n_sm, const float *h_taps, int ntaps, const float *d_in, s
     constexpr int R = RFor<DECIM>::R, NT = 128;
     using C = Cfg<NTAPS, DECIM, R, NT>;
     auto kern = fir_gentile_kernel<NTAPS, DECIM, R, NT>;
-    LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
-    int occ = 1;
-    LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, C::SMEM_BYTES));
-    if (occ < 1) occ = 1;
+    size_t ctas;
+    LRC_CUDA(lrc_resident_ctas(kern, NT, C::SMEM_BYTES, n_sm, &ctas));
     const size_t n_tiles = ceil_div(n_out, (size_t)C::TILE_OUT) * n_ch;
     static const size_t gm = lrc_grid_mult("LRC_FIR_GRID", 1024);
-    size_t blocks = (size_t)n_sm * occ * gm;
+    size_t blocks = ctas * gm;
     if (blocks > n_tiles) blocks = n_tiles;
     // TMA needs 16-byte aligned sources: base, and the channel stride when there is more than one channel row
     const int use_tma = (((uintptr_t)d_in & 15) == 0) && (n_ch == 1 || in_stride % 2 == 0);

@@ -23,10 +23,9 @@
 
 using namespace lrfft;
 
-int    lrc_make_twiddles(int nfft, float2 **d_tw);
+int    lrc_make_twiddles(int nfft, DevBuf<float2> &d_tw);
 int    lrc_log2_exact(int n);
 size_t lrc_psd_frames_per_item(size_t k_avg);
-int    lrc_psd_ensure_partial(float **d_partial, size_t *cap, size_t need_floats);
 int    lrc_psd_reduce(const float *d_partial, float *d_rows, int nfft, size_t ipr, size_t n_rows, float scale,
                       int accumulate, cudaStream_t s);
 
@@ -36,18 +35,18 @@ struct lrc_chain {
     bool     fused;            // the BASELINE instance chain_kernel<64,10,10,7> (cf32 and u8 input)
     bool     fused_generic;    // an instance of chain_gen_kernel (chain_generic.cuh): ntaps <= 128, decim in {4,5,8,10,16}, nfft in {512,1024,2048}
     std::vector<float> taps;
-    float2  *d_tw;
-    float   *d_win;
-    float   *d_partial; size_t partial_cap;
+    DevBuf<float2> d_tw;
+    DevBuf<float>  d_win;
+    DevBuf<float>  d_partial;
     // unfused fallback for shapes without a fused instance
     lrc_fir *fir; lrc_psd *psd;
-    float   *d_tmp; size_t tmp_cap;            // decimated signal (floats)
+    DevBuf<float>  d_tmp;                      // decimated signal
     // host ring (lrc_chain_run_host)
-    float   *d_ring[2]; size_t ring_cap;       // samples per slot
-    uint8_t *d_ring_u8[2]; size_t ring_u8_cap; // samples per slot (u8 IQ staging of lrc_chain_run_host_u8)
-    cudaEvent_t ev_ready[2], ev_free[2];
-    float   *d_rows; size_t rows_cap;          // floats
-    float   *d_u8tmp; size_t u8tmp_cap;        // lrc_chain_run_u8 without a fused instance: unpacked input (samples)
+    DevBuf<float>  d_ring[2];                  // cf32
+    DevBuf<uint8_t> d_ring_u8[2];              // u8 IQ staging of lrc_chain_run_host_u8 (2 bytes per sample)
+    DevEvent ev_ready[2], ev_free[2];
+    DevBuf<float>  d_rows;
+    DevBuf<float>  d_u8tmp;                    // lrc_chain_run_u8 without a fused instance: unpacked input (cf32)
 };
 
 template <int NTAPS, int DECIM, int LOG2N, int R>
@@ -259,21 +258,15 @@ extern "C" int lrc_chain_create(lrc_ctx *ctx, const float *h_taps, int ntaps, in
     if (!c->fused && !getenv("LRC_CHAIN_NO_GENERIC")) {
         c->fused_generic = lrc_chaing_has(ntaps, decim, l2, getenv("LRC_CHAIN_GENERIC_ALL") != nullptr);
     }
-    c->d_tw = nullptr; c->d_win = nullptr; c->d_partial = nullptr; c->partial_cap = 0;
-    c->fir = nullptr; c->psd = nullptr; c->d_tmp = nullptr; c->tmp_cap = 0;
-    c->d_ring[0] = c->d_ring[1] = nullptr; c->ring_cap = 0; c->d_rows = nullptr; c->rows_cap = 0;
-    c->d_ring_u8[0] = c->d_ring_u8[1] = nullptr; c->ring_u8_cap = 0;
-    c->d_u8tmp = nullptr; c->u8tmp_cap = 0;
-    c->ev_ready[0] = c->ev_ready[1] = c->ev_free[0] = c->ev_free[1] = nullptr;
     int rc = lrc_fir_create(ctx, h_taps, ntaps, decim, &c->fir);       // also validates the taps
     if (!rc) rc = lrc_psd_create(ctx, nfft, window, &c->psd);
-    if (!rc) rc = lrc_make_twiddles(nfft, &c->d_tw);
+    if (!rc) rc = lrc_make_twiddles(nfft, c->d_tw);
     if (!rc) {
         std::vector<float> w(nfft);
         const double pi = 3.14159265358979323846264338327950288;
         for (int i = 0; i < nfft; ++i)
             w[i] = window == LRC_WINDOW_HANN ? (float)(0.5 - 0.5 * cos(2.0 * pi * i / nfft)) : 1.0f;
-        if (cudaMalloc(&c->d_win, sizeof(float) * nfft) != cudaSuccess ||
+        if (c->d_win.alloc(nfft) != cudaSuccess ||
             cudaMemcpy(c->d_win, w.data(), sizeof(float) * nfft, cudaMemcpyHostToDevice) != cudaSuccess) {
             lrc_set_error("lrc_chain_create: %s", cudaGetErrorString(cudaGetLastError()));
             rc = LRC_ERR_CUDA;
@@ -289,13 +282,6 @@ extern "C" int lrc_chain_destroy(lrc_chain *c)
     if (!c) return LRC_OK;
     cudaSetDevice(c->ctx->device);
     lrc_fir_destroy(c->fir); lrc_psd_destroy(c->psd);
-    cudaFree(c->d_tw); cudaFree(c->d_win); cudaFree(c->d_partial); cudaFree(c->d_tmp);
-    cudaFree(c->d_ring[0]); cudaFree(c->d_ring[1]); cudaFree(c->d_rows);
-    cudaFree(c->d_ring_u8[0]); cudaFree(c->d_ring_u8[1]); cudaFree(c->d_u8tmp);
-    for (int i = 0; i < 2; ++i) {
-        if (c->ev_ready[i]) cudaEventDestroy(c->ev_ready[i]);
-        if (c->ev_free[i]) cudaEventDestroy(c->ev_free[i]);
-    }
     delete c;
     return LRC_OK;
 }
@@ -319,12 +305,10 @@ static int chain_launch_fused(lrc_chain *c, const void *d_in, size_t k_local, si
 {
     using Cfg = ChainCfg<64, 10, 10, 7>;
     auto kern = chain_kernel<64, 10, 10, 7, IS_U8>;
-    LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-    int occ = 1;
-    LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, Cfg::NT, Cfg::SMEM_BYTES));
-    if (occ < 1) occ = 1;
+    size_t ctas;
+    LRC_CUDA(lrc_resident_ctas(kern, Cfg::NT, Cfg::SMEM_BYTES, c->ctx->n_sm, &ctas));
     static const size_t gm = lrc_grid_mult("LRC_CHAIN_GRID", 1);
-    size_t blocks = (size_t)c->ctx->n_sm * occ * gm;
+    size_t blocks = ctas * gm;
     if (blocks > n_items) blocks = n_items;
     FirTaps<64> taps;
     for (int i = 0; i < 64; ++i) taps.h[i] = c->taps[i];
@@ -344,8 +328,8 @@ static int chain_launch(lrc_chain *c, const void *d_in_any, int input_is_u8, siz
     const size_t fpi = lrc_psd_frames_per_item(k_local);
     const size_t ipr = ceil_div(k_local, fpi);
     const size_t n_items = rows_local * ipr;
-    int rc = lrc_psd_ensure_partial(&c->d_partial, &c->partial_cap, n_items * (size_t)c->nfft);
-    if (rc) return rc;
+    LRC_CUDA(c->d_partial.ensure(n_items * (size_t)c->nfft));
+    int rc;
     if (c->fused) {
         rc = input_is_u8 ? chain_launch_fused<true>(c, d_in_any, k_local, fpi, ipr, n_items, s)
                          : chain_launch_fused<false>(c, d_in_any, k_local, fpi, ipr, n_items, s);
@@ -366,11 +350,7 @@ static int chain_launch(lrc_chain *c, const void *d_in_any, int input_is_u8, siz
     const size_t n_frames = rows_local * k_local;
     const size_t n_dec = n_frames * (size_t)c->nfft;
     const size_t n_in = (n_dec - 1) * (size_t)c->decim + c->ntaps;
-    if (c->tmp_cap < n_dec * 2 + (size_t)c->nfft * rows_local) {
-        cudaFree(c->d_tmp); c->d_tmp = nullptr; c->tmp_cap = 0;
-        LRC_CUDA(cudaMalloc(&c->d_tmp, (n_dec * 2 + (size_t)c->nfft * rows_local) * sizeof(float)));
-        c->tmp_cap = n_dec * 2 + (size_t)c->nfft * rows_local;
-    }
+    LRC_CUDA(c->d_tmp.ensure(n_dec * 2 + (size_t)c->nfft * rows_local));
     rc = lrc_fir_run_cf32(c->fir, d_in, 1, n_in, n_in, c->d_tmp, n_dec, s);
     if (rc) return rc;
     float *rows_tmp = c->d_tmp + n_dec * 2;
@@ -412,11 +392,7 @@ extern "C" int lrc_chain_run_u8(lrc_chain *c, const uint8_t *d_iq, size_t n_in, 
         return chain_launch(c, d_iq, 1, rows, k_avg, d_rows, 1.0f / (float)k_avg, 0, s);
     }
     const size_t need = (rows * k_avg - 1) * (size_t)c->nfft * c->decim + (size_t)(c->nfft - 1) * c->decim + c->ntaps;
-    if (c->u8tmp_cap < need) {
-        cudaFree(c->d_u8tmp); c->d_u8tmp = nullptr; c->u8tmp_cap = 0;
-        LRC_CUDA(cudaMalloc(&c->d_u8tmp, need * sizeof(float2)));
-        c->u8tmp_cap = need;
-    }
+    LRC_CUDA(c->d_u8tmp.ensure(need * 2));
     const int urc = lrc_unpack_u8_cf32(c->ctx, d_iq, need * 2, c->d_u8tmp, s);
     if (urc) return urc;
     return chain_launch(c, c->d_u8tmp, 0, rows, k_avg, d_rows, 1.0f / (float)k_avg, 0, s);
@@ -442,26 +418,14 @@ static int chain_run_host_impl(lrc_chain *c, const void *h_in_any, int input_is_
     const size_t seg_frames = slice_rows ? SEG_FRAMES / 16 * 16 : (SEG_FRAMES / k_avg) * k_avg;
     const size_t slot_samples = seg_frames * adv + tail + 8;
     const bool direct_u8 = input_is_u8 && c->fused;     // the fused u8 instance reads the raw slot itself
-    if (!direct_u8 && c->ring_cap < slot_samples) {
-        for (int i = 0; i < 2; ++i) { cudaFree(c->d_ring[i]); c->d_ring[i] = nullptr; }
-        c->ring_cap = 0;
-        for (int i = 0; i < 2; ++i) LRC_CUDA(cudaMalloc(&c->d_ring[i], slot_samples * sizeof(float2)));
-        c->ring_cap = slot_samples;
-    }
-    if (input_is_u8 && c->ring_u8_cap < slot_samples) {
-        for (int i = 0; i < 2; ++i) { cudaFree(c->d_ring_u8[i]); c->d_ring_u8[i] = nullptr; }
-        c->ring_u8_cap = 0;
-        for (int i = 0; i < 2; ++i) LRC_CUDA(cudaMalloc(&c->d_ring_u8[i], slot_samples * 2));
-        c->ring_u8_cap = slot_samples;
-    }
-    if (c->rows_cap < rows * (size_t)c->nfft) {
-        cudaFree(c->d_rows); c->d_rows = nullptr; c->rows_cap = 0;
-        LRC_CUDA(cudaMalloc(&c->d_rows, rows * (size_t)c->nfft * sizeof(float)));
-        c->rows_cap = rows * (size_t)c->nfft;
-    }
     for (int i = 0; i < 2; ++i) {
-        if (!c->ev_ready[i]) LRC_CUDA(cudaEventCreateWithFlags(&c->ev_ready[i], cudaEventDisableTiming));
-        if (!c->ev_free[i]) LRC_CUDA(cudaEventCreateWithFlags(&c->ev_free[i], cudaEventDisableTiming));
+        if (!direct_u8) LRC_CUDA(c->d_ring[i].ensure(slot_samples * 2));
+        if (input_is_u8) LRC_CUDA(c->d_ring_u8[i].ensure(slot_samples * 2));
+    }
+    LRC_CUDA(c->d_rows.ensure(rows * (size_t)c->nfft));
+    for (int i = 0; i < 2; ++i) {
+        LRC_CUDA(c->ev_ready[i].ensure());
+        LRC_CUDA(c->ev_free[i].ensure());
     }
     cudaStream_t cs = c->ctx->copy_stream, ks = c->ctx->stream;
     const size_t total_frames = rows * k_avg;
@@ -489,7 +453,7 @@ static int chain_run_host_impl(lrc_chain *c, const void *h_in_any, int input_is_
             const int urc = lrc_unpack_u8_cf32(c->ctx, c->d_ring_u8[b], ns * 2, c->d_ring[b], ks);
             if (urc) return urc;
         }
-        const void *seg_in = direct_u8 ? (const void *)c->d_ring_u8[b] : (const void *)c->d_ring[b];
+        const void *seg_in = direct_u8 ? (const void *)c->d_ring_u8[b].get() : (const void *)c->d_ring[b].get();
         int rc;
         if (slice_rows) {
             const size_t row = f / k_avg;

@@ -32,16 +32,16 @@
 
 using namespace lrfft;
 
-int lrc_make_twiddles(int nfft, float2 **d_tw);
+int lrc_make_twiddles(int nfft, DevBuf<float2> &d_tw);
 int lrc_log2_exact(int n);
 
 struct lrc_fastfir {
     lrc_ctx *ctx;
     size_t   nh, nfft, ngood;   // nfft/ngood: the block size that fixes the OUTPUT LENGTH (kiss_fastfir's, or the caller's)
     int      log2n;             // log2(nfft): the fastfir_kernel instance when !compute16k
-    float2  *d_tw;              // twiddles of the compute block size (nfft, or 16384)
-    float2  *d_H;               // FFT(h rotated) / compute block size, in the order the plan's kernel reads it
-    float2  *d_tw1k;            // 16384-point kernel: W_1024^k for the warp-level sub-transforms
+    DevBuf<float2> d_tw;        // twiddles of the compute block size (nfft, or 16384)
+    DevBuf<float2> d_H;         // FFT(h rotated) / compute block size, in the order the plan's kernel reads it
+    DevBuf<float2> d_tw1k;      // 16384-point kernel: W_1024^k for the warp-level sub-transforms
     bool     compute16k;        // blocks are COMPUTED 16384 points at a time whatever nfft says (see lrc_fastfir_create)
 };
 
@@ -157,10 +157,11 @@ extern "C" int lrc_fastfir_create(lrc_ctx *ctx, const float *h_taps_cpx, size_t 
     // taps instead of 4097 of 8192.
     const bool c16 = nh > 1024 || nfft >= 8192;
     const size_t nc = c16 ? 16384 : nfft;        // the compute block size
-    lrc_fastfir *f = new (std::nothrow) lrc_fastfir{ctx, nh, nfft, nfft - nh + 1, l2, nullptr, nullptr, nullptr, c16};
+    lrc_fastfir *f = new (std::nothrow) lrc_fastfir();
     LRC_REQUIRE(f != nullptr, LRC_ERR_NOMEM, "out of host memory");
-    int rc = lrc_make_twiddles((int)nc, &f->d_tw);
-    if (!rc && c16) rc = lrc_make_twiddles(1024, &f->d_tw1k);
+    f->ctx = ctx; f->nh = nh; f->nfft = nfft; f->ngood = nfft - nh + 1; f->log2n = l2; f->compute16k = c16;
+    int rc = lrc_make_twiddles((int)nc, f->d_tw);
+    if (!rc && c16) rc = lrc_make_twiddles(1024, f->d_tw1k);
     if (!rc && c16) rc = lrc_fastfir16k_prepare();
     if (rc) { lrc_fastfir_destroy(f); return rc; }
     // H = FFT(h rotated left by nh-1) / nc (:148-169) in f64 on the host, rounded once to f32
@@ -175,7 +176,7 @@ extern "C" int lrc_fastfir_create(lrc_ctx *ctx, const float *h_taps_cpx, size_t 
         const std::vector<float2> Hn(H);
         lrc_fastfir16k_permute_H(Hn.data(), H.data());
     }
-    cudaError_t e = cudaMalloc(&f->d_H, nc * sizeof(float2));
+    cudaError_t e = f->d_H.alloc(nc);
     if (e == cudaSuccess) e = cudaMemcpy(f->d_H, H.data(), nc * sizeof(float2), cudaMemcpyHostToDevice);
     if (e != cudaSuccess) {
         lrc_set_error("lrc_fastfir_create: %s", cudaGetErrorString(e));
@@ -190,7 +191,6 @@ extern "C" int lrc_fastfir_destroy(lrc_fastfir *f)
 {
     if (!f) return LRC_OK;
     cudaSetDevice(f->ctx->device);
-    cudaFree(f->d_tw); cudaFree(f->d_H); cudaFree(f->d_tw1k);
     delete f;
     return LRC_OK;
 }
@@ -222,11 +222,8 @@ static int launch_fastfir(lrc_fastfir *f, const float2 *in, size_t n_in, float2 
     const int threads = FF::T;
     const size_t smem = (size_t)FF::SMEM_CPX * sizeof(float2);
     auto kern = fastfir_kernel<LOG2N, STREAM>;
-    if (smem > 48 * 1024) LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int occ = 1;
-    LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
-    if (occ < 1) occ = 1;
-    size_t blocks = (size_t)f->ctx->n_sm * occ;
+    size_t blocks;
+    LRC_CUDA(lrc_resident_ctas(kern, threads, smem, f->ctx->n_sm, &blocks, true));
     if (blocks > nblk) blocks = nblk;
     kern<<<(unsigned)blocks, threads, smem, s>>>(in, n_in, out, full, nblk, f->ngood, keep, f->d_tw, f->d_H, sa);
     LRC_CUDA(cudaGetLastError());
@@ -271,7 +268,7 @@ struct lrc_fastfir_stream {
     size_t       n_ch;
     size_t       nc, ngood;     // the compute block (nfft, or 16384) and its advance nc - nh + 1
     size_t       held;          // samples every channel carries, < nc
-    float2      *d_carry[2];    // [n_ch][nc] each, ping-pong; d_carry[cur] holds the history
+    DevBuf<float2> d_carry[2];  // [n_ch][nc] each, ping-pong; d_carry[cur] holds the history
     int          cur;
 };
 
@@ -285,9 +282,8 @@ extern "C" int lrc_fastfir_stream_create(lrc_fastfir *f, size_t n_ch, lrc_fastfi
     st->nc = f->compute16k ? 16384 : f->nfft;
     st->ngood = st->nc - f->nh + 1;
     st->held = 0; st->cur = 0;
-    st->d_carry[0] = st->d_carry[1] = nullptr;
     for (auto &p : st->d_carry) {
-        const cudaError_t e = cudaMalloc(&p, n_ch * st->nc * sizeof(float2));
+        const cudaError_t e = p.alloc(n_ch * st->nc);
         if (e != cudaSuccess) {
             lrc_set_error("lrc_fastfir_stream_create: %s", cudaGetErrorString(e));
             lrc_fastfir_stream_destroy(st);
@@ -302,7 +298,6 @@ extern "C" int lrc_fastfir_stream_destroy(lrc_fastfir_stream *st)
 {
     if (!st) return LRC_OK;
     cudaSetDevice(st->ff->ctx->device);
-    cudaFree(st->d_carry[0]); cudaFree(st->d_carry[1]);
     delete st;
     return LRC_OK;
 }

@@ -30,21 +30,20 @@ int lrc_fft_mixed_launch(const lrc_ctx *ctx, int nfft, int inverse, const MixedP
 struct lrc_fft {
     lrc_ctx *ctx;
     int      nfft, log2n, inverse;   // log2n < 0: mixed-radix plan
-    float2  *d_tw;     // exp(-2 pi j k / nfft), k < nfft (forward table; kernels conjugate for inverse)
+    DevBuf<float2> d_tw;     // exp(-2 pi j k / nfft), k < nfft (forward table; kernels conjugate for inverse)
     MixedPlan mixed;
 };
 
 struct lrc_psd {
     lrc_ctx *ctx;
     int      nfft, log2n;
-    float2  *d_tw;
-    float   *d_win;        // nfft window values (all ones for LRC_WINDOW_NONE)
-    float   *d_partial;    // [n_items][nfft] scratch
-    size_t   partial_cap;  // in floats
+    DevBuf<float2> d_tw;
+    DevBuf<float>  d_win;        // nfft window values (all ones for LRC_WINDOW_NONE)
+    DevBuf<float>  d_partial;    // [n_items][nfft] scratch
 };
 
 // twiddles exactly as kiss_fft_alloc builds them (kiss_fft.c:357-363): phase in double, cast to float
-int lrc_make_twiddles(int nfft, float2 **d_tw)
+int lrc_make_twiddles(int nfft, DevBuf<float2> &d_tw)
 {
     std::vector<float2> tw(nfft);
     const double pi = 3.141592653589793238462643383279502884197169399375105820974944;
@@ -52,8 +51,8 @@ int lrc_make_twiddles(int nfft, float2 **d_tw)
         double ph = -2.0 * pi * i / nfft;
         tw[i] = make_float2((float)cos(ph), (float)sin(ph));
     }
-    LRC_CUDA(cudaMalloc(d_tw, sizeof(float2) * nfft));
-    LRC_CUDA(cudaMemcpy(*d_tw, tw.data(), sizeof(float2) * nfft, cudaMemcpyHostToDevice));
+    LRC_CUDA(d_tw.alloc(nfft));
+    LRC_CUDA(cudaMemcpy(d_tw, tw.data(), sizeof(float2) * nfft, cudaMemcpyHostToDevice));
     return LRC_OK;
 }
 
@@ -195,13 +194,11 @@ template <bool INV>
 static int launch_fft1024(const lrc_fft *p, const float2 *in, float2 *out, size_t batch, cudaStream_t s)
 {
     auto kern = fft1024_warp_kernel<INV>;
-    LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, FFTW_SMEM_BYTES));
-    int occ = 1;
-    LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, FFTW_WARPS * 32, FFTW_SMEM_BYTES));
-    if (occ < 1) occ = 1;
+    size_t ctas;
+    LRC_CUDA(lrc_resident_ctas(kern, FFTW_WARPS * 32, FFTW_SMEM_BYTES, p->ctx->n_sm, &ctas));
     size_t blocks = ceil_div(batch, (size_t)FFTW_WARPS);
     static const size_t gm = lrc_grid_mult("LRC_FFT_GRID", 32);
-    const size_t max_blocks = (size_t)p->ctx->n_sm * occ * gm;
+    const size_t max_blocks = ctas * gm;
     if (blocks > max_blocks) blocks = max_blocks;
     kern<<<(unsigned)blocks, FFTW_WARPS * 32, FFTW_SMEM_BYTES, s>>>(in, out, batch, p->d_tw);
     LRC_CUDA(cudaGetLastError());
@@ -218,12 +215,9 @@ static int launch_fft(const lrc_fft *p, const float2 *in, float2 *out, size_t ba
         if (((uintptr_t)in & 15) == 0 && batch >= 64) {
             using Cfg = FftTmaCfg<LOG2N, INV>;
             auto kern = fft_tma_kernel<LOG2N, INV>;
-            LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-            int occ = 1;
-            LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, Cfg::THREADS, Cfg::SMEM_BYTES));
-            if (occ < 1) occ = 1;
+            size_t max_blocks;
+            LRC_CUDA(lrc_resident_ctas(kern, Cfg::THREADS, Cfg::SMEM_BYTES, p->ctx->n_sm, &max_blocks));
             size_t blocks = ceil_div(batch, (size_t)Cfg::G);
-            const size_t max_blocks = (size_t)p->ctx->n_sm * occ;
             if (blocks > max_blocks) blocks = max_blocks;
             kern<<<(unsigned)blocks, Cfg::THREADS, Cfg::SMEM_BYTES, s>>>(in, out, batch, p->d_tw);
             LRC_CUDA(cudaGetLastError());
@@ -284,10 +278,11 @@ extern "C" int lrc_fft_create(lrc_ctx *ctx, int nfft, int inverse, lrc_fft **out
         }
         l2 = -1;
     }
-    lrc_fft *p = new (std::nothrow) lrc_fft{ctx, nfft, l2, inverse ? 1 : 0, nullptr, mp};
+    lrc_fft *p = new (std::nothrow) lrc_fft();
     LRC_REQUIRE(p != nullptr, LRC_ERR_NOMEM, "out of host memory");
-    int rc = lrc_make_twiddles(nfft, &p->d_tw);
-    if (rc) { delete p; return rc; }
+    p->ctx = ctx; p->nfft = nfft; p->log2n = l2; p->inverse = inverse ? 1 : 0; p->mixed = mp;
+    int rc = lrc_make_twiddles(nfft, p->d_tw);
+    if (rc) { lrc_fft_destroy(p); return rc; }
     *out = p;
     return LRC_OK;
 }
@@ -296,7 +291,6 @@ extern "C" int lrc_fft_destroy(lrc_fft *p)
 {
     if (!p) return LRC_OK;
     cudaSetDevice(p->ctx->device);
-    cudaFree(p->d_tw);
     delete p;
     return LRC_OK;
 }
@@ -591,13 +585,11 @@ static int launch_psd(lrc_psd *p, const float2 *in, size_t k_avg, size_t fpi, si
         if (((uintptr_t)in & 15) == 0) {
             if constexpr (LOG2N == 10) {
                 auto kern = psd1024_warp_kernel;
-                LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, PSDW_SMEM_BYTES));
-                int occ = 1;
-                LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, PSDW_WARPS * 32, PSDW_SMEM_BYTES));
-                if (occ < 1) occ = 1;
+                size_t ctas;
+                LRC_CUDA(lrc_resident_ctas(kern, PSDW_WARPS * 32, PSDW_SMEM_BYTES, p->ctx->n_sm, &ctas));
                 size_t blocks = ceil_div(n_items, (size_t)PSDW_WARPS);
                 static const size_t gm = lrc_grid_mult("LRC_PSD_GRID", 16);
-                const size_t max_blocks = (size_t)p->ctx->n_sm * occ * gm;
+                const size_t max_blocks = ctas * gm;
                 if (blocks > max_blocks) blocks = max_blocks;
                 kern<<<(unsigned)blocks, PSDW_WARPS * 32, PSDW_SMEM_BYTES, s>>>(in, p->d_tw, p->d_win, p->d_partial, k_avg, fpi, ipr, n_items);
                 LRC_CUDA(cudaGetLastError());
@@ -605,12 +597,9 @@ static int launch_psd(lrc_psd *p, const float2 *in, size_t k_avg, size_t fpi, si
             } else {
                 using Cfg = PsdTmaCfg<LOG2N>;
                 auto kern = psd_tma_kernel<LOG2N>;
-                LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-                int occ = 1;
-                LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, Cfg::THREADS, Cfg::SMEM_BYTES));
-                if (occ < 1) occ = 1;
+                size_t max_blocks;
+                LRC_CUDA(lrc_resident_ctas(kern, Cfg::THREADS, Cfg::SMEM_BYTES, p->ctx->n_sm, &max_blocks));
                 size_t blocks = ceil_div(n_items, (size_t)Cfg::G);
-                const size_t max_blocks = (size_t)p->ctx->n_sm * occ;
                 if (blocks > max_blocks) blocks = max_blocks;
                 kern<<<(unsigned)blocks, Cfg::THREADS, Cfg::SMEM_BYTES, s>>>(in, p->d_tw, p->d_win, p->d_partial, k_avg, fpi, ipr, n_items);
                 LRC_CUDA(cudaGetLastError());
@@ -622,12 +611,9 @@ static int launch_psd(lrc_psd *p, const float2 *in, size_t k_avg, size_t fpi, si
     const int G = threads / T;
     const size_t smem = (size_t)G * F::SMEM_CPX * sizeof(float2);
     auto kern = psd_kernel<LOG2N>;
-    if (smem > 48 * 1024) LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int occ = 1;
-    LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
-    if (occ < 1) occ = 1;
+    size_t max_blocks;
+    LRC_CUDA(lrc_resident_ctas(kern, threads, smem, p->ctx->n_sm, &max_blocks, true));
     size_t blocks = ceil_div(n_items, (size_t)G);
-    const size_t max_blocks = (size_t)p->ctx->n_sm * occ;
     if (blocks > max_blocks) blocks = max_blocks;
     kern<<<(unsigned)blocks, threads, smem, s>>>(in, p->d_tw, p->d_win, p->d_partial, k_avg, fpi, ipr, n_items);
     LRC_CUDA(cudaGetLastError());
@@ -644,17 +630,20 @@ extern "C" int lrc_psd_create(lrc_ctx *ctx, int nfft, int window, lrc_psd **out)
         return LRC_ERR_UNSUPPORTED;
     }
     LRC_REQUIRE(window == LRC_WINDOW_NONE || window == LRC_WINDOW_HANN, LRC_ERR_INVALID, "unknown window");
-    lrc_psd *p = new (std::nothrow) lrc_psd{ctx, nfft, l2, nullptr, nullptr, nullptr, 0};
+    lrc_psd *p = new (std::nothrow) lrc_psd();
     LRC_REQUIRE(p != nullptr, LRC_ERR_NOMEM, "out of host memory");
-    int rc = lrc_make_twiddles(nfft, &p->d_tw);
-    if (rc) { delete p; return rc; }
+    p->ctx = ctx; p->nfft = nfft; p->log2n = l2;
+    int rc = lrc_make_twiddles(nfft, p->d_tw);
+    if (rc) { lrc_psd_destroy(p); return rc; }
     std::vector<float> w(nfft);
     const double pi = 3.14159265358979323846264338327950288;
     for (int i = 0; i < nfft; ++i)
         w[i] = window == LRC_WINDOW_HANN ? (float)(0.5 - 0.5 * cos(2.0 * pi * i / nfft)) : 1.0f;
-    if (cudaMalloc(&p->d_win, sizeof(float) * nfft) != cudaSuccess) { lrc_psd_destroy(p); lrc_set_error("cudaMalloc window"); return LRC_ERR_CUDA; }
+    if (p->d_win.alloc(nfft) != cudaSuccess) { lrc_psd_destroy(p); lrc_set_error("cudaMalloc window"); return LRC_ERR_CUDA; }
+    rc = lrc_psd_set_window(p, w.data());
+    if (rc) { lrc_psd_destroy(p); return rc; }
     *out = p;
-    return lrc_psd_set_window(p, w.data());
+    return LRC_OK;
 }
 
 extern "C" int lrc_psd_set_window(lrc_psd *p, const float *h_window)
@@ -669,7 +658,6 @@ extern "C" int lrc_psd_destroy(lrc_psd *p)
 {
     if (!p) return LRC_OK;
     cudaSetDevice(p->ctx->device);
-    cudaFree(p->d_tw); cudaFree(p->d_win); cudaFree(p->d_partial);
     delete p;
     return LRC_OK;
 }
@@ -677,16 +665,6 @@ extern "C" int lrc_psd_destroy(lrc_psd *p)
 // frames per work item: small enough that items outnumber resident transform groups several times,
 // large enough that the 4*nfft-byte partial written per item is noise next to fpi*8*nfft bytes read
 size_t lrc_psd_frames_per_item(size_t k_avg) { return k_avg < 16 ? (k_avg ? k_avg : 1) : 16; }
-
-int lrc_psd_ensure_partial(float **d_partial, size_t *cap, size_t need_floats)
-{
-    if (*cap >= need_floats) return LRC_OK;
-    if (*d_partial) cudaFree(*d_partial);
-    *d_partial = nullptr; *cap = 0;
-    LRC_CUDA(cudaMalloc(d_partial, need_floats * sizeof(float)));
-    *cap = need_floats;
-    return LRC_OK;
-}
 
 int lrc_psd_reduce(const float *d_partial, float *d_rows, int nfft, size_t ipr, size_t n_rows, float scale,
                    int accumulate, cudaStream_t s)
@@ -713,8 +691,8 @@ extern "C" int lrc_psd_run(lrc_psd *p, const float *d_in, size_t n_frames, size_
     const size_t fpi = lrc_psd_frames_per_item(k_avg);
     const size_t ipr = ceil_div(k_avg, fpi);
     const size_t n_items = n_rows * ipr;
-    int rc = lrc_psd_ensure_partial(&p->d_partial, &p->partial_cap, n_items * (size_t)p->nfft);
-    if (rc) return rc;
+    LRC_CUDA(p->d_partial.ensure(n_items * (size_t)p->nfft));
+    int rc;
     const float2 *in = (const float2 *)d_in;
     switch (p->log2n) {
 #define PSD_CASE(L) case L: rc = launch_psd<L>(p, in, k_avg, fpi, ipr, n_items, s); break;

@@ -18,7 +18,6 @@
 using namespace lrfft;
 
 struct lrc_fft;                                   // k_fft.cu
-int lrc_make_twiddles(int nfft, float2 **d_tw);
 
 constexpr int MIXED_MAX_FACTORS = 24;
 constexpr int MIXED_MAX_NFFT = 8192;              // 2 x nfft x 8 B of shared memory
@@ -184,10 +183,9 @@ int lrc_fft_mixed_launch(const lrc_ctx *ctx, int nfft, int inverse, const MixedP
 struct lrc_rfft {
     lrc_ctx *ctx;
     int      nfft, ncfft, inverse;
-    lrc_fft *sub;          // complex plan of ncfft points
-    float2  *d_super;      // ncfft/2 super twiddles
-    float2  *d_tmp;        // [batch][ncfft] scratch
-    size_t   tmp_cap;      // in float2
+    lrc_fft *sub;                // complex plan of ncfft points
+    DevBuf<float2> d_super;      // ncfft/2 super twiddles
+    DevBuf<float2> d_tmp;        // [batch][ncfft] scratch
 };
 
 // kiss_fftr.c:93-119: tmp = FFT_ncfft(time data as complex) -> freq[0..ncfft]
@@ -251,10 +249,11 @@ extern "C" int lrc_rfft_create(lrc_ctx *ctx, int nfft, int inverse, lrc_rfft **o
         lrc_set_error("lrc_rfft_create: nfft=%d: real FFT size must be even (kiss_fftr.c:34-37)", nfft);
         return LRC_ERR_INVALID;
     }
-    lrc_rfft *p = new (std::nothrow) lrc_rfft{ctx, nfft, nfft / 2, inverse ? 1 : 0, nullptr, nullptr, nullptr, 0};
+    lrc_rfft *p = new (std::nothrow) lrc_rfft();
     LRC_REQUIRE(p != nullptr, LRC_ERR_NOMEM, "out of host memory");
+    p->ctx = ctx; p->nfft = nfft; p->ncfft = nfft / 2; p->inverse = inverse ? 1 : 0;
     int rc = lrc_fft_create(ctx, p->ncfft, inverse, &p->sub);
-    if (rc) { delete p; return rc; }
+    if (rc) { lrc_rfft_destroy(p); return rc; }
     const int ns = p->ncfft / 2;
     std::vector<float2> sup(ns > 0 ? ns : 1);
     for (int i = 0; i < ns; ++i) {
@@ -262,11 +261,11 @@ extern "C" int lrc_rfft_create(lrc_ctx *ctx, int nfft, int inverse, lrc_rfft **o
         if (inverse) phase *= -1;
         sup[i] = make_float2((float)cos(phase), (float)sin(phase));
     }
-    cudaError_t e = cudaMalloc(&p->d_super, sup.size() * sizeof(float2));
+    cudaError_t e = p->d_super.alloc(sup.size());
     if (e == cudaSuccess) e = cudaMemcpy(p->d_super, sup.data(), sup.size() * sizeof(float2), cudaMemcpyHostToDevice);
     if (e != cudaSuccess) {
         lrc_set_error("lrc_rfft_create: %s", cudaGetErrorString(e));
-        lrc_fft_destroy(p->sub); cudaFree(p->d_super); delete p;
+        lrc_rfft_destroy(p);
         return LRC_ERR_CUDA;
     }
     *out = p;
@@ -278,7 +277,6 @@ extern "C" int lrc_rfft_destroy(lrc_rfft *p)
     if (!p) return LRC_OK;
     cudaSetDevice(p->ctx->device);
     lrc_fft_destroy(p->sub);
-    cudaFree(p->d_super); cudaFree(p->d_tmp);
     delete p;
     return LRC_OK;
 }
@@ -293,19 +291,14 @@ extern "C" int lrc_rfft_run(lrc_rfft *p, const float *d_in, float *d_out, size_t
                 "lrc_rfft_run: buffers must be 8-byte aligned");
     cudaStream_t s = lrc_stream(p->ctx, stream);
     const size_t need = batch * (size_t)p->ncfft;
-    if (p->tmp_cap < need) {
-        if (p->d_tmp) cudaFree(p->d_tmp);
-        p->d_tmp = nullptr; p->tmp_cap = 0;
-        LRC_CUDA(cudaMalloc(&p->d_tmp, need * sizeof(float2)));
-        p->tmp_cap = need;
-    }
+    LRC_CUDA(p->d_tmp.ensure(need));
     const size_t items = batch * (size_t)(p->ncfft / 2 + 1);
     size_t blocks = ceil_div(items, 256);
     const size_t cap = (size_t)p->ctx->n_sm * 16;
     if (blocks > cap) blocks = cap;
     if (!p->inverse) {
         // nfft reals == ncfft complex samples, frames contiguous (kiss_fftr.c:84)
-        int rc = lrc_fft_run(p->sub, d_in, (float *)p->d_tmp, batch, s);
+        int rc = lrc_fft_run(p->sub, d_in, (float *)p->d_tmp.get(), batch, s);
         if (rc) return rc;
         rfft_split_kernel<<<(unsigned)blocks, 256, 0, s>>>(p->d_tmp, (float2 *)d_out, batch, p->ncfft, p->d_super);
         LRC_CUDA(cudaGetLastError());
@@ -313,7 +306,7 @@ extern "C" int lrc_rfft_run(lrc_rfft *p, const float *d_in, float *d_out, size_t
     }
     rfft_merge_kernel<<<(unsigned)blocks, 256, 0, s>>>((const float2 *)d_in, p->d_tmp, batch, p->ncfft, p->d_super);
     LRC_CUDA(cudaGetLastError());
-    return lrc_fft_run(p->sub, (const float *)p->d_tmp, d_out, batch, s);
+    return lrc_fft_run(p->sub, (const float *)p->d_tmp.get(), d_out, batch, s);
 }
 
 extern "C" int lrc_rfft_run_host(lrc_rfft *p, const float *h_in, float *h_out, size_t batch)
@@ -325,16 +318,15 @@ extern "C" int lrc_rfft_run_host(lrc_rfft *p, const float *h_in, float *h_out, s
     const size_t time_b = batch * (size_t)p->nfft * sizeof(float);
     const size_t freq_b = batch * (size_t)(p->ncfft + 1) * sizeof(float2);
     const size_t in_b = p->inverse ? freq_b : time_b, out_b = p->inverse ? time_b : freq_b;
-    float *d_a = nullptr, *d_b = nullptr;
-    LRC_CUDA(cudaMalloc(&d_a, in_b));
-    if (cudaMalloc(&d_b, out_b) != cudaSuccess) { cudaFree(d_a); lrc_set_error("lrc_rfft_run_host: cudaMalloc"); return LRC_ERR_CUDA; }
+    DevBuf<float> d_a, d_b;
+    LRC_CUDA(d_a.alloc(in_b / sizeof(float)));
+    if (d_b.alloc(out_b / sizeof(float)) != cudaSuccess) { lrc_set_error("lrc_rfft_run_host: cudaMalloc"); return LRC_ERR_CUDA; }
     cudaStream_t s = p->ctx->stream;
     cudaError_t e = cudaMemcpyAsync(d_a, h_in, in_b, cudaMemcpyHostToDevice, s);
     int rc = LRC_OK;
     if (e == cudaSuccess) rc = lrc_rfft_run(p, d_a, d_b, batch, s);
     if (e == cudaSuccess && rc == LRC_OK) e = cudaMemcpyAsync(h_out, d_b, out_b, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    cudaFree(d_a); cudaFree(d_b);
     if (e != cudaSuccess) { lrc_set_error("lrc_rfft_run_host: %s", cudaGetErrorString(e)); return LRC_ERR_CUDA; }
     return rc;
 }

@@ -17,8 +17,8 @@ struct lrc_fir {
     lrc_ctx *ctx;
     int      ntaps, decim;
     std::vector<float> taps;      // host copy
-    float   *d_taps;              // device copy (generic path)
-    float   *d_taps127;           // taps / 127 (u8 generic path)
+    DevBuf<float> d_taps;         // device copy (generic path)
+    DevBuf<float> d_taps127;      // taps / 127 (u8 generic path)
 };
 
 struct lrc_fir_stream {
@@ -28,8 +28,8 @@ struct lrc_fir_stream {
     size_t   esize;                  // bytes per sample (8 or 2)
     size_t   held;                   // samples carried at the row fronts
     size_t   skip;                   // samples of future input to drop (only when decim > ntaps)
-    uint8_t *d_buf;                  // [n_ch][cap] staging rows: carry followed by the new chunk
-    uint8_t *d_carry;                // [n_ch][ntaps + decim] scratch for the carry move
+    DevBuf<uint8_t> d_buf;           // [n_ch][cap] staging rows: carry followed by the new chunk
+    DevBuf<uint8_t> d_carry;         // [n_ch][ntaps + decim] scratch for the carry move
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -154,9 +154,7 @@ extern "C" int lrc_fir_create(lrc_ctx *ctx, const float *h_taps, int ntaps, int 
     f->taps.assign(h_taps, h_taps + ntaps);
     std::vector<float> t127(ntaps);
     for (int i = 0; i < ntaps; ++i) t127[i] = (float)((double)h_taps[i] / 127.0);
-    f->d_taps = f->d_taps127 = nullptr;
-    if (cudaMalloc(&f->d_taps, sizeof(float) * ntaps) != cudaSuccess ||
-        cudaMalloc(&f->d_taps127, sizeof(float) * ntaps) != cudaSuccess ||
+    if (f->d_taps.alloc(ntaps) != cudaSuccess || f->d_taps127.alloc(ntaps) != cudaSuccess ||
         cudaMemcpy(f->d_taps, h_taps, sizeof(float) * ntaps, cudaMemcpyHostToDevice) != cudaSuccess ||
         cudaMemcpy(f->d_taps127, t127.data(), sizeof(float) * ntaps, cudaMemcpyHostToDevice) != cudaSuccess) {
         lrc_set_error("lrc_fir_create: %s", cudaGetErrorString(cudaGetLastError()));
@@ -171,7 +169,6 @@ extern "C" int lrc_fir_destroy(lrc_fir *f)
 {
     if (!f) return LRC_OK;
     cudaSetDevice(f->ctx->device);
-    cudaFree(f->d_taps); cudaFree(f->d_taps127);
     delete f;
     return LRC_OK;
 }
@@ -197,13 +194,11 @@ static int fir_launch(lrc_fir *f, const void *d_in, size_t n_ch, size_t n_in, si
         constexpr int R = 7, NT = 128;
         using Cfg = FirTileCfg<64, 10, R, NT, IS_U8>;
         auto kern = fir_tile_kernel<64, 10, R, NT, IS_U8>;
-        LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        int occ = 1;
-        LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, Cfg::SMEM_BYTES));
-        if (occ < 1) occ = 1;
+        size_t ctas;
+        LRC_CUDA(lrc_resident_ctas(kern, NT, Cfg::SMEM_BYTES, f->ctx->n_sm, &ctas));
         const size_t n_tiles = ceil_div(n_out, (size_t)Cfg::TILE_OUT) * n_ch;
         static const size_t gm = lrc_grid_mult(IS_U8 ? "LRC_FIRU8_GRID" : "LRC_FIR_GRID", IS_U8 ? 16 : 1024);
-        size_t blocks = (size_t)f->ctx->n_sm * occ * gm;
+        size_t blocks = ctas * gm;
         if (blocks > n_tiles) blocks = n_tiles;
         // TMA needs 16-byte aligned sources: base, channel stride and (always true) tile stride
         const int use_tma = (((uintptr_t)d_in & 15) == 0) && (n_ch == 1 || (in_stride * ES) % 16 == 0);
@@ -257,9 +252,8 @@ extern "C" int lrc_fir_stream_create(lrc_fir *f, size_t n_ch, size_t max_chunk, 
     // a row holds at most ntaps-1 carried samples plus one chunk; rows are 16-byte multiples so
     // every row start stays TMA-aligned
     st->cap = ((size_t)f->ntaps + max_chunk + 7) / 8 * 8;
-    st->d_buf = st->d_carry = nullptr;
-    if (cudaMalloc(&st->d_buf, n_ch * st->cap * st->esize) != cudaSuccess ||
-        cudaMalloc(&st->d_carry, n_ch * (size_t)(f->ntaps + 8) * st->esize) != cudaSuccess) {
+    if (st->d_buf.alloc(n_ch * st->cap * st->esize) != cudaSuccess ||
+        st->d_carry.alloc(n_ch * (size_t)(f->ntaps + 8) * st->esize) != cudaSuccess) {
         lrc_set_error("lrc_fir_stream_create: %s", cudaGetErrorString(cudaGetLastError()));
         lrc_fir_stream_destroy(st);
         return LRC_ERR_CUDA;
@@ -272,7 +266,6 @@ extern "C" int lrc_fir_stream_destroy(lrc_fir_stream *st)
 {
     if (!st) return LRC_OK;
     cudaSetDevice(st->fir->ctx->device);
-    cudaFree(st->d_buf); cudaFree(st->d_carry);
     delete st;
     return LRC_OK;
 }

@@ -121,10 +121,10 @@ struct lrc_resampler {
     int      L, M;
     size_t   n_ch, max_chunk, tpp, ntaps, cap;   // cap: floats per staging row
     std::vector<double> h;                       // prototype (f64)
-    float   *d_hp;                               // [L][tpp] polyphase rows, f32
-    float   *d_carry[2];                         // [n_ch][tpp] x2: the tpp-1 samples before the next chunk (ping-pong)
+    DevBuf<float> d_hp;                          // [L][tpp] polyphase rows, f32
+    DevBuf<float> d_carry[2];                    // [n_ch][tpp] x2: the tpp-1 samples before the next chunk (ping-pong)
     int      cur;                                // which carry buffer is current
-    float   *d_hin, *d_hout; size_t hin_cap, hout_cap;   // staging for the host entry point (floats)
+    DevBuf<float> d_hin, d_hout;                 // staging for the host entry point
     unsigned long long n_total, m_next;          // inputs consumed / next output index (same for all channels)
 };
 
@@ -305,12 +305,9 @@ static int launch_resample_dec(lrc_resampler *r, const float *d_in, size_t n_in,
     constexpr int NT = 128;
     using Cfg = RsDecCfg<M, R, NT>;
     auto kern = resample_dec_kernel<M, R, NT>;
-    LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-    int occ = 1;
-    LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, Cfg::SMEM_BYTES));
-    if (occ < 1) occ = 1;
+    size_t blocks;
+    LRC_CUDA(lrc_resident_ctas(kern, NT, Cfg::SMEM_BYTES, r->ctx->n_sm, &blocks));
     const size_t n_tiles = ceil_div(no, (size_t)Cfg::TILE_OUT) * r->n_ch;
-    size_t blocks = (size_t)r->ctx->n_sm * occ;
     if (blocks > n_tiles) blocks = n_tiles;
     RsTaps<Cfg::TPP> taps;
     for (int i = 0; i < Cfg::TPP; ++i) taps.g[i] = (float)r->h[Cfg::TPP - 1 - i];      // reversed: correlation form
@@ -451,13 +448,11 @@ static int launch_resample_dec2(lrc_resampler *r, const float *d_in, size_t n_in
     using Cfg = RsDec2Cfg<M, R, NT>;
     constexpr int SMEM = Cfg::SMEM_BYTES;
     auto kern = resample_dec2_kernel<M, R, NT>;
-    LRC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    int occ = 1;
-    LRC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, SMEM));
-    if (occ < 1) occ = 1;
+    size_t ctas;
+    LRC_CUDA(lrc_resident_ctas(kern, NT, SMEM, r->ctx->n_sm, &ctas));
     const size_t n_pairs = (ceil_div(no, (size_t)Cfg::TILE_OUT) * r->n_ch + 1) / 2;
     static const size_t gm = lrc_grid_mult("LRC_RS_GRID", 1024);
-    size_t blocks = (size_t)r->ctx->n_sm * occ * gm;
+    size_t blocks = ctas * gm;
     if (blocks > n_pairs) blocks = n_pairs;
     RsTaps<Cfg::TPP> taps;
     for (int i = 0; i < Cfg::TPP; ++i) taps.g[i] = (float)r->h[Cfg::TPP - 1 - i];      // reversed: correlation form
@@ -504,26 +499,23 @@ extern "C" int lrc_resampler_create(lrc_ctx *ctx, double ratio, size_t n_ch, siz
             if (idx < r->ntaps) hp[(size_t)p * r->tpp + j] = (float)r->h[idx];
         }
     r->cap = (r->tpp + max_chunk + 3) / 4 * 4;
-    r->d_hp = r->d_carry[0] = r->d_carry[1] = nullptr; r->cur = 0;
-    r->d_hin = r->d_hout = nullptr; r->hin_cap = r->hout_cap = 0;
-    r->n_total = 0; r->m_next = 0;
-    if (cudaMalloc(&r->d_hp, hp.size() * sizeof(float)) != cudaSuccess ||
-        cudaMalloc(&r->d_carry[0], n_ch * r->tpp * sizeof(float)) != cudaSuccess ||
-        cudaMalloc(&r->d_carry[1], n_ch * r->tpp * sizeof(float)) != cudaSuccess ||
+    if (r->d_hp.alloc(hp.size()) != cudaSuccess || r->d_carry[0].alloc(n_ch * r->tpp) != cudaSuccess ||
+        r->d_carry[1].alloc(n_ch * r->tpp) != cudaSuccess ||
         cudaMemcpy(r->d_hp, hp.data(), hp.size() * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess) {
         lrc_set_error("lrc_resampler_create: %s", cudaGetErrorString(cudaGetLastError()));
         lrc_resampler_destroy(r);
         return LRC_ERR_CUDA;
     }
+    const int rc = lrc_resampler_reset(r);
+    if (rc) { lrc_resampler_destroy(r); return rc; }
     *out = r;
-    return lrc_resampler_reset(r);
+    return LRC_OK;
 }
 
 extern "C" int lrc_resampler_destroy(lrc_resampler *r)
 {
     if (!r) return LRC_OK;
     cudaSetDevice(r->ctx->device);
-    cudaFree(r->d_hp); cudaFree(r->d_carry[0]); cudaFree(r->d_carry[1]); cudaFree(r->d_hin); cudaFree(r->d_hout);
     delete r;
     return LRC_OK;
 }
@@ -635,16 +627,8 @@ extern "C" int lrc_resampler_process_host(lrc_resampler *r, const float *h_in, s
     LRC_REQUIRE(h_in != nullptr, LRC_ERR_INVALID, "lrc_resampler_process_host: null input");
     const size_t no = lrc_resampler_next_out_len(r, n_in);
     LRC_REQUIRE(no == 0 || (h_out && out_cap >= no), LRC_ERR_CAPACITY, "lrc_resampler_process_host: output too small");
-    if (r->hin_cap < r->n_ch * n_in) {
-        cudaFree(r->d_hin); r->d_hin = nullptr; r->hin_cap = 0;
-        LRC_CUDA(cudaMalloc(&r->d_hin, r->n_ch * n_in * sizeof(float)));
-        r->hin_cap = r->n_ch * n_in;
-    }
-    if (r->hout_cap < r->n_ch * (no + 1)) {
-        cudaFree(r->d_hout); r->d_hout = nullptr; r->hout_cap = 0;
-        LRC_CUDA(cudaMalloc(&r->d_hout, r->n_ch * (no + 1) * sizeof(float)));
-        r->hout_cap = r->n_ch * (no + 1);
-    }
+    LRC_CUDA(r->d_hin.ensure(r->n_ch * n_in));
+    LRC_CUDA(r->d_hout.ensure(r->n_ch * (no + 1)));
     cudaStream_t s = r->ctx->stream;
     LRC_CUDA(cudaMemcpyAsync(r->d_hin, h_in, r->n_ch * n_in * sizeof(float), cudaMemcpyHostToDevice, s));
     size_t got = 0;

@@ -281,11 +281,12 @@ struct lrc_fmrx {
     // fused instance (64 taps / 10, ratio 1/5)
     FirTaps<fmrx::NTAPS> taps127;
     RsTaps<fmrx::TPP>    rtaps;
-    uint8_t *d_carry[2]; int cur; size_t carry_stride;    // bytes per channel row
+    DevBuf<uint8_t> d_carry[2]; int cur; size_t carry_stride;    // bytes per channel row
     long long held, n_raw, m_next;
     // composition for every other shape: the three stand-alone stages with their own carried state
     lrc_fir *fir; lrc_fir_stream *fs; lrc_resampler *rs;
-    float   *d_bb, *d_fm, *d_state; size_t bb_cap;
+    DevBuf<float> d_bb, d_fm, d_state;                    // [n_ch][bb_stride] cf32, [n_ch][bb_stride] f32, [n_ch] cf32
+    size_t   bb_stride;
     int      decim, ntaps, rs_L, rs_M;
 };
 
@@ -300,8 +301,6 @@ extern "C" int lrc_fmrx_create(lrc_ctx *ctx, const float *h_taps, int ntaps, int
     lrc_fmrx *f = new (std::nothrow) lrc_fmrx();
     LRC_REQUIRE(f != nullptr, LRC_ERR_NOMEM, "out of host memory");
     f->ctx = ctx; f->n_ch = n_ch; f->max_chunk = max_chunk; f->decim = decim; f->ntaps = ntaps;
-    f->d_carry[0] = f->d_carry[1] = nullptr; f->cur = 0; f->carry_stride = 0; f->held = f->n_raw = f->m_next = 0;
-    f->fir = nullptr; f->fs = nullptr; f->rs = nullptr; f->d_bb = f->d_fm = f->d_state = nullptr; f->bb_cap = 0;
     f->fused = ntaps == fmrx::NTAPS && decim == fmrx::DECIM && fabs(ratio - 0.2) < 1e-15;
     // both forms need the plans: the fused one takes its taps from them (one designer, one rounding)
     int rc = lrc_fir_create(ctx, h_taps, ntaps, decim, &f->fir);           // validates the taps (finite)
@@ -322,7 +321,7 @@ extern "C" int lrc_fmrx_create(lrc_ctx *ctx, const float *h_taps, int ntaps, int
         for (int i = 0; i < fmrx::TPP; ++i) f->rtaps.g[i] = (float)h[fmrx::TPP - 1 - i];      // reversed: correlation form
         f->carry_stride = FMRX_CARRY_CAP * 2;
         for (int i = 0; i < 2; ++i) {
-            if (cudaMalloc(&f->d_carry[i], n_ch * f->carry_stride) != cudaSuccess) {
+            if (f->d_carry[i].alloc(n_ch * f->carry_stride) != cudaSuccess) {
                 lrc_set_error("lrc_fmrx_create: %s", cudaGetErrorString(cudaGetLastError()));
                 lrc_fmrx_destroy(f);
                 return LRC_ERR_CUDA;
@@ -333,10 +332,9 @@ extern "C" int lrc_fmrx_create(lrc_ctx *ctx, const float *h_taps, int ntaps, int
     } else {
         rc = lrc_fir_stream_create(f->fir, n_ch, max_chunk, 1, &f->fs);
         if (!rc) {
-            f->bb_cap = bb_max;
-            if (cudaMalloc(&f->d_bb, n_ch * bb_max * sizeof(float2)) != cudaSuccess ||
-                cudaMalloc(&f->d_fm, n_ch * bb_max * sizeof(float)) != cudaSuccess ||
-                cudaMalloc(&f->d_state, n_ch * sizeof(float2)) != cudaSuccess ||
+            f->bb_stride = bb_max;
+            if (f->d_bb.alloc(n_ch * bb_max * 2) != cudaSuccess || f->d_fm.alloc(n_ch * bb_max) != cudaSuccess ||
+                f->d_state.alloc(n_ch * 2) != cudaSuccess ||
                 cudaMemset(f->d_state, 0, n_ch * sizeof(float2)) != cudaSuccess) {
                 lrc_set_error("lrc_fmrx_create: %s", cudaGetErrorString(cudaGetLastError()));
                 rc = LRC_ERR_CUDA;
@@ -352,7 +350,6 @@ extern "C" int lrc_fmrx_destroy(lrc_fmrx *f)
 {
     if (!f) return LRC_OK;
     cudaSetDevice(f->ctx->device);
-    cudaFree(f->d_carry[0]); cudaFree(f->d_carry[1]); cudaFree(f->d_bb); cudaFree(f->d_fm); cudaFree(f->d_state);
     lrc_fir_stream_destroy(f->fs); lrc_resampler_destroy(f->rs); lrc_fir_destroy(f->fir);
     delete f;
     return LRC_OK;
@@ -388,13 +385,13 @@ extern "C" int lrc_fmrx_push(lrc_fmrx *f, const uint8_t *d_iq, size_t n, size_t 
     if (!f->fused) {
         size_t n_bb = 0, n_a = 0;
         f->n_raw += (long long)n;
-        int rc = lrc_fir_stream_push(f->fs, d_iq, n, chunk_stride, (float *)f->d_bb, f->bb_cap, &n_bb, s);
+        int rc = lrc_fir_stream_push(f->fs, d_iq, n, chunk_stride, f->d_bb, f->bb_stride, &n_bb, s);
         if (rc || n_bb == 0) return rc;
-        rc = lrc_fmdemod_run(f->ctx, (const float *)f->d_bb, f->n_ch, n_bb, f->bb_cap, f->d_state, f->d_fm, f->bb_cap, s);
+        rc = lrc_fmdemod_run(f->ctx, f->d_bb, f->n_ch, n_bb, f->bb_stride, f->d_state, f->d_fm, f->bb_stride, s);
         if (rc) return rc;
         const size_t want = lrc_resampler_next_out_len(f->rs, n_bb);
         LRC_REQUIRE(want == 0 || (d_audio && out_stride >= want), LRC_ERR_CAPACITY, "lrc_fmrx_push: output too small");
-        rc = lrc_resampler_process(f->rs, f->d_fm, n_bb, f->bb_cap, d_audio, out_stride, &n_a, s);
+        rc = lrc_resampler_process(f->rs, f->d_fm, n_bb, f->bb_stride, d_audio, out_stride, &n_a, s);
         f->m_next += (long long)n_a;
         *n_out = n_a;
         return rc;

@@ -107,27 +107,27 @@ struct lrc_ook {
     size_t   n_streams, n_blocks, max_runs, max_packets, max_bursts;
     unsigned sample_rate;
     uint32_t guard_samples;           // bitfount.rs:52 1000 * trigger_duration * block_size (LRC_OOK_TEST_GUARD_BLOCKS: a test hook)
-    float    *d_sum, *d_max;          // [n_streams][n_blocks]
-    int32_t  *d_tag;                  // [n_streams][n_blocks] burst index the block is collected into, -1 = none
-    float    *d_half;                 // [n_streams][max_bursts]  max/2 of the burst
-    uint8_t  *d_bflags;               // [n_streams][max_bursts]  bit0 = emitted, bit1 = leading 0.0 sample
-    uint32_t *d_bend;                 // [n_streams][max_bursts]  last block that can belong to the burst (the one that sent / dropped it)
-    uint32_t *d_nbursts;              // [n_streams]
-    uint32_t *d_trans;                // [n_streams][max_runs] positions where the bit stream changes value
-    uint32_t *d_ntrans;               // [n_streams]  (may exceed max_runs: overflow is detected on fetch)
-    uint32_t *d_nbits;                // [n_streams]  length of the flattened bit stream
-    unsigned long long *d_packets;    // [n_streams][2][max_packets] packets packed MSB-first
-    uint32_t *d_npackets;             // [n_streams][2]
-    uint32_t *d_runs_dbg;             // [n_streams][max_runs] (value << 31 | length), filled by K-D
-    float    *d_flut;                 // folded envelope table, OOK_FLUT_N floats (the block-sum kernel's)
+    DevBuf<float>    d_sum, d_max;    // [n_streams][n_blocks]
+    DevBuf<int32_t>  d_tag;           // [n_streams][n_blocks] burst index the block is collected into, -1 = none
+    DevBuf<float>    d_half;          // [n_streams][max_bursts]  max/2 of the burst
+    DevBuf<uint8_t>  d_bflags;        // [n_streams][max_bursts]  bit0 = emitted, bit1 = leading 0.0 sample
+    DevBuf<uint32_t> d_bend;          // [n_streams][max_bursts]  last block that can belong to the burst (the one that sent / dropped it)
+    DevBuf<uint32_t> d_nbursts;       // [n_streams]
+    DevBuf<uint32_t> d_trans;         // [n_streams][max_runs] positions where the bit stream changes value
+    DevBuf<uint32_t> d_ntrans;        // [n_streams]  (may exceed max_runs: overflow is detected on fetch)
+    DevBuf<uint32_t> d_nbits;         // [n_streams]  length of the flattened bit stream
+    DevBuf<unsigned long long> d_packets;   // [n_streams][2][max_packets] packets packed MSB-first
+    DevBuf<uint32_t> d_npackets;      // [n_streams][2]
+    DevBuf<uint32_t> d_runs_dbg;      // [n_streams][max_runs] (value << 31 | length), filled by K-D
+    DevBuf<float>    d_flut;          // folded envelope table, OOK_FLUT_N floats (the block-sum kernel's)
     void     *encode_tiled;           // cuTensorMapEncodeTiled (driver entry point, fetched once)
-    uint16_t *d_mask;                 // [n_streams][n_blocks][32] slicer output of collected blocks, 512 bits each (K-C)
-    uint32_t *d_hrank;                // [n_streams][max_bursts] rank threshold of a sent burst (K-C)
-    uint32_t *d_next;                 // [1] next (stream, group) the slice kernel hands out
-    uint32_t *d_bsum;                 // [n_streams][n_blocks] {inner transitions, first bit, last bit} of a collected block
-    uint4    *d_binfo;                // [n_streams][n_blocks] place of a collected block in the bit stream and the transition list
-    uint16_t *d_rank;                 // [65536] rank of the pair's envelope among the distinct envelope values
-    float    *d_uniq;                 // [n_uniq] the distinct envelope values, ascending
+    DevBuf<uint16_t> d_mask;          // [n_streams][n_blocks][32] slicer output of collected blocks, 512 bits each (K-C)
+    DevBuf<uint32_t> d_hrank;         // [n_streams][max_bursts] rank threshold of a sent burst (K-C)
+    DevBuf<uint32_t> d_next;          // [1] next (stream, group) the slice kernel hands out
+    DevBuf<uint32_t> d_bsum;          // [n_streams][n_blocks] {inner transitions, first bit, last bit} of a collected block
+    DevBuf<uint4>    d_binfo;         // [n_streams][n_blocks] place of a collected block in the bit stream and the transition list
+    DevBuf<uint16_t> d_rank;          // [65536] rank of the pair's envelope among the distinct envelope values
+    DevBuf<float>    d_uniq;          // [n_uniq] the distinct envelope values, ascending
     uint32_t  n_uniq;
     size_t    cpitch;                 // carry slots per stream in front of the blocks of d_mask / d_bsum / d_binfo (0: batch plan)
 };
@@ -1271,6 +1271,32 @@ __global__ void ook_envelope_table_kernel(float *__restrict__ table)
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
+// bitfount.rs:52 `1000*trigger_duration*block_size`.  LRC_OOK_TEST_GUARD_BLOCKS shrinks it (in blocks) so that a test can reach
+// the guard with a capture of a few hundred blocks instead of 50 000; the oracle has the same hook (orc_test_set_trigger_guard)
+static size_t ook_guard_blocks()
+{
+    if (const char *g = getenv("LRC_OOK_TEST_GUARD_BLOCKS")) { const long v = atol(g); if (v >= 1) return (size_t)v; }
+    return 1000u * (size_t)OOK_TRIGGER_DURATION;
+}
+
+// stream s's packets of both protocols from the matcher's output pk ([stream][2][mp], packed MSB-first): n[proto] of them,
+// numbered from seq0[proto], written from `out` on; returns the end of what it wrote
+static lrc_ook_packet *ook_put_packets(lrc_ook_packet *out, const unsigned long long *pk, size_t mp, size_t s, const uint32_t n[2],
+                                       const uint32_t seq0[2])
+{
+    for (int proto = 0; proto < 2; ++proto) {
+        const uint32_t nbits = proto == 0 ? 36u : 24u;
+        for (uint32_t k = 0; k < n[proto]; ++k) {
+            lrc_ook_packet &p = *out++;
+            p.stream = (uint32_t)s; p.proto = (uint32_t)proto; p.seq = seq0[proto] + k; p.nbits = nbits;
+            memset(p.bits, 0, sizeof(p.bits));
+            const unsigned long long v = pk[(s * 2 + proto) * mp + k];
+            for (uint32_t i = 0; i < nbits; ++i) p.bits[i] = (uint8_t)((v >> (nbits - 1 - i)) & 1ull);
+        }
+    }
+    return out;
+}
+
 // cpitch: carry slots per stream in front of the blocks of the slicer's per-block arrays (stream plans; 0 for a batch plan)
 static int ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, size_t cpitch, unsigned sample_rate,
                       size_t max_runs, size_t max_packets, lrc_ook **out)
@@ -1282,14 +1308,10 @@ static int ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, size_t cp
                 "lrc_ook_create: too many 32-block groups (2^31)");
     lrc_ook *o = new (std::nothrow) lrc_ook();
     LRC_REQUIRE(o != nullptr, LRC_ERR_NOMEM, "out of host memory");
-    memset(o, 0, sizeof(*o));
     o->ctx = ctx; o->n_streams = n_streams; o->n_blocks = n_blocks; o->sample_rate = sample_rate; o->cpitch = cpitch;
     o->max_runs = max_runs ? max_runs : 4096;
     o->max_packets = max_packets ? max_packets : 64;
-    // bitfount.rs:52 `1000*trigger_duration*block_size`.  LRC_OOK_TEST_GUARD_BLOCKS shrinks it (in blocks) so that a test can reach
-    // the guard with a capture of a few hundred blocks instead of 50 000; the oracle has the same hook (orc_test_set_trigger_guard)
-    size_t guard_blocks = 1000u * (size_t)OOK_TRIGGER_DURATION;
-    if (const char *g = getenv("LRC_OOK_TEST_GUARD_BLOCKS")) { const long v = atol(g); if (v >= 1) guard_blocks = (size_t)v; }
+    const size_t guard_blocks = ook_guard_blocks();
     o->guard_samples = (uint32_t)(guard_blocks * OOK_BLOCK);
     // a sent burst is at least 49 collected blocks, except the pieces the guard cuts one into (an abandoned burst of more than
     // guard_blocks blocks followed by its remainder, possibly empty): at least guard_blocks / 2 blocks per index on average
@@ -1298,7 +1320,7 @@ static int ook_create(lrc_ctx *ctx, size_t n_streams, size_t n_blocks, size_t cp
     o->max_bursts = n_blocks / min_burst + 2 + (cpitch ? 1 : 0);
     const size_t sb = n_streams * n_blocks, sr = n_streams * (cpitch + n_blocks);
     cudaError_t e = cudaSuccess;
-#define OOK_ALLOC(ptr, count) if (e == cudaSuccess) e = cudaMalloc(&o->ptr, (count) * sizeof(*o->ptr))
+#define OOK_ALLOC(buf, count) if (e == cudaSuccess) e = o->buf.alloc(count)
     OOK_ALLOC(d_sum, sb); OOK_ALLOC(d_max, sb); OOK_ALLOC(d_tag, sb);
     OOK_ALLOC(d_half, n_streams * o->max_bursts); OOK_ALLOC(d_bflags, n_streams * o->max_bursts);
     OOK_ALLOC(d_bend, n_streams * o->max_bursts);
@@ -1370,10 +1392,6 @@ extern "C" int lrc_ook_destroy(lrc_ook *o)
 {
     if (!o) return LRC_OK;
     cudaSetDevice(o->ctx->device);
-    cudaFree(o->d_sum); cudaFree(o->d_max); cudaFree(o->d_tag); cudaFree(o->d_half); cudaFree(o->d_bflags); cudaFree(o->d_bend);
-    cudaFree(o->d_nbursts); cudaFree(o->d_trans); cudaFree(o->d_ntrans); cudaFree(o->d_nbits);
-    cudaFree(o->d_packets); cudaFree(o->d_npackets); cudaFree(o->d_runs_dbg); cudaFree(o->d_flut);
-    cudaFree(o->d_rank); cudaFree(o->d_uniq); cudaFree(o->d_mask); cudaFree(o->d_bsum); cudaFree(o->d_binfo); cudaFree(o->d_hrank); cudaFree(o->d_next);
     delete o;
     return LRC_OK;
 }
@@ -1494,18 +1512,8 @@ extern "C" int lrc_ook_fetch_packets(lrc_ook *o, lrc_ook_packet *h_packets, size
     }
     std::vector<unsigned long long> pk(ns * 2 * o->max_packets);
     LRC_CUDA(cudaMemcpy(pk.data(), o->d_packets, pk.size() * 8, cudaMemcpyDeviceToHost));
-    size_t w = 0;
-    for (size_t s = 0; s < ns; ++s)
-        for (int proto = 0; proto < 2; ++proto) {
-            const uint32_t nbits = proto == 0 ? 36u : 24u;
-            for (uint32_t k = 0; k < np[2 * s + proto]; ++k) {
-                lrc_ook_packet &p = h_packets[w++];
-                p.stream = (uint32_t)s; p.proto = (uint32_t)proto; p.seq = k; p.nbits = nbits;
-                memset(p.bits, 0, sizeof(p.bits));
-                const unsigned long long v = pk[(s * 2 + proto) * o->max_packets + k];
-                for (uint32_t i = 0; i < nbits; ++i) p.bits[i] = (uint8_t)((v >> (nbits - 1 - i)) & 1ull);
-            }
-        }
+    const uint32_t seq0[2] = {0, 0};
+    for (size_t s = 0; s < ns; ++s) h_packets = ook_put_packets(h_packets, pk.data(), o->max_packets, s, &np[2 * s], seq0);
     return LRC_OK;
 }
 
@@ -1525,11 +1533,11 @@ struct lrc_ook_stream {
     lrc_ook  *o;                      // the chain's buffers, sized for max_push_blocks; its d_mask / d_bsum / d_binfo rows start
                                       // with cpitch carry slots
     size_t    max_carry, max_packets;
-    OokSeam  *d_seam;                 // [n_streams]
-    uint8_t  *d_carry;                // [n_streams][cpitch][1024] the open burst's collected blocks
-    float    *d_cmax;                 // [n_streams][cpitch] their maxima
-    uint32_t *d_live;                 // [n_streams] carried blocks sliced in the current push
-    uint32_t *d_pbase;                // [n_streams][2] sequence number of the first packet not fetched yet
+    DevBuf<OokSeam>  d_seam;          // [n_streams]
+    DevBuf<uint8_t>  d_carry;         // [n_streams][cpitch][1024] the open burst's collected blocks
+    DevBuf<float>    d_cmax;          // [n_streams][cpitch] their maxima
+    DevBuf<uint32_t> d_live;          // [n_streams] carried blocks sliced in the current push
+    DevBuf<uint32_t> d_pbase;         // [n_streams][2] sequence number of the first packet not fetched yet
     size_t    last_push;              // blocks per stream of the last push (the debug block sums' row length)
     bool      failed;                 // a fetch reported an overflow: every call fails until reset
 };
@@ -1551,11 +1559,8 @@ extern "C" int lrc_ook_stream_reset(lrc_ook_stream *st)
 extern "C" int lrc_ook_stream_destroy(lrc_ook_stream *st)
 {
     if (!st) return LRC_OK;
-    if (st->o) {
-        cudaSetDevice(st->o->ctx->device);
-        cudaFree(st->d_seam); cudaFree(st->d_carry); cudaFree(st->d_cmax); cudaFree(st->d_live); cudaFree(st->d_pbase);
-        lrc_ook_destroy(st->o);
-    }
+    cudaSetDevice(st->o->ctx->device);
+    lrc_ook_destroy(st->o);
     delete st;
     return LRC_OK;
 }
@@ -1570,22 +1575,19 @@ extern "C" int lrc_ook_stream_create(lrc_ctx *ctx, size_t n_streams, size_t max_
     // an open burst never holds more than guard + 1 blocks (bitfount.rs:52-54): the buffer is reset before a block is pushed once it
     // exceeds the guard, so it ends at most one block past it, plus one more when it did not start with the 0.0.  That carry is
     // exact for every input; a smaller one is the caller's memory choice, and a burst that outgrows it is reported.
-    size_t guard_blocks = 1000u * (size_t)OOK_TRIGGER_DURATION;
-    if (const char *g = getenv("LRC_OOK_TEST_GUARD_BLOCKS")) { const long v = atol(g); if (v >= 1) guard_blocks = (size_t)v; }
-    const size_t max_carry = max_carry_blocks ? max_carry_blocks : guard_blocks + 1;
+    const size_t max_carry = max_carry_blocks ? max_carry_blocks : ook_guard_blocks() + 1;
     const size_t cpitch = (max_carry + 31) / 32 * 32;
     lrc_ook_stream *st = new (std::nothrow) lrc_ook_stream();
     LRC_REQUIRE(st != nullptr, LRC_ERR_NOMEM, "out of host memory");
-    memset(st, 0, sizeof(*st));
     const int rc = ook_create(ctx, n_streams, max_push_blocks, cpitch, sample_rate, max_runs_per_push, max_packets_per_fetch, &st->o);
     if (rc != LRC_OK) { delete st; return rc; }
     st->max_carry = max_carry;
     st->max_packets = st->o->max_packets;
-    cudaError_t e = cudaMalloc(&st->d_seam, n_streams * sizeof(OokSeam));
-    if (e == cudaSuccess) e = cudaMalloc(&st->d_carry, n_streams * cpitch * (size_t)(OOK_BLOCK * 2));
-    if (e == cudaSuccess) e = cudaMalloc(&st->d_cmax, n_streams * cpitch * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&st->d_live, n_streams * sizeof(uint32_t));
-    if (e == cudaSuccess) e = cudaMalloc(&st->d_pbase, n_streams * 2 * sizeof(uint32_t));
+    cudaError_t e = st->d_seam.alloc(n_streams);
+    if (e == cudaSuccess) e = st->d_carry.alloc(n_streams * cpitch * (size_t)(OOK_BLOCK * 2));
+    if (e == cudaSuccess) e = st->d_cmax.alloc(n_streams * cpitch);
+    if (e == cudaSuccess) e = st->d_live.alloc(n_streams);
+    if (e == cudaSuccess) e = st->d_pbase.alloc(n_streams * 2);
     if (e != cudaSuccess) {
         lrc_set_error("lrc_ook_stream_create: %s (carry of %zu blocks x %zu streams)", cudaGetErrorString(e), max_carry, n_streams);
         lrc_ook_stream_destroy(st);
@@ -1653,18 +1655,10 @@ extern "C" int lrc_ook_stream_fetch_packets(lrc_ook_stream *st, lrc_ook_packet *
     }
     std::vector<unsigned long long> pk(ns * 2 * mp);
     LRC_CUDA(cudaMemcpy(pk.data(), o->d_packets, pk.size() * 8, cudaMemcpyDeviceToHost));
-    size_t w = 0;
-    for (size_t s = 0; s < ns; ++s)
-        for (int proto = 0; proto < 2; ++proto) {
-            const uint32_t nbits = proto == 0 ? 36u : 24u;
-            for (uint32_t k = 0; k < z[s].m_count[proto] - base[2 * s + proto]; ++k) {
-                lrc_ook_packet &p = h_packets[w++];
-                p.stream = (uint32_t)s; p.proto = (uint32_t)proto; p.seq = base[2 * s + proto] + k; p.nbits = nbits;
-                memset(p.bits, 0, sizeof(p.bits));
-                const unsigned long long v = pk[(s * 2 + proto) * mp + k];
-                for (uint32_t i = 0; i < nbits; ++i) p.bits[i] = (uint8_t)((v >> (nbits - 1 - i)) & 1ull);
-            }
-        }
+    for (size_t s = 0; s < ns; ++s) {
+        const uint32_t n[2] = {z[s].m_count[0] - base[2 * s], z[s].m_count[1] - base[2 * s + 1]};
+        h_packets = ook_put_packets(h_packets, pk.data(), mp, s, n, &base[2 * s]);
+    }
     for (size_t s = 0; s < ns; ++s) { base[2 * s] = z[s].m_count[0]; base[2 * s + 1] = z[s].m_count[1]; }
     LRC_CUDA(cudaMemcpy(st->d_pbase, base.data(), ns * 2 * sizeof(uint32_t), cudaMemcpyHostToDevice));
     return LRC_OK;

@@ -76,23 +76,23 @@ extern "C" int lrc_psdpng_rows(lrc_ctx *ctx, const int16_t *d_pcm, size_t n_samp
     lrc_rfft *plan = nullptr;
     int rc = lrc_rfft_create(ctx, nfft, 0, &plan);                          // kiss_fftr_alloc(nfft,0,0,0)  :131
     if (rc) return rc;
-    float *d_frames = nullptr, *d_freq = nullptr;
-    cudaError_t e = cudaMalloc(&d_frames, use * (size_t)nfft * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&d_freq, use * (size_t)nfreqs * sizeof(float2));
+    DevBuf<float> d_frames;
+    DevBuf<float2> d_freq;
+    cudaError_t e = d_frames.alloc(use * (size_t)nfft);
+    if (e == cudaSuccess) e = d_freq.alloc(use * (size_t)nfreqs);
     if (e == cudaSuccess) {
         psdpng_frames_kernel<<<(unsigned)use, 256, 0, s>>>(d_pcm, d_frames, nfft, stereo ? 1 : 0, remove_dc ? 1 : 0);
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) rc = lrc_rfft_run(plan, d_frames, d_freq, use, s);
+    if (e == cudaSuccess) rc = lrc_rfft_run(plan, d_frames, (float *)d_freq.get(), use, s);
     if (e == cudaSuccess && rc == LRC_OK) {
         size_t blocks = ceil_div(rows * (size_t)nfreqs, 256);
         const size_t cap = (size_t)ctx->n_sm * 16;
         if (blocks > cap) blocks = cap;
-        psdpng_rows_kernel<<<(unsigned)blocks, 256, 0, s>>>((const float2 *)d_freq, d_rows, rows, nfreqs, navg);
+        psdpng_rows_kernel<<<(unsigned)blocks, 256, 0, s>>>(d_freq, d_rows, rows, nfreqs, navg);
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);                     // scratch is freed below
-    cudaFree(d_frames); cudaFree(d_freq);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);                     // scratch is freed on return
     lrc_rfft_destroy(plan);
     if (e != cudaSuccess) { lrc_set_error("lrc_psdpng_rows: %s", cudaGetErrorString(e)); return LRC_ERR_CUDA; }
     return rc;
